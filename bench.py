@@ -6,6 +6,7 @@
     python bench.py --impl reference --steps K --warmup W   # the reference algorithm on the host cores
     python bench.py --config {1,2,3,5} [--joint]            # the other BASELINE configs (2 = default)
     python bench.py --mode operator [--grid full]           # config 4: operator sweep (table, JSON lines)
+    python bench.py --steps K --warmup W --dump-outputs DIR # also write the timed run's outputs as DIR/*.npy
 
 Workload of the contract line (config.workload): BASELINE configs[1] per-GPU slice -- 8 chains of
 T=184184 samples at 22.05 kHz per GPU (64 chains over 8 GPUs), random-init CQTDiff+ (44.5 M parameters,
@@ -203,7 +204,8 @@ def run_ours(a):
     smp.joint = joint
     T = cfg["T"]
     K, W = a.steps, a.warmup
-    assert W + K <= args.tester.T, "steps + warmup must fit the sampler schedule"
+    if W + K > args.tester.T:
+        raise SystemExit(f"--steps {K} + --warmup {W} exceed the {args.tester.T}-step sampler schedule")
     n_par = len(cfg["fc"])
 
     def timed_run(mode):
@@ -273,6 +275,7 @@ def run_ours(a):
                 xg = segments.merge(xg, extra["spans"], extra["L"])
             ev["gathered"] = [tuple(xg.shape), tuple(pg.shape)]
             finish()
+        ev["out"] = (x.clone(), p.clone())         # outside the timed region; later passes must not overwrite it
         ms = ev["s"].elapsed_time(ev["e"])
         ev["ms"] = bd.max_over_ranks(ms, device)
         return ev, h2d, d2h
@@ -305,6 +308,7 @@ def run_ours(a):
     ct = torch.tensor([float(chains)], dtype=torch.float64, device=device)
     bd.sum_over_ranks_(ct)
     total_chains = int(ct.item())
+    dumped = dump_outputs(a.dump_outputs, *dev_run["out"], rank) if a.dump_outputs else None
     value = total_chains * K / (dev_run["ms"] / 1e3)
     e2e_value = total_chains * K / (e2e_run["ms"] / 1e3)
 
@@ -395,7 +399,38 @@ def run_ours(a):
         "clocks": clocks,
         "roofline": roof, "operator_roofline": op_roof, "cpu_baseline": cpu,
     }
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     print(json.dumps(line))
+
+
+DUMP_BYTES = 64_000_000          # all files of one dump, .npy headers included
+NPY_HEADER_BYTES = 4096          # generous bound on one .npy header
+
+
+def dump_outputs(out_dir, x, p, rank):
+    """Write what the timed device-resident run returned after its last step -- the audio estimates of all
+    ranks' chains and each rank's filter parameters -- as float32 DIR/<name>.npy, so that two builds can be
+    compared output for output on identical inputs.  Estimates above the byte budget are written as every
+    k-th element of the flattened rows (x_every_<k>.npy).  Arrays an earlier dump left in DIR are removed
+    first.  Returns {name: shape} on rank 0."""
+    import glob
+    import numpy as np
+    from babe_b200 import distributed as bd
+    x, p = bd.gather_rows(x), bd.gather_params(p)
+    if rank != 0:
+        return None
+    x, p = x.float().cpu(), p.float().cpu()
+    k = -(-x.numel() * 4 // (DUMP_BYTES - 2 * NPY_HEADER_BYTES - p.numel() * 4))
+    arrays = {"x" if k == 1 else f"x_every_{k}": x if k == 1 else x.reshape(-1)[::k], "filter_params": p}
+    os.makedirs(out_dir, exist_ok=True)
+    for old in glob.glob(os.path.join(out_dir, "x_every_*.npy")) + [os.path.join(out_dir, n) for n in
+                                                                   ("x.npy", "filter_params.npy")]:
+        if os.path.exists(old):
+            os.remove(old)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr.numpy())
+    return {name: list(arr.shape) for name, arr in arrays.items()}
 
 
 # ---------------------------------------------------------------------------
@@ -600,16 +635,16 @@ def run_reference(a):
         return
     cfg = CONFIGS[a.config]
     K, W = a.steps, a.warmup
-    # bounded sample: ONE of the GPU arm's chains at full length; to stay within a few minutes the timed
-    # steps are capped (the per-step time of the CPU path does not depend on the step index)
-    Kc = min(K, a.ref_max_steps)
+    # bounded sample: ONE of the GPU arm's chains at full length; main() rejects more timed steps than
+    # --ref-max-steps, and the warm-up is capped (the per-step time of the CPU path does not depend on the step index)
+    Kc = K
     Wc = min(W, 5)
     dt = cpu_time_steps(a.config, Kc, Wc)
     v = Kc / dt
     cpu = {"value": round(v, 5), "unit": "chain-steps/s", "cores": torch.get_num_threads(), "kind": "port",
            "sample": f"1 chain of the workload at full length T={cfg['T']}, {Kc} timed sampler steps after {Wc} warm-up "
-                     f"steps (requested {K}/{W}; capped to bound the run), measured, not extrapolated; the reference is "
-                     "Python: the oracle port restates it and /root/reference is not on the GPU box"}
+                     f"steps (requested {K}/{W}; warm-up capped to bound the run), measured, not extrapolated; the reference is "
+                     "Python: the oracle port restates it"}
     n_par = len(cfg["fc"])
     line = {"impl": "reference", "metric": "blind-BWE sampler chain-steps/s", "value": round(v, 5),
             "unit": "chain-steps/s", "n_gpus": a.gpus, "steps": Kc, "warmup": Wc,
@@ -709,7 +744,7 @@ def main():
     ap.add_argument("--grid", default="", choices=["", "full"], help="operator mode: the full 2^14..2^20 x 1..512 grid")
     ap.add_argument("--nffts", default="4096", help="operator mode: comma-separated NFFTs (e.g. 4096,1024)")
     ap.add_argument("--ref-max-steps", type=int, default=30,
-                    help="reference arm: cap on timed steps (each ~7 s of host time at T=184184)")
+                    help="reference arm: largest --steps accepted (each step ~7 s of host time at T=184184)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling aid: skip the host-buffer leg")
     ap.add_argument("--no-cuda-graph", action="store_true",
@@ -719,8 +754,15 @@ def main():
     ap.add_argument("--single-pass", action="store_true",
                     help="profiling aid: skip the second (per-kernel event timing) pass")
     ap.add_argument("--no-autotune", action="store_true", help="profiling aid: cudnn.benchmark off")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the audio estimates and filter parameters of the timed run's last step as DIR/*.npy")
     a = ap.parse_args()
-    a.steps = max(1, a.steps)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.impl == "reference" and a.steps > a.ref_max_steps:
+        ap.error(f"--impl reference times at most --ref-max-steps ({a.ref_max_steps}) steps; raise it to time more")
+    if a.dump_outputs and (a.impl == "reference" or a.mode == "operator"):
+        ap.error("--dump-outputs writes the outputs of the CUDA sampler run (--impl ours --mode sampler)")
     if a.impl != "reference":
         a.warmup = max(1, a.warmup)          # the timed region starts after a completed (untimed) step
     if a.impl == "reference":

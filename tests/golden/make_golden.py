@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Generate golden vectors by importing the UNMODIFIED reference.
 
-Run in the authoring container only (needs /root/reference):
+Needs BABE_REFERENCE set to a checkout of eloimoliner/BABE:
 
     python tests/golden/make_golden.py
 
@@ -20,7 +20,7 @@ from types import SimpleNamespace as NS
 import numpy as np
 import torch
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
+REF = os.environ.get("BABE_REFERENCE") or sys.exit("set BABE_REFERENCE to a checkout of eloimoliner/BABE")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))          # tests/ for toy_model
 sys.path.insert(0, REF)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Golden vectors for the non-blind / autoregressive sampling methods, produced by the UNMODIFIED
 reference sampler (testing/blind_bwe_sampler.py: predict_bwe_AR :259-303, predict_bwe :306-364,
-predict :406-497) with the toy denoiser.  Authoring container only (needs /root/reference):
+predict :406-497) with the toy denoiser.  Needs BABE_REFERENCE set to a checkout of eloimoliner/BABE:
 
     python tests/golden/make_golden_ar.py        ->  tests/golden/sampler_ar.npz
 """

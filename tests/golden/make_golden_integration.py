@@ -6,7 +6,7 @@
 
 Small configuration: 3 octaves x 8 bins, T = 4096 samples, NFFT 1024, 2 sampler steps, 5 fit iterations,
 torch.manual_seed(0) network init (zero-initialised gates scaled so that they matter), torch.manual_seed(42) sampling.
-Run in the authoring container only:   python tests/golden/make_golden_integration.py  ->  integration.npz
+Needs BABE_REFERENCE set to a checkout of eloimoliner/BABE:   python tests/golden/make_golden_integration.py  ->  integration.npz
 """
 import importlib
 import os

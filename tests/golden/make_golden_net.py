@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Golden vectors for the denoiser layer glue, produced by the UNMODIFIED reference modules
 (networks/cqtdiff+.py: ResnetBlock :382-487 with BiasFreeGroupNorm :137-163, UpDownResample
-:522-580).  Authoring container only (needs /root/reference):
+:522-580).  Needs BABE_REFERENCE set to a checkout of eloimoliner/BABE:
 
     python tests/golden/make_golden_net.py        ->  tests/golden/net_glue.npz
 
@@ -16,7 +16,7 @@ import types
 import numpy as np
 import torch
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
+REF = os.environ.get("BABE_REFERENCE") or sys.exit("set BABE_REFERENCE to a checkout of eloimoliner/BABE")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REF)
 stub = types.ModuleType("cqt_nsgt_pytorch")

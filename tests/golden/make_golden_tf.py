@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Teacher-forcing goldens from the UNMODIFIED reference (run in the authoring container only):
+"""Teacher-forcing goldens from the UNMODIFIED reference (needs BABE_REFERENCE set to a checkout of eloimoliner/BABE):
 
     python tests/golden/make_golden_tf.py      ->  tests/golden/teacher_forced.npz, optional_branches.npz
 
@@ -12,6 +12,9 @@
   wrapping ``move_timestep`` / ``fit_params`` / ``torch.randn`` from the outside.
 * ``optional_branches.npz``: two-step runs of the non-default branches of ``get_rec_grads`` and of the loop
   (:63-73, :80-86, :99-115): data consistency, smooth-L1, cosine, STFT / STFT-magnitude / log-magnitude distances.
+  Each array is stored once (the file stays under 1 MB): the observation of every run is ``fit_sampler.npz``'s
+  ``y`` (its first 4000 samples for the STFT distances), and runs of one length draw the same noise
+  (``opt_draws_4096``, ``opt_draws_4000``) except SNR_observations, which draws more (``opt_snr_draws``).
 
 A test that starts the CUDA kernels from each reference iterate / state and compares ONE iteration / ONE step
 closes the parity argument that the chained comparisons (chaotic amplification of fp32 rounding in the
@@ -172,10 +175,13 @@ def gen_optional():
         torch.manual_seed(1)
         with Recorder(sampler) as rec:
             x, p = sampler.predict_blind_bwe(y.clone(), rid=False)
-        out[f"opt_{variant}_y"] = y
+        assert torch.equal(y, torch.from_numpy(g["y"])[:, :T_len])
+        draws = torch.stack(rec.draws)
+        key = "opt_snr_draws" if variant == "snr" else f"opt_draws_{T_len}"
+        assert key not in out or torch.equal(out[key], draws), variant
+        out[key] = draws
         out[f"opt_{variant}_x"] = x
         out[f"opt_{variant}_p"] = p
-        out[f"opt_{variant}_draws"] = torch.stack(rec.draws)
         print("optional", variant, float(x.abs().mean()), p.flatten()[:3].tolist())
     return out
 

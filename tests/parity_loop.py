@@ -3,9 +3,9 @@ testing/blind_bwe_sampler.py:9 imports it -- so that after ``babe_b200.install()
 CUDA drop-ins through the reference's own call pattern (apply_stft on both signals, design_filter inside the
 closure, autograd.grad(create_graph=True) on the weighted STFT-magnitude norm, in-place sequential clamps,
 apply_filter inside the guidance graph, autograd.grad wrt the noisy input through the denoiser).  Default branches of
-conf/tester/blind_bwe.yaml only.  On the CPU (authoring container) the same loop runs on the reference's own module
-and must reproduce the golden of the unmodified BlindSampler bit for bit (tests/test_integration_cpu.py), which is
-what validates this restatement."""
+conf/tester/blind_bwe.yaml only.  On the CPU the same loop runs on the oracle operators and must reproduce the golden
+of the unmodified BlindSampler (tests/test_integration_cpu.py), which is what validates this restatement; with
+BABE_REFERENCE set it also runs on the reference's own module."""
 import torch
 
 

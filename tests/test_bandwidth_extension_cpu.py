@@ -1,5 +1,5 @@
 """CPU: the design helpers / dispatcher of babe_b200.bandwidth_extension against the reference module
-(needs /root/reference; skipped elsewhere) and against closed forms."""
+(needs BABE_REFERENCE set to a checkout of eloimoliner/BABE; skipped elsewhere) and against closed forms."""
 import importlib
 import math
 import os
@@ -11,7 +11,7 @@ import torch
 
 from conftest import rel_l2
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
+REF = os.environ.get("BABE_REFERENCE", "")
 
 
 def _cfg(kind):
@@ -40,7 +40,7 @@ def test_decimate_and_dispatch():
     assert abs(bwe.prepare_filter(_cfg("resample"), 22050) - 22050 / 2000) < 1e-12
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="BABE_REFERENCE (reference checkout) not set")
 @pytest.mark.parametrize("kind", ["firwin", "firwin_hpf", "cheby1", "biquad", "resample", "decimate"])
 def test_prepare_filter_matches_reference(kind):
     from babe_b200 import bandwidth_extension as bwe
@@ -60,7 +60,7 @@ def test_prepare_filter_matches_reference(kind):
         assert a == b
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="BABE_REFERENCE (reference checkout) not set")
 def test_iir_models_match_reference():
     """The library-delegated observation models (outside the hand-written path) behave like the reference's."""
     from babe_b200 import bandwidth_extension as bwe

@@ -1,6 +1,7 @@
 """CPU: the in-repo CQTDiff+ restatement (babe_b200/denoiser.py) against the
-reference network file, both running on the oracle CQT.  Needs /root/reference
-(authoring container); skipped elsewhere."""
+reference network file, both running on the oracle CQT.  Needs BABE_REFERENCE set to a checkout of
+eloimoliner/BABE; skipped elsewhere (tests/test_integration_cpu.py checks the network's output against the
+reference's stored output everywhere)."""
 import importlib
 import os
 import sys
@@ -12,8 +13,8 @@ import torch
 from conftest import rel_l2
 from oracle.cqt_shim import OracleCQT
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+REF = os.environ.get("BABE_REFERENCE", "")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="BABE_REFERENCE (reference checkout) not set")
 
 
 def _small_args():

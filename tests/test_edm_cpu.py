@@ -1,5 +1,6 @@
-"""CPU: babe_b200.edm.EDM against the reference class diff_params/edm.py (needs /root/reference;
-skipped elsewhere): schedules, preconditioning, training-side members under the same seeds."""
+"""CPU: babe_b200.edm.EDM against the reference class diff_params/edm.py: the sampler's schedules against the
+values the reference produced (tests/golden/fit_sampler.npz), and -- with BABE_REFERENCE set to a checkout of
+eloimoliner/BABE -- schedules, preconditioning, training-side members under the same seeds."""
 import importlib
 import os
 import sys
@@ -12,8 +13,21 @@ import torch
 from conftest import rel_l2
 from toy_model import ToyDenoiser
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+REF = os.environ.get("BABE_REFERENCE", "")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="BABE_REFERENCE (reference checkout) not set")
+
+
+def test_sampler_schedules_match_reference_golden(golden):
+    """The schedule and gamma of the sampler's EDM (tester block applied, as the reference sampler does) are
+    bit-identical to the reference's (tests/golden/make_golden.py)."""
+    from babe_b200 import edm, sampler
+    g = golden("fit_sampler.npz")
+    args = sampler.make_args(sample_rate=int(g["sr"]), audio_len=g["x"].shape[1], T=4, NFFT=int(g["nfft"]))
+    diff = sampler.BlindSamplerFused(ToyDenoiser(), edm.EDM(args), args).diff_params
+    t = diff.create_schedule_from_initial_t(0.2, 35)
+    assert np.array_equal(t.numpy(), g["sched35"])
+    assert np.array_equal(diff.get_gamma(t).numpy(), g["gamma35"])
+    assert np.array_equal(diff.create_schedule(35).numpy(), g["sched_full"])
 
 
 def _pair():
@@ -30,6 +44,7 @@ def _pair():
     return edm.EDM(args), ref.EDM(args)
 
 
+@needs_ref
 def test_schedules_and_preconditioning():
     mine, ref = _pair()
     for n in (4, 35):
@@ -42,6 +57,7 @@ def test_schedules_and_preconditioning():
         assert rel_l2(getattr(mine, f)(s), getattr(ref, f)(s)) < 1e-7
 
 
+@needs_ref
 def test_training_side_members():
     mine, ref = _pair()
     np.random.seed(3)

@@ -1,9 +1,12 @@
-"""CPU (authoring container, needs /root/reference): integration row of SURVEY section 4.
+"""CPU: integration row of SURVEY section 4, against the golden the unmodified reference sampler + unmodified
+reference network produced (tests/golden/integration.npz).
 
-* the UNMODIFIED reference sampler on the in-repo denoiser restatement (babe_b200.denoiser.CQTDiffPlus on the oracle
-  CQT) reproduces the golden the unmodified sampler + unmodified network produced (tests/golden/integration.npz);
-* the test-local restatement of the loop (tests/parity_loop.py) on the reference's OWN operator module reproduces the
-  same golden -- which validates the helper that the GPU tests run on the CUDA drop-ins through babe_b200.install();
+* the in-repo denoiser restatement (babe_b200.denoiser.CQTDiffPlus on the oracle CQT) gives the reference network's
+  output, and the test-local restatement of the loop (tests/parity_loop.py) on it and on the oracle operators
+  reproduces the reference run -- which validates the helper that the GPU tests run on the CUDA drop-ins through
+  babe_b200.install();
+* with BABE_REFERENCE set to a checkout of eloimoliner/BABE: the UNMODIFIED reference sampler on the denoiser
+  restatement, and the loop restatement on the reference's OWN operator module, reproduce the same golden;
 * the three Hydra callable strings resolve through babe_b200.callables (and through the reference's own dnnlib) to
   classes with the constructor signatures the reference uses (utils/setup.py:49,55; testing/blind_bwe_tester.py:214).
 """
@@ -17,8 +20,8 @@ import torch
 
 from conftest import rel_l2
 
-REF = os.environ.get("BABE_REFERENCE", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+REF = os.environ.get("BABE_REFERENCE", "")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="BABE_REFERENCE (reference checkout) not set")
 
 
 def _small(golden):
@@ -50,6 +53,29 @@ def _ref_modules():
     from testing.blind_bwe_sampler import BlindSampler
     from diff_params.edm import EDM
     return ref_ops, BlindSampler, EDM
+
+
+def test_denoiser_restatement_matches_reference_network(golden):
+    from oracle.cqt_shim import OracleCQT
+    args, g = _small(golden)
+    net = _my_network(args, cqt=OracleCQT(3, 8, fs=22050, audio_len=4096))
+    assert rel_l2(net(torch.from_numpy(g["net_in"]), torch.from_numpy(g["net_sigma"])), g["net_out"]) < 1e-5
+
+
+def test_parity_loop_helper_on_oracle_operators(golden):
+    import parity_loop
+    from babe_b200.edm import EDM
+    from oracle import stft_filter as osf
+    from oracle.cqt_shim import OracleCQT
+    args, g = _small(golden)
+    net = _my_network(args, cqt=OracleCQT(3, 8, fs=22050, audio_len=4096))
+    torch.manual_seed(42)
+    trace = []
+    x, p = parity_loop.predict_blind_bwe(osf, net, EDM(args), args, torch.from_numpy(g["y"]).clone(), trace=trace)
+    assert rel_l2(x, g["x"]) < 2e-5 and rel_l2(p, g["params"]) < 2e-5
+    assert len(trace) == g["x_out"].shape[0]
+    for i, (xi, pi, di) in enumerate(trace):
+        assert rel_l2(xi, g["x_out"][i]) < 2e-5 and rel_l2(di, g["x_den"][i]) < 2e-5
 
 
 @needs_ref

@@ -69,9 +69,14 @@ def test_smooth_mask_literal():
     assert torch.equal(S.prepare_smooth_mask(m, 50), literal(m, 50))
 
 
-def test_cuda_graph_option_falls_back_to_eager_without_cuda(golden):
-    """``cuda_graph=True`` must never break sampling: any capture problem -> eager model + a warning."""
+def test_cuda_graph_option_falls_back_to_eager_without_cuda(golden, monkeypatch):
+    """``cuda_graph=True`` must never break sampling: any capture problem -> eager model + a warning.  The capture is
+    made to fail, as it does without a CUDA device, so that the fallback is exercised on GPU machines too."""
     import pytest
+
+    def no_capture(*a, **k):
+        raise RuntimeError("CUDA-graph capture unavailable")
+    monkeypatch.setattr(torch.cuda, "make_graphed_callables", no_capture)
     g = golden("sampler_ar.npz")
     s, args = _sampler(g)
     s.cuda_graph = True

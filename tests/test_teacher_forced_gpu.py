@@ -103,7 +103,8 @@ def test_optional_branches_match_reference(golden, variant):
     from babe_b200 import edm, sampler
     g = golden("optional_branches.npz")
     fs = golden("fit_sampler.npz")
-    y = cuda(g[f"opt_{variant}_y"])
+    T = 4000 if variant.startswith("stft") else fs["y"].shape[1]       # see make_golden_tf.gen_optional
+    y = cuda(fs["y"][:, :T])
     args = sampler.make_args(sample_rate=int(fs["sr"]), audio_len=y.shape[1], T=2, NFFT=int(fs["nfft"]), max_iter=2)
     ps = args.tester.posterior_sampling
     if variant == "data_consistency":
@@ -119,7 +120,7 @@ def test_optional_branches_match_reference(golden, variant):
         ps.stft_distance.mag = variant != "stft"
         ps.stft_distance.logmag = variant == "stft_logmag"
     s = sampler.BlindSamplerFused(ToyDenoiser().cuda(), edm.EDM(args), args, rid=False)
-    draws = iter(g[f"opt_{variant}_draws"])
+    draws = iter(g["opt_snr_draws" if variant == "snr" else f"opt_draws_{T}"])
     s.noise_fn = lambda shape, dev: cuda(next(draws))
     x, p = s.predict_blind_bwe(y.clone())
     assert rel_l2(p.cpu(), g[f"opt_{variant}_p"]) < 1e-4, variant
