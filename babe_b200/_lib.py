@@ -68,6 +68,10 @@ SIGNATURES = {
                                   c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                   c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p,
                                   c_void_p]),
+    "babe_apply_filter_rows": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p,
+                                       c_void_p]),
     "babe_stft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                           c_int, c_void_p, c_void_p]),
     "babe_istft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
@@ -90,6 +94,9 @@ SIGNATURES = {
     "babe_stft_stats_workspace": (c_size_t, [c_int, c_int, c_int]),
     "babe_stft_stats": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
                                 c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "babe_stft_stats_rows_workspace": (c_size_t, [c_int, c_int, c_int]),
+    "babe_stft_stats_rows": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_size_t, c_void_p]),
     "babe_spec_mag_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                     c_void_p, c_void_p]),
     "babe_spec_mag_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
@@ -99,6 +106,8 @@ SIGNATURES = {
                                     c_void_p, c_void_p, c_void_p]),
     "babe_fit_params": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int,
                                 POINTER(FitConfig), c_void_p, c_void_p]),
+    "babe_fit_params_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int,
+                                     POINTER(FitConfig), c_void_p, c_void_p]),
     "babe_cqt_workspace": (c_size_t, [POINTER(CqtPlan), c_int]),
     "babe_rfft": (c_int, [POINTER(CqtPlan), c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_size_t,
                           c_void_p]),

@@ -156,6 +156,30 @@ def apply_filter(x, H, NFFT):
     return _FilterOp.apply(x, H, int(NFFT), False)
 
 
+class _RowFilterOp(torch.autograd.Function):
+    """y_b = A_{fc_b, A_b} x_b (or its adjoint): one filter per row, designed inside the kernel.  Linear in x; the
+    filter parameters get no gradient."""
+
+    @staticmethod
+    def forward(ctx, x, freqs, fc, A, nfft, adjoint):
+        ctx.nfft, ctx.adjoint = nfft, adjoint
+        ctx.save_for_backward(freqs, fc, A)
+        return ops.apply_filter_rows(x, nfft, freqs, fc, A, adjoint=adjoint)
+
+    @staticmethod
+    def backward(ctx, g):
+        freqs, fc, A = ctx.saved_tensors
+        gx = None
+        if ctx.needs_input_grad[0]:
+            gx = _RowFilterOp.apply(g.contiguous(), freqs, fc, A, ctx.nfft, not ctx.adjoint)
+        return gx, None, None, None, None, None
+
+
+def apply_filter_rows(x, freqs, fc, A, NFFT):
+    """Row b of x (B, T) through the lowpass designed from fc[b], A[b] (fc, A: (B, K))."""
+    return _RowFilterOp.apply(x, freqs, fc.contiguous(), A.contiguous(), int(NFFT), False)
+
+
 def apply_stft(x, NFFT):
     """utils/blind_bwe_utils.py:15-26."""
     return _Stft.apply(x, int(NFFT))

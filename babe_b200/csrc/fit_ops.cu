@@ -554,12 +554,23 @@ __global__ void __launch_bounds__(FIT_THREADS, 1) k_fit_params2(const FitArgs a)
 constexpr int FIT3_NC = 4;            // CTAs per cluster
 constexpr int FIT3_NB = 2;            // bins per thread: F <= 4 * 512 * 2
 
-template <int K>
+// ROWS: one independent fit per cluster; cluster b reads abc[b] (3 F doubles) and owns params[b] (2 K floats) and
+// iters_out[b].  Every exchange stays inside the cluster.
+template <int K, bool ROWS>
 __global__ void __cluster_dims__(FIT3_NC, 1, 1) __launch_bounds__(FIT_THREADS, 1) k_fit_params3(const FitArgs a) {
   cg::cluster_group cluster = cg::this_cluster();
   const int rank = (int)cluster.block_rank();
   constexpr int KP = K;
   const int F = a.F;
+  const double* abc = a.abc;
+  float* params = a.params;
+  int* iters_out = a.iters_out;
+  if (ROWS) {
+    const size_t b = blockIdx.x / FIT3_NC;
+    abc += b * 3 * F;
+    params += b * 2 * K;
+    if (iters_out != nullptr) iters_out += b;
+  }
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* sf = reinterpret_cast<float*>(smem_raw);                       // bin frequencies
   __shared__ int s_kf[KMAX];
@@ -589,9 +600,9 @@ __global__ void __cluster_dims__(FIT3_NC, 1, 1) __launch_bounds__(FIT_THREADS, 1
       const int k = kb0 + FIT_THREADS * i;
       const double w2 = (double)a.w[k] * (double)a.w[k];
       fk[i] = a.freqs[k];
-      wa[i] = w2 * a.abc[k];
-      wb[i] = w2 * a.abc[F + k];
-      ct += w2 * a.abc[2 * F + k];
+      wa[i] = w2 * abc[k];
+      wb[i] = w2 * abc[F + k];
+      ct += w2 * abc[2 * F + k];
     }
   }
   for (int k = tid; k < F; k += FIT_THREADS) sf[k] = a.freqs[k];
@@ -603,7 +614,7 @@ __global__ void __cluster_dims__(FIT3_NC, 1, 1) __launch_bounds__(FIT_THREADS, 1
   // ---- breakpoint state in the registers of warp 0, lanes 0..K-1 --------------------------------------------
   const bool bp = warp == 0 && lane < K;
   float fc = 0.f, A = 0.f, fc_prev = 0.f, A_prev = 0.f;
-  if (bp) { fc = a.params[lane]; A = a.params[K + lane]; }
+  if (bp) { fc = params[lane]; A = params[K + lane]; }
   const float f0 = sf[0];
   const float df = F > 1 ? (sf[F - 1] - sf[0]) / (float)(F - 1) : 1.0f;
   const float inv_df = 1.0f / df;
@@ -849,8 +860,8 @@ __global__ void __cluster_dims__(FIT3_NC, 1, 1) __launch_bounds__(FIT_THREADS, 1
     it = iter + 1;
     if (stop_flag) break;
   }
-  if (rank == 0 && bp) { a.params[lane] = fc; a.params[K + lane] = A; }
-  if (rank == 0 && tid == 0 && a.iters_out != nullptr) *a.iters_out = it;
+  if (rank == 0 && bp) { params[lane] = fc; params[K + lane] = A; }
+  if (rank == 0 && tid == 0 && iters_out != nullptr) *iters_out = it;
   cluster.sync();                           // no CTA exits while a peer may still address its shared memory
   (void)my_kf;
 }
@@ -1025,6 +1036,23 @@ __global__ void __launch_bounds__(SPEC_THREADS) k_spec_dist_grad(const float2* X
   }
 }
 
+template <bool ROWS>
+static int launch_fit3(const FitArgs& a, int B, cudaStream_t st) {
+  const size_t smem3 = (size_t)a.F * sizeof(float) + 16;
+  const int grid = FIT3_NC * B;
+  switch (a.K) {
+    case 1: k_fit_params3<1, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 2: k_fit_params3<2, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 3: k_fit_params3<3, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 4: k_fit_params3<4, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 5: k_fit_params3<5, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 6: k_fit_params3<6, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    case 7: k_fit_params3<7, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+    default: k_fit_params3<8, ROWS><<<grid, FIT_THREADS, smem3, st>>>(a); break;
+  }
+  return check_launch("k_fit_params3");
+}
+
 static int g_fit_variant = 0;     // 0: k_fit_params3 (4-CTA cluster), 1: k_fit_params2 (one CTA), -1: round-1 k_fit_params
                                   // (A/B: babe_set_fit_variant; babe_set_fused_variant(-1 / 0) sets it too)
 void set_fit_variant(int v) { g_fit_variant = v; }
@@ -1071,19 +1099,7 @@ extern "C" int babe_fit_params(const double* abc, const float* w, const float* f
   BABE_REQUIRE(F >= 1 && smem <= 200 * 1024, BABE_EUNSUPPORTED, "fit_params: F=%d too large", F);
   FitArgs a{abc, w, freqs, F, params, K, *cfg, iters_out};
   if (K <= 8 && F <= FIT3_NC * FIT_THREADS * FIT3_NB && g_fit_variant == 0) {     // cluster kernel (default)
-    const size_t smem3 = (size_t)F * sizeof(float) + 16;
-    cudaStream_t st3 = static_cast<cudaStream_t>(stream);
-    switch (K) {
-      case 1: k_fit_params3<1><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 2: k_fit_params3<2><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 3: k_fit_params3<3><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 4: k_fit_params3<4><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 5: k_fit_params3<5><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 6: k_fit_params3<6><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      case 7: k_fit_params3<7><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-      default: k_fit_params3<8><<<FIT3_NC, FIT_THREADS, smem3, st3>>>(a); break;
-    }
-    return check_launch("k_fit_params3");
+    return launch_fit3<false>(a, 1, static_cast<cudaStream_t>(stream));
   }
   if (K <= 8 && F <= FIT_THREADS * FIT2_NB && g_fit_variant >= 0) {     // second-generation kernel
     const size_t smem2 = (size_t)F * sizeof(float) + 16;
@@ -1103,6 +1119,24 @@ extern "C" int babe_fit_params(const double* abc, const float* w, const float* f
   cudaFuncSetAttribute(k_fit_params, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   k_fit_params<<<1, FIT_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(a);
   return check_launch("k_fit_params");
+}
+
+extern "C" int babe_fit_params_rows(const double* abc, const float* w, const float* freqs, int F, float* params,
+                                    int B, int K, const babe_fit_config* cfg, int* iters_out, void* stream) {
+  BABE_REQUIRE(abc && w && freqs && params && cfg, BABE_EBADARG, "fit_params_rows: null pointer");
+  BABE_REQUIRE(B >= 0, BABE_EBADARG, "fit_params_rows: B=%d", B);
+  BABE_REQUIRE(K >= 1 && K <= KMAX, BABE_EBADARG, "fit_params_rows: K=%d outside [1,%d]", K, KMAX);
+  if (B == 0) return BABE_OK;
+  if (K <= 8 && F >= 1 && F <= FIT3_NC * FIT_THREADS * FIT3_NB && g_fit_variant == 0) {   // one cluster per row
+    FitArgs a{abc, w, freqs, F, params, K, *cfg, iters_out};
+    return launch_fit3<true>(a, B, static_cast<cudaStream_t>(stream));
+  }
+  for (int b = 0; b < B; ++b) {           // other kernels: one shared-mode fit per row
+    const int rc = babe_fit_params(abc + (size_t)b * 3 * F, w, freqs, F, params + (size_t)b * 2 * K, K, cfg,
+                                   iters_out == nullptr ? nullptr : iters_out + b, stream);
+    if (rc) return rc;
+  }
+  return BABE_OK;
 }
 
 extern "C" int babe_spec_mag_stats(const float* X, const float* Xref, const float* H,

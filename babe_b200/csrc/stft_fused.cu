@@ -87,7 +87,9 @@ constexpr size_t fused_smem_bytes() {
 //
 // EPI: 0 none, 1 subtract + sum of squares (guidance residual), 2 row scale (guidance adjoint),
 //      3 any combination decided at run time
-template <bool ADJ, int EPI>
+// ROWS: one filter per row, fc / A are [B, K] and status is int[B]; H is (re)designed whenever the CTA's
+//       segment loop enters a new row, between two segments, when no bulk copy is in flight
+template <bool ADJ, int EPI, bool ROWS>
 __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
   using C = Core4k;
   constexpr bool SUBSTAGE = EPI == 1 || EPI == 3;
@@ -118,7 +120,9 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
     ws[n] = ADJ ? plain : fold;
   }
   constexpr float inv_n = 1.0f / C::N;
-  if (a.H != nullptr) {
+  if (ROWS) {
+    // per-row H: designed in the segment loop
+  } else if (a.H != nullptr) {
     for (int k = t; k < C::F; k += 256) hp[C::perm_of_bin(k)] = a.H[k] * inv_n;
   } else {
     float* fs = stage;                                           // the staging area is still free
@@ -151,9 +155,24 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
   const long long total = (long long)a.B * a.nblk;
   long long b0 = (long long)blockIdx.x * a.q;
   const long long b1 = b0 + a.q < total ? b0 + a.q : total;
+  int designed = -1;                                             // ROWS: row whose H is in hp
   while (b0 < b1) {
     // ---- one segment: blocks [j0, j1) of one row -------------------------------------------------------
     const int row = (int)(b0 / a.nblk);
+    if (ROWS && row != designed) {
+      // H of this row.  The staging area is scratch for the bin frequencies, as in the prologue: between two
+      // segments no bulk copy is in flight (the last pair's copy was consumed before its closing barrier, which
+      // every thread has passed, so hp and segs are no longer read either)
+      float* fs = stage;
+      for (int k = t; k < C::F; k += 256) fs[k] = a.freqs[k];
+      __syncthreads();
+      build_segments_coop(segs, fkf, a.fc + (size_t)row * a.K, a.A + (size_t)row * a.K, a.K, fs, C::F);
+      if (t == 0 && segs.bad && a.status != nullptr) a.status[row] = 1;
+      for (int k = t; k < C::F; k += 256) hp[C::perm_of_bin(k)] = bin_gain(segs, k, fs[k]) * inv_n;
+      designed = row;
+      __syncthreads();                                           // hp complete, fs read before the copy below
+      if (t == 0) fence_proxy_async();                           // generic-proxy writes of the stage before the copy
+    }
     const int j0 = (int)(b0 - (long long)row * a.nblk);
     const int j1 = (int)((long long)j0 + (b1 - b0) < a.nblk ? (long long)j0 + (b1 - b0) : a.nblk);
     b0 += j1 - j0;
@@ -318,6 +337,10 @@ constexpr size_t stats_smem_bytes() {
          sizeof(float) * 2 * Core4k::N + 32;
 }
 
+// ROWS: statistics per row.  A CTA's run of frames may cross row boundaries: its register sums are written out and
+// cleared whenever the row changes, one partial per (CTA, row) segment at slot CTA + row (as k_segment_sumsq indexes
+// the residual partials), and k_reduce_stats_rows adds a row's slots in a fixed order.
+template <bool ROWS>
 __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) {
   using C = Core4k;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -361,6 +384,21 @@ __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) 
       bulk_g2s(stage + C::N, a.y + (size_t)row * a.T + base, bytes, mbar);
     } else {
       mbar_arrive(mbar);
+    }
+  };
+  auto flush = [&](long long slot) {
+    float* out = a.partial + (size_t)slot * 3 * C::F;
+#pragma unroll
+    for (int k3 = 0; k3 < 8; ++k3) {
+      const int k = C::bin_of(t, k3);
+      out[k] = 0.25f * sa[k3];
+      out[C::F + k] = 0.25f * sb[k3];
+      out[2 * C::F + k] = 0.25f * sc[k3];
+    }
+    if (t == 0) {
+      out[2048] = 0.25f * na;
+      out[C::F + 2048] = 0.25f * nb;
+      out[2 * C::F + 2048] = 0.25f * nc;
     }
   };
   if (t == 0 && g0 < g1) issue(g0);
@@ -414,19 +452,34 @@ __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) 
       const float sx = 4.f * z[8].x * z[8].x, sy = 4.f * z[8].y * z[8].y;
       na += sx; nb += sqrtf(sx * sy); nc += sy;
     }
-  }
-  float* out = a.partial + (size_t)blockIdx.x * 3 * C::F;
+    if (ROWS && (g + 1 == g1 || (g + 1) % a.frames == 0)) {    // last frame of the run or of its row
+      flush(blockIdx.x + (int)(g / a.frames));
 #pragma unroll
-  for (int k3 = 0; k3 < 8; ++k3) {
-    const int k = C::bin_of(t, k3);
-    out[k] = 0.25f * sa[k3];
-    out[C::F + k] = 0.25f * sb[k3];
-    out[2 * C::F + k] = 0.25f * sc[k3];
+      for (int i = 0; i < 8; ++i) { sa[i] = 0.f; sb[i] = 0.f; sc[i] = 0.f; }
+      na = nb = nc = 0.f;
+    }
   }
-  if (t == 0) {
-    out[2048] = 0.25f * na;
-    out[C::F + 2048] = 0.25f * nb;
-    out[2 * C::F + 2048] = 0.25f * nc;
+  if (!ROWS) flush(blockIdx.x);
+}
+
+// abc[row][i] = sum of the row's segment partials (slots g + row of the CTAs g whose run touches the row); the same
+// 8-slice fixed-order sum as k_reduce_stats, so one row alone gives k_reduce_stats' result bit for bit
+__global__ void __launch_bounds__(256) k_reduce_stats_rows(const float* partial, int frames, int q, int n, double* abc) {
+  __shared__ double sl[8][33];
+  const int row = blockIdx.y;
+  const int o = threadIdx.x & 31, sidx = threadIdx.x >> 5;
+  const int i = blockIdx.x * 32 + o;
+  const long long g_lo = ((long long)row * frames) / q, g_hi = ((long long)(row + 1) * frames - 1) / q;
+  double s = 0.0;
+  if (i < n)
+    for (long long g = g_lo + sidx; g <= g_hi; g += 8) s += (double)partial[(size_t)(g + row) * n + i];
+  sl[sidx][o] = s;
+  __syncthreads();
+  if (sidx == 0 && i < n) {
+    double t = 0.0;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) t += sl[k][o];
+    abc[(size_t)row * n + i] = t;
   }
 }
 
@@ -569,12 +622,12 @@ static int fused_run_length(int B, int nblk) {
   return (int)q;
 }
 
-template <bool ADJ, int EPI>
+template <bool ADJ, int EPI, bool ROWS>
 static int launch_epi(FusedArgs a, cudaStream_t st) {
   const long long total = (long long)a.B * a.nblk;
   const int grid = (int)((total + a.q - 1) / a.q);
   constexpr size_t smem = fused_smem_bytes<EPI == 1 || EPI == 3>();
-  auto kern = k_filter_fused<ADJ, EPI>;
+  auto kern = k_filter_fused<ADJ, EPI, ROWS>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   kern<<<grid, 256, smem, st>>>(a);
   return check_launch("k_filter_fused");
@@ -592,21 +645,25 @@ size_t fused_sumsq_slots(int B, int T) {
   return (size_t)((total + q - 1) / q) + (size_t)B;
 }
 
+template <bool ROWS>
+static int launch_variant(const FusedArgs& a, cudaStream_t st) {
+  const bool sub = a.sub != nullptr, sc = a.row_scale != nullptr, ss = a.item_sumsq != nullptr;
+  if (a.adjoint) {
+    if (!sub && !sc && !ss) return launch_epi<true, 0, ROWS>(a, st);
+    if (!sub && sc && !ss) return launch_epi<true, 2, ROWS>(a, st);
+    return launch_epi<true, 3, ROWS>(a, st);
+  }
+  if (!sub && !sc && !ss) return launch_epi<false, 0, ROWS>(a, st);
+  if (sub && !sc && ss) return launch_epi<false, 1, ROWS>(a, st);
+  return launch_epi<false, 3, ROWS>(a, st);
+}
+
 int launch_filter_fused(FusedArgs a, double* row_sumsq, cudaStream_t st) {
   a.frames = 1 + a.T / Core4k::HOP;
   a.nblk = (a.T - 1) / Core4k::HOP + 1;
   a.q = fused_run_length(a.B, a.nblk);
-  const bool sub = a.sub != nullptr, sc = a.row_scale != nullptr, ss = a.item_sumsq != nullptr;
-  int rc;
-  if (a.adjoint) {
-    if (!sub && !sc && !ss) rc = launch_epi<true, 0>(a, st);
-    else if (!sub && sc && !ss) rc = launch_epi<true, 2>(a, st);
-    else rc = launch_epi<true, 3>(a, st);
-  } else {
-    if (!sub && !sc && !ss) rc = launch_epi<false, 0>(a, st);
-    else if (sub && !sc && ss) rc = launch_epi<false, 1>(a, st);
-    else rc = launch_epi<false, 3>(a, st);
-  }
+  const bool ss = a.item_sumsq != nullptr;
+  const int rc = a.per_row ? launch_variant<true>(a, st) : launch_variant<false>(a, st);
   if (rc || !ss) return rc;
   k_segment_sumsq<<<a.B, 1, 0, st>>>(a.item_sumsq, a.nblk, a.q, row_sumsq);
   return check_launch("k_segment_sumsq");
@@ -617,19 +674,46 @@ bool fused_stats_eligible(const float* x, const float* y, int T, int mode) {
   return g_fused_variant >= 0 && mode == 0 && (T % 4 == 0) && al(x) && al(y);
 }
 
-int launch_stats_fused(FusedStatsArgs a, int* n_partials, cudaStream_t st) {
-  a.frames = 1 + a.T / Core4k::HOP;
-  const long long total = (long long)a.B * a.frames;
+static int stats_run_length(int B, int frames) {
+  const long long total = (long long)B * frames;
   const long long ctas = 2LL * sm_count();
   long long q = (total + ctas - 1) / ctas;
   if (q < 1) q = 1;
-  a.q = (int)q;
-  const int grid = (int)((total + q - 1) / q);
+  return (int)q;
+}
+
+int launch_stats_fused(FusedStatsArgs a, int* n_partials, cudaStream_t st) {
+  a.frames = 1 + a.T / Core4k::HOP;
+  const long long total = (long long)a.B * a.frames;
+  a.q = stats_run_length(a.B, a.frames);
+  const int grid = (int)((total + a.q - 1) / a.q);
   *n_partials = grid;
   constexpr size_t smem = stats_smem_bytes();
-  cudaFuncSetAttribute(k_stats_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  k_stats_fused<<<grid, 256, smem, st>>>(a);
+  cudaFuncSetAttribute(k_stats_fused<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  k_stats_fused<false><<<grid, 256, smem, st>>>(a);
   return check_launch("k_stats_fused");
+}
+
+size_t fused_stats_rows_slots(int B, int T) {
+  const int frames = 1 + T / Core4k::HOP;
+  const long long total = (long long)B * frames;
+  const int q = stats_run_length(B, frames);
+  return (size_t)((total + q - 1) / q) + (size_t)B;
+}
+
+int launch_stats_rows_fused(FusedStatsArgs a, double* abc, cudaStream_t st) {
+  a.frames = 1 + a.T / Core4k::HOP;
+  const long long total = (long long)a.B * a.frames;
+  a.q = stats_run_length(a.B, a.frames);
+  const int grid = (int)((total + a.q - 1) / a.q);
+  constexpr size_t smem = stats_smem_bytes();
+  cudaFuncSetAttribute(k_stats_fused<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  k_stats_fused<true><<<grid, 256, smem, st>>>(a);
+  int rc = check_launch("k_stats_fused");
+  if (rc) return rc;
+  const int n = 3 * Core4k::F;
+  k_reduce_stats_rows<<<dim3((n + 31) / 32, a.B), 256, 0, st>>>(a.partial, a.frames, a.q, n, abc);
+  return check_launch("k_reduce_stats_rows");
 }
 
 bool fused_fir_eligible(const float* x, int T) {

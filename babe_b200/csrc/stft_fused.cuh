@@ -14,6 +14,7 @@ struct FusedArgs {
   const float* sub; const float* row_scale; double* item_sumsq;
   int* status;
   int q, nblk, frames;                                  // filled by the launcher (q: output blocks per CTA)
+  int per_row;                                          // 1: fc, A are [B, K], status is int[B] (one filter per row)
 };
 
 // rows can be bulk-copied: T % 4 == 0 and a 16-byte aligned base
@@ -30,6 +31,9 @@ struct FusedStatsArgs {
 bool fused_stats_eligible(const float* x, const float* y, int T, int mode);
 // launches k_stats_fused; *n_partials = rows of `partial` written (<= 2 * SM count)
 int launch_stats_fused(FusedStatsArgs a, int* n_partials, cudaStream_t st);
+// per-row statistics: abc[B][3][F]; `partial` needs fused_stats_rows_slots(B, T) rows of 3 F floats
+size_t fused_stats_rows_slots(int B, int T);
+int launch_stats_rows_fused(FusedStatsArgs a, double* abc, cudaStream_t st);
 
 struct FusedFirArgs {
   const float* x; float* y; int B, T;

@@ -957,3 +957,78 @@ extern "C" int babe_fir_filter(const float* x, float* y, int B, int T, const flo
   k_fir_filter<Core3><<<grid, Core3::TPF, smem, static_cast<cudaStream_t>(stream)>>>(a);
   return check_launch("k_fir_filter");
 }
+
+// ---------------------------------------------------------------------------
+// one filter per row.  NFFT = 4096 rows that can be bulk-copied take the per-row instantiations of the fused
+// kernels (stft_fused.cu); every other case (NFFT 512 / 1024 / 2048, rows that cannot be bulk-copied,
+// babe_set_fused_variant(-1)) runs the shared-filter entry point once per row on pointer offsets, which gives each
+// row its B = 1 result by construction.
+// ---------------------------------------------------------------------------
+extern "C" int babe_apply_filter_rows(const float* x, float* y, int B, int T, int nfft,
+                                      const float* window, const float* twiddle,
+                                      const float* freqs, const float* fc, const float* A, int K,
+                                      int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
+                                      void* workspace, size_t workspace_bytes, int* status, void* stream) {
+  BABE_REQUIRE(x && y && window && twiddle, BABE_EBADARG, "apply_filter_rows: null pointer");
+  BABE_REQUIRE(B >= 0 && T >= 0, BABE_EBADARG, "apply_filter_rows: bad shape B=%d T=%d", B, T);
+  BABE_REQUIRE(freqs && fc && A && K >= 1 && K <= BABE_MAX_BREAKPOINTS, BABE_EBADARG,
+               "apply_filter_rows: need (freqs, fc, A, 1<=K<=%d)", BABE_MAX_BREAKPOINTS);
+  BABE_REQUIRE(babe_stft_supported(nfft), BABE_EUNSUPPORTED, "unsupported NFFT %d", nfft);
+  if (B == 0 || T == 0) return BABE_OK;
+  const float* sub_ = adjoint ? nullptr : sub;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (nfft == 4096 && fused_filter_eligible(x, sub_, T)) {
+    FusedArgs f{};
+    f.x = x; f.y = y; f.B = B; f.T = T; f.window = window; f.roots = reinterpret_cast<const float2*>(twiddle);
+    f.freqs = freqs; f.fc = fc; f.A = A; f.K = K; f.adjoint = adjoint;
+    f.sub = sub_; f.row_scale = row_scale; f.status = status; f.per_row = 1;
+    if (row_sumsq != nullptr) {
+      BABE_REQUIRE(workspace != nullptr && workspace_bytes >= fused_sumsq_slots(B, T) * sizeof(double), BABE_EBADARG,
+                   "apply_filter_rows: row_sumsq needs a workspace of babe_apply_filter_workspace() bytes");
+      f.item_sumsq = static_cast<double*>(workspace);
+    }
+    return launch_filter_fused(f, row_sumsq, st);
+  }
+  for (int b = 0; b < B; ++b) {
+    const size_t o = (size_t)b * T;
+    const int rc = babe_apply_filter(x + o, y + o, 1, T, nfft, window, twiddle, nullptr, freqs, fc + (size_t)b * K,
+                                     A + (size_t)b * K, K, adjoint, sub_ ? sub_ + o : nullptr,
+                                     row_scale ? row_scale + b : nullptr, row_sumsq ? row_sumsq + b : nullptr,
+                                     workspace, workspace_bytes, status ? status + b : nullptr, stream);
+    if (rc) return rc;
+  }
+  return BABE_OK;
+}
+
+extern "C" size_t babe_stft_stats_rows_workspace(int B, int T, int nfft) {
+  if (!babe_stft_supported(nfft) || B < 1 || T < 1) return 0;
+  const size_t fallback = babe_stft_stats_workspace(1, T, nfft);
+  if (nfft != 4096) return fallback;
+  return std::max(fallback, fused_stats_rows_slots(B, T) * 3 * Core3::F * sizeof(float));
+}
+
+extern "C" int babe_stft_stats_rows(const float* x, const float* y, int B, int T, int nfft,
+                                    const float* window, const float* twiddle,
+                                    double* abc, void* workspace, size_t workspace_bytes, void* stream) {
+  BABE_REQUIRE(x && y && window && twiddle && abc, BABE_EBADARG, "stft_stats_rows: null pointer");
+  BABE_REQUIRE(B >= 1 && T >= 1, BABE_EBADARG, "stft_stats_rows: bad shape B=%d T=%d", B, T);
+  BABE_REQUIRE(babe_stft_supported(nfft), BABE_EUNSUPPORTED, "unsupported NFFT %d", nfft);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (nfft == 4096 && fused_stats_eligible(x, y, T, 0)) {
+    const size_t need = fused_stats_rows_slots(B, T) * 3 * Core3::F * sizeof(float);
+    BABE_REQUIRE(workspace != nullptr && workspace_bytes >= need, BABE_EBADARG,
+                 "stft_stats_rows: workspace too small (%zu < %zu)", workspace_bytes, need);
+    FusedStatsArgs f{};
+    f.x = x; f.y = y; f.B = B; f.T = T; f.window = window; f.roots = reinterpret_cast<const float2*>(twiddle);
+    f.partial = static_cast<float*>(workspace);
+    return launch_stats_rows_fused(f, abc, st);
+  }
+  const int F = nfft / 2 + 1;
+  for (int b = 0; b < B; ++b) {
+    const size_t o = (size_t)b * T;
+    const int rc = babe_stft_stats(x + o, y + o, 1, T, nfft, window, twiddle, 0, abc + (size_t)b * 3 * F,
+                                   workspace, workspace_bytes, stream);
+    if (rc) return rc;
+  }
+  return BABE_OK;
+}

@@ -139,6 +139,56 @@ def apply_filter(x, nfft, H=None, freqs=None, fc=None, A=None, adjoint=False, su
     return y
 
 
+def _row_params(x, fc, A):
+    """Shape checks of the per-row filter parameters: fc, A (B, K) with the B of x (B, T)."""
+    if not (torch.is_tensor(x) and torch.is_tensor(fc) and torch.is_tensor(A)):
+        raise TypeError("x, fc and A must be tensors")
+    if x.dim() != 2:
+        raise ValueError("x must be (B, T)")
+    if fc.dim() != 2 or A.shape != fc.shape or fc.shape[0] != x.shape[0]:
+        raise ValueError(f"fc and A must both be (B, K) with B = {x.shape[0]} rows of x, got "
+                         f"{tuple(fc.shape)} and {tuple(A.shape)}")
+
+
+def apply_filter_rows(x, nfft, freqs, fc, A, adjoint=False, sub=None, row_scale=None, row_sumsq=None, out=None,
+                      status=None):
+    """``apply_filter`` with one filter per row: row b of x[B,T] goes through the H designed from fc[b], A[b]
+    (fc, A: (B, K)).  ``status`` (optional int32[B]) flags the rows whose design the reference would reject."""
+    _row_params(x, fc, A)
+    x = _cuda_f32(x, "x")
+    fc = _cuda_f32(fc, "fc")
+    A = _cuda_f32(A, "A")
+    freqs = _cuda_f32(freqs, "f")
+    B, T = x.shape
+    K = fc.shape[1]
+    if freqs.numel() != nfft // 2 + 1:
+        raise ValueError(f"freqs must have {nfft // 2 + 1} bins, got {freqs.numel()}")
+    win, tw = stft_tables(nfft, x.device)
+    if sub is not None:
+        sub = _cuda_f32(sub, "sub")
+        if sub.shape != x.shape:
+            raise ValueError("sub must match x")
+    if row_scale is not None:
+        row_scale = _cuda_f32(row_scale, "row_scale")
+        if row_scale.numel() != B:
+            raise ValueError("row_scale must have B entries")
+    if row_sumsq is not None and (row_sumsq.dtype != torch.float64 or row_sumsq.numel() != B):
+        raise ValueError("row_sumsq must be float64[B]")
+    if status is not None and (status.dtype != torch.int32 or status.numel() != B):
+        raise ValueError("status must be int32[B]")
+    y = torch.empty_like(x) if out is None else out
+    ws, nbytes = None, 0
+    if row_sumsq is not None:
+        nbytes = lib().babe_apply_filter_workspace(B, T, int(nfft))
+        ws = torch.empty(nbytes // 8, dtype=torch.float64, device=x.device)
+    with profiling.op("apply_filter_rows_adj" if adjoint else "apply_filter_rows",
+                      2 if row_sumsq is not None else 1, (12 if sub is not None else 8) * B * T):
+        check(lib().babe_apply_filter_rows(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), _p(freqs), _p(fc), _p(A),
+                                           K, int(bool(adjoint)), _p(sub), _p(row_scale), _p(row_sumsq), _p(ws),
+                                           nbytes, _p(status), _stream()), "apply_filter_rows")
+    return y
+
+
 def stft(x, nfft, frames=0, in_env_div=False, bin_scale=None):
     x = _cuda_f32(x, "x")
     B, T = x.shape
@@ -186,6 +236,26 @@ def stft_stats(x, y, nfft, mode=0):
     with profiling.op("stft_stats", 2, 8 * B * T):
         check(lib().babe_stft_stats(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), int(mode), _p(abc),
                                     _p(ws), nbytes, _stream()), "stft_stats")
+    return abc
+
+
+def stft_stats_rows(x, y, nfft):
+    """float64[B,3,F]: ``stft_stats`` (mode 0) of every row on its own."""
+    if not (torch.is_tensor(x) and torch.is_tensor(y)):
+        raise TypeError("x and y must be tensors")
+    if x.shape != y.shape or x.dim() != 2:
+        raise ValueError("x and y must both be (B, T)")
+    x = _cuda_f32(x, "x")
+    y = _cuda_f32(y, "y")
+    B, T = x.shape
+    win, tw = stft_tables(nfft, x.device)
+    F = nfft // 2 + 1
+    nbytes = lib().babe_stft_stats_rows_workspace(B, T, int(nfft))
+    ws = torch.empty(nbytes // 4, dtype=torch.float32, device=x.device)
+    abc = torch.empty(B, 3, F, dtype=torch.float64, device=x.device)
+    with profiling.op("stft_stats_rows", 2, 8 * B * T):
+        check(lib().babe_stft_stats_rows(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), _p(abc), _p(ws), nbytes,
+                                         _stream()), "stft_stats_rows")
     return abc
 
 
@@ -268,6 +338,36 @@ def fit_params(abc, w, freqs, params, cfg, return_iters=False):
     with profiling.op("fit_params", 1, 3 * F * 8):
         check(lib().babe_fit_params(_p(abc), _p(w), _p(freqs), F, _p(params), params.shape[1],
                                     ctypes.byref(cfg), _p(iters), _stream()), "fit_params")
+    return (params, iters) if return_iters else params
+
+
+def fit_params_rows(abc, w, freqs, params, cfg, return_iters=False):
+    """``fit_params`` on every row on its own, IN PLACE on params[B,2,K] from abc[B,3,F] (``stft_stats_rows``);
+    with ``return_iters`` also the int32[B] iteration counts."""
+    if not (torch.is_tensor(abc) and torch.is_tensor(params)):
+        raise TypeError("abc and params must be tensors")
+    if params.dim() != 3 or params.shape[1] != 2:
+        raise ValueError(f"params must be (B, 2, K), got {tuple(params.shape)}")
+    if abc.dim() != 3 or abc.shape[0] != params.shape[0] or abc.shape[1] != 3:
+        raise ValueError(f"abc must be (B, 3, F) with B = {params.shape[0]}, got {tuple(abc.shape)}")
+    if not (abc.is_cuda and params.is_cuda):
+        raise BabeError("abc and params must be CUDA tensors: babe_b200 runs on CUDA tensors only "
+                        "(there is no CPU fallback)")
+    if abc.dtype != torch.float64:
+        raise TypeError("abc must be a CUDA float64 tensor")
+    if not (params.dtype == torch.float32 and params.is_contiguous()):
+        raise TypeError("params must be a contiguous CUDA float32 tensor of shape (B, 2, K)")
+    w = _cuda_f32(w, "w")
+    freqs = _cuda_f32(freqs, "f")
+    F = freqs.numel()
+    if abc.shape[2] != F:
+        raise ValueError(f"abc has {abc.shape[2]} bins, freqs {F}")
+    B, K = params.shape[0], params.shape[2]
+    abc = abc.contiguous()
+    iters = torch.zeros(B, dtype=torch.int32, device=params.device) if return_iters else None
+    with profiling.op("fit_params_rows", 1, 3 * F * 8 * B):
+        check(lib().babe_fit_params_rows(_p(abc), _p(w), _p(freqs), F, _p(params), B, K, ctypes.byref(cfg),
+                                         _p(iters), _stream()), "fit_params_rows")
     return (params, iters) if return_iters else params
 
 

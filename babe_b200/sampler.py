@@ -17,6 +17,11 @@ purely in execution:
 * noise may be drawn on the device (``device_noise=True``); the default keeps
   the reference's host generator stream so that outputs are comparable for a
   fixed ``torch.manual_seed``.
+
+One behaviour goes beyond the reference: with ``filter_per_row`` every row of ``y``
+is an independent restoration (its own fit statistics, filter fit, guidance
+filter and guidance normaliser), i.e. row r of one call with B rows is what a
+call on ``y[r:r+1]`` alone returns with the same noise for that row.
 """
 import types
 import warnings
@@ -38,11 +43,12 @@ def _ns(**kw):
 
 def make_args(sample_rate=22050, audio_len=184184, T=35, xi=0.2, start_sigma=0.2,
               NFFT=4096, fc_init=(280, 285, 290, 295, 300), A_init=(-15, -17, -20, -25, -30),
-              max_iter=100, Schurn=20, num_octs=7, bins_per_oct=64, **extra):
+              max_iter=100, Schurn=20, num_octs=7, bins_per_oct=64, filter_per_row=False, **extra):
     """Nested attribute namespace carrying exactly the fields the sampler, EDM
     and the CQTDiff+ constructor read, with the values of
     conf/tester/blind_bwe.yaml, conf/exp/maestro22k_8s.yaml,
-    conf/diff_params/edm.yaml and conf/network/cqtdiff+.yaml."""
+    conf/diff_params/edm.yaml and conf/network/cqtdiff+.yaml.  ``filter_per_row`` sets
+    ``tester.blind_bwe.filter_per_row`` (one filter estimate per row, see ``BlindSamplerFused``)."""
     args = _ns(
         exp=_ns(sample_rate=sample_rate, audio_len=audio_len, seed=42),
         diff_params=_ns(callable="babe_b200.edm.EDM", sigma_data=0.063, sigma_min=1e-5,
@@ -68,7 +74,7 @@ def make_args(sample_rate=22050, audio_len=184184, T=35, xi=0.2, start_sigma=0.2
                                    stft_distance=_ns(use=False, mag=False, use_multires=False,
                                                      nfft=2048, logmag=False)),
             blind_bwe=_ns(fcmin=20, fcmax="nyquist", Amin=-50, Amax=30, NFFT=NFFT,
-                          sigma_den_estimate=0.0,
+                          sigma_den_estimate=0.0, filter_per_row=bool(filter_per_row),
                           test_filter=_ns(fc=[1000], A=[-20]),
                           initial_conditions=_ns(fc=list(fc_init), A=list(A_init)),
                           optimization=_ns(max_iter=max_iter, tol=[5e-3, 5e-3], mu=[1000, 10],
@@ -101,6 +107,7 @@ class FilterFit:
         w = bu.freq_weight_vector(freq_weighting, self.nfft // 2 + 1, device)
         self.w = w if w is not None else torch.ones(self.nfft // 2 + 1, device=device)
         self.joint = False
+        self.per_row = False           # True: params (B, 2, K), one fit per row on that row's statistics
 
     @classmethod
     def from_args(cls, args, device):
@@ -116,13 +123,17 @@ class FilterFit:
                 c.clamp_fc, c.clamp_A, c.only_negative_A)
 
     def stats(self, x_den, y):
+        if self.per_row:
+            return ops.stft_stats_rows(x_den, y, self.nfft)
         return ops.stft_stats(x_den, y, self.nfft, mode=0)
 
     def __call__(self, x_den, y, params, return_iters=False, abc=None):
         """params (2,K) is updated in place (the reference also mutates it,
-        testing/blind_bwe_sampler.py:577-583) and returned."""
+        testing/blind_bwe_sampler.py:577-583) and returned; (B,2,K) per row with ``per_row``."""
         if abc is None:
             abc = self.stats(x_den, y)
+        if self.per_row:
+            return ops.fit_params_rows(abc, self.w, self.freqs, params, self.cfg, return_iters=return_iters)
         if self.joint:                 # one filter for the rows of ALL ranks (SURVEY 8e)
             from . import distributed
             distributed.sum_over_ranks_(abc)
@@ -135,12 +146,15 @@ class FilterFit:
 class _RecGuidanceNorm(torch.autograd.Function):
     """norm_b = || y_b - A_{fc,A}(x_b) ||_2  (testing/blind_bwe_sampler.py:89,117)
     with backward  g_b * A^T((A x_b - y_b) / norm_b)  (what :120 back-propagates
-    into the denoiser).  H is designed inside both kernels."""
+    into the denoiser).  H is designed inside both kernels; fc, A of shape (B, K) give every row its own filter."""
 
     @staticmethod
     def forward(ctx, x, y, freqs, fc, A, nfft):
         ss = torch.zeros(x.shape[0], dtype=torch.float64, device=x.device)
-        r = ops.apply_filter(x, nfft, freqs=freqs, fc=fc, A=A, sub=y, row_sumsq=ss)
+        if fc.dim() == 2:
+            r = ops.apply_filter_rows(x, nfft, freqs, fc, A, sub=y, row_sumsq=ss)
+        else:
+            r = ops.apply_filter(x, nfft, freqs=freqs, fc=fc, A=A, sub=y, row_sumsq=ss)
         norms = torch.sqrt(ss).to(torch.float32)
         ctx.save_for_backward(r, norms, freqs, fc, A)
         ctx.nfft = nfft
@@ -151,13 +165,17 @@ class _RecGuidanceNorm(torch.autograd.Function):
     def backward(ctx, g):
         r, norms, freqs, fc, A = ctx.saved_tensors
         scale = (g / norms).contiguous()
-        gx = ops.apply_filter(r, ctx.nfft, freqs=freqs, fc=fc, A=A, adjoint=True, row_scale=scale)
+        if fc.dim() == 2:
+            gx = ops.apply_filter_rows(r, ctx.nfft, freqs, fc, A, adjoint=True, row_scale=scale)
+        else:
+            gx = ops.apply_filter(r, ctx.nfft, freqs=freqs, fc=fc, A=A, adjoint=True, row_scale=scale)
         return gx, None, None, None, None, None
 
 
 def rec_guidance_norms(x, y, freqs, filter_params, nfft):
-    return _RecGuidanceNorm.apply(x, y, freqs, filter_params[0].contiguous(),
-                                  filter_params[1].contiguous(), int(nfft))
+    """filter_params (2, K): one filter for all rows; (B, 2, K): row b filtered with filter_params[b]."""
+    fc, A = (filter_params[:, 0], filter_params[:, 1]) if filter_params.dim() == 3 else filter_params
+    return _RecGuidanceNorm.apply(x, y, freqs, fc.contiguous(), A.contiguous(), int(nfft))
 
 
 _PINNED_NOISE = {}
@@ -197,6 +215,9 @@ class BlindSamplerFused:
         self.generator = None          # optional torch.Generator for device noise
         self.noise_fn = None           # optional callable(shape, device) -> tensor (benchmarks, parity runs)
         self.joint = False             # True: ranks reproduce ONE reference call on the whole batch
+        # True: every row of y is an independent restoration (own filter estimate and guidance scale); Hydra-style
+        # configs switch it on with tester.blind_bwe.filter_per_row
+        self.filter_per_row = bool(getattr(args.tester.blind_bwe, "filter_per_row", False))
         self._fit = None
 
     def update_diff_params(self):
@@ -290,7 +311,11 @@ class BlindSamplerFused:
         return net
 
     def apply_filter_fcA(self, x, filter_params):
-        """testing/blind_bwe_sampler.py:518-520, H designed inside the kernel."""
+        """testing/blind_bwe_sampler.py:518-520, H designed inside the kernel; filter_params (B, 2, K) filters
+        row b with filter_params[b]."""
+        if filter_params.dim() == 3:
+            return bu.apply_filter_rows(x, self.freqs, filter_params[:, 0], filter_params[:, 1],
+                                        self.args.tester.blind_bwe.NFFT)
         H = bu.design_filter(filter_params[0], filter_params[1], self.freqs)
         return bu.apply_filter(x, H, self.args.tester.blind_bwe.NFFT)
 
@@ -337,7 +362,9 @@ class BlindSamplerFused:
             else:
                 norm = torch.linalg.norm(y - den_rec, dim=1, ord=ps.norm)
         (rec_grads,) = torch.autograd.grad(outputs=norm.sum(), inputs=x)
-        if self.joint:                 # Frobenius norm over the rows of ALL ranks (:125)
+        if self.filter_per_row:        # each row is its own restoration: its own normaliser
+            normguide = torch.linalg.norm(rec_grads, dim=1, keepdim=True) / self.args.exp.audio_len ** 0.5
+        elif self.joint:               # Frobenius norm over the rows of ALL ranks (:125)
             from . import distributed
             sq = (rec_grads.double() ** 2).sum().reshape(1)
             normguide = torch.sqrt(distributed.sum_over_ranks_(sq))[0].float() / self.args.exp.audio_len ** 0.5
@@ -364,6 +391,21 @@ class BlindSamplerFused:
             x_den_3 = self.data_consistency_step_classic(x_den_3, y, filter_params)
             score = (x_den_3 - x_in) / t_in ** 2
         return score, filter_params, x_den_2
+
+    def _check_per_row(self, compute_sweep):
+        """Modes that cannot run with one filter per row."""
+        if self.joint:
+            raise ValueError("filter_per_row and joint exclude each other: joint shares ONE filter over all rows "
+                             "of all ranks, filter_per_row gives every row its own")
+        sd = self.args.tester.posterior_sampling.stft_distance
+        if sd.use:
+            raise NotImplementedError("filter_per_row with the STFT-distance guidance: its norm is one sum over the "
+                                      "whole batch, not a per-row quantity" if not sd.use_multires else
+                                      "filter_per_row with use_multires: the multi-resolution STFT distance is a "
+                                      "batch-wide norm (and dead code in the reference)")
+        if compute_sweep:
+            raise NotImplementedError("filter_per_row with compute_sweep: the sweep evaluates one loss surface on "
+                                      "the statistics of the whole batch")
 
     def compute_sweep(self, denoised_estimate, y):
         """testing/blind_bwe_sampler.py:598-616 on the collapsed statistics."""
@@ -400,7 +442,7 @@ class BlindSamplerFused:
 
     def _step_graph_for(self, y, filter_params, heun):
         """Capture (once per shape / variant) and return the replayable step."""
-        key = (tuple(y.shape), y.device, tuple(filter_params.shape), self._fit.cfg_key())
+        key = (tuple(y.shape), y.device, tuple(filter_params.shape), self.filter_per_row, self._fit.cfg_key())
         if self._step_key != key:
             self._step_key, self._step_graphs = key, {}
         if heun in self._step_graphs:
@@ -454,12 +496,19 @@ class BlindSamplerFused:
         """testing/blind_bwe_sampler.py:619-769.  ``max_steps`` bounds the loop
         (benchmarks); ``step_hook(i, x, filter_params)`` is called after each
         step.  ``start_step`` / ``init_x`` / ``init_params`` resume the loop from a given state
-        (teacher-forced parity tests: one step from each state of a reference run)."""
+        (teacher-forced parity tests: one step from each state of a reference run).
+
+        With ``filter_per_row`` the rows of y are independent restorations: the returned filter is (B, 2, K),
+        ``init_params`` may be (2, K) (every row) or (B, 2, K), and with ``rid`` the logged filters are
+        (T, B, 2, K)."""
         args = self.args
+        if self.filter_per_row:
+            self._check_per_row(compute_sweep)
         device = y.device
         self.freqs = torch.fft.rfftfreq(args.tester.blind_bwe.NFFT, d=1 / args.exp.sample_rate).to(device)
         self._fit = FilterFit.from_args(args, device)
         self._fit.joint = self.joint
+        self._fit.per_row = self.filter_per_row
         shape = y.shape
         filter_params = torch.Tensor([args.tester.blind_bwe.initial_conditions.fc,
                                       args.tester.blind_bwe.initial_conditions.A]).to(device)
@@ -467,6 +516,13 @@ class BlindSamplerFused:
             filter_params.unsqueeze_(1)
         if init_params is not None:
             filter_params = init_params.to(device).clone()
+        if self.filter_per_row:
+            if filter_params.dim() == 2:
+                filter_params = filter_params.unsqueeze(0).expand(shape[0], -1, -1)
+            if filter_params.dim() != 3 or filter_params.shape[0] != shape[0]:
+                raise ValueError(f"per-row filter parameters must be (2, K) or ({shape[0]}, 2, K), "
+                                 f"got {tuple(filter_params.shape)}")
+            filter_params = filter_params.contiguous().clone()
         if compute_sweep:
             self.fc_s = torch.logspace(2.5, 4, 15).to(device)
             self.A_s = torch.linspace(-80, -5, 12).to(device)

@@ -59,13 +59,23 @@ def merge(preds, spans, L, ola=256, discard_end=200):
     return out
 
 
-def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, joint=False):
+def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, joint=False, batched=False):
     """Blind restoration of a whole recording, segments sharded over the ranks of the
     current process group.  Returns (final_pred (1, L), filter_data) on every rank,
     ``filter_data`` being the list [((ix0, ix1), filter_params), ...] the reference
     pickles (:466-467,:576-577).  ``joint=True`` processes a rank's segments as one
-    batch and shares ONE filter across all ranks (testing/blind_bwe_tester.py:758-781)."""
+    batch and shares ONE filter across all ranks (testing/blind_bwe_tester.py:758-781).
+
+    ``batched=True`` (with ``joint=False``) restores a rank's segments in ONE sampler call with
+    ``filter_per_row``: every segment still gets its own filter estimate and guidance scale, as in
+    the sequential loop, but the denoiser and the filter kernels run on all of them at once.  The
+    noise is drawn for the whole batch at each step, so the host noise stream is consumed in a
+    different order than by the loop of B = 1 calls: the two restorations agree statistically,
+    not bitwise (they agree to rounding when every segment gets the same noise either way, e.g.
+    through ``sampler.noise_fn``)."""
     import torch.distributed as dist
+    if joint and batched:
+        raise ValueError("batched=True restores every segment with its own filter; joint=True shares one")
     rank = dist.get_rank() if dist.is_initialized() else 0
     world = dist.get_world_size() if dist.is_initialized() else 1
     segs, spans = split(degraded, seg_len, ola, discard_end)
@@ -78,6 +88,13 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
         sampler.joint = True
         pred, filt = sampler.predict_blind_bwe(mine, rid=False)
         filts = filt.unsqueeze(0).expand(mine.shape[0], -1, -1).contiguous()
+    elif batched:
+        was = sampler.filter_per_row
+        sampler.filter_per_row = True
+        try:
+            pred, filts = sampler.predict_blind_bwe(mine.clone(), rid=False)
+        finally:
+            sampler.filter_per_row = was
     else:
         preds, fl = [], []
         for s in range(mine.shape[0]):

@@ -116,6 +116,18 @@ int babe_apply_filter(const float* x, float* y, int B, int T, int nfft,
                       int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
                       void* workspace, size_t workspace_bytes, int* status, void* stream);
 
+/* One filter per row: the same operator with fc[B,K], A[B,K] (row b filtered by the H designed from
+ * fc[b], A[b]) and status int[B] (status[b] set like babe_design_filter's for row b).  Epilogues and workspace
+ * as above.  Every row's output equals babe_apply_filter on that row alone with its own (fc, A).  NFFT 4096 rows
+ * that can be bulk-copied run the per-row variant of the fused kernel (H redesigned where a CTA's run of blocks
+ * enters a new row); NFFT 512 / 1024 / 2048, other rows and babe_set_fused_variant(-1) call babe_apply_filter
+ * once per row. */
+int babe_apply_filter_rows(const float* x, float* y, int B, int T, int nfft,
+                           const float* window, const float* twiddle,
+                           const float* freqs, const float* fc, const float* A, int K,
+                           int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
+                           void* workspace, size_t workspace_bytes, int* status, void* stream);
+
 /* ---- a1: STFT, a2: filter + iSTFT (unfused signatures) ------------------ */
 /* apply_stft (utils/blind_bwe_utils.py:15-26): x[B,T] -> X[B,F,frames,2].
  * frames = 0 means the reference's 1 + T/(nfft/2) (x is treated as right
@@ -155,6 +167,15 @@ size_t babe_stft_stats_workspace(int B, int T, int nfft);
 int babe_stft_stats(const float* x, const float* y, int B, int T, int nfft,
                     const float* window, const float* twiddle, int mode,
                     double* abc, void* workspace, size_t workspace_bytes, void* stream);
+/* Mode-0 statistics per row: abc is double[B,3F], row b's block is what babe_stft_stats gives for row b
+ * alone.  NFFT 4096 rows that can be bulk-copied: one launch of the fused statistics kernel with one partial
+ * per (CTA, row) segment and a fixed-order fp64 reduction per row (deterministic; a row's result does not
+ * depend on the other rows); otherwise babe_stft_stats once per row.  workspace:
+ * babe_stft_stats_rows_workspace() bytes. */
+size_t babe_stft_stats_rows_workspace(int B, int T, int nfft);
+int babe_stft_stats_rows(const float* x, const float* y, int B, int T, int nfft,
+                         const float* window, const float* twiddle,
+                         double* abc, void* workspace, size_t workspace_bytes, void* stream);
 /* Same statistics from precomputed spectrograms X, Xref [B,F,frames,2] as the
  * reference signature apply_filter_and_norm_STFTmag_fweighted(X, Xref, H, w)
  * (utils/blind_bwe_utils.py:250-296) receives them.  out is double[4F]:
@@ -201,6 +222,13 @@ int babe_set_fit_variant(int variant);
 int babe_fit_params(const double* abc, const float* w, const float* freqs, int F,
                     float* params, int K, const babe_fit_config* cfg_host,
                     int* iters_out, void* stream);
+/* B independent fits: abc[B,3F] (babe_stft_stats_rows), params[B,2,K] updated in place, iters_out int[B]
+ * (optional); clamps and the stopping test apply per row.  Row b's result is bitwise what babe_fit_params gives
+ * on abc[b], params[b].  Fit variant 0 with K <= 8 and F <= 4096 launches B clusters of k_fit_params3 (cluster b
+ * fits row b); the other variants and sizes call babe_fit_params once per row. */
+int babe_fit_params_rows(const double* abc, const float* w, const float* freqs, int F,
+                         float* params, int B, int K, const babe_fit_config* cfg_host,
+                         int* iters_out, void* stream);
 
 /* ---- a15-a18: NSGT constant-Q transform (cqt_nsgt_pytorch.CQT_nsgt) -------- */
 /* Replaces the third-party class the reference imports at
