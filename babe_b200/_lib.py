@@ -119,6 +119,8 @@ SIGNATURES = {
                                   c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "babe_cqt_synthesis": (c_int, [POINTER(CqtPlan), POINTER(c_void_p), c_int, c_void_p, c_int,
                                    c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "babe_row_noise": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
+                               c_float, c_void_p]),
 }
 
 _lib = None

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbabe_b200.so")
-SOURCES = ["api.cu", "stft_ops.cu", "stft_fused.cu", "fit_ops.cu", "cqt_ops.cu", "net_ops.cu"]
+SOURCES = ["api.cu", "stft_ops.cu", "stft_fused.cu", "fit_ops.cu", "cqt_ops.cu", "net_ops.cu", "row_noise.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

@@ -371,6 +371,60 @@ def fit_params_rows(abc, w, freqs, params, cfg, return_iters=False):
     return (params, iters) if return_iters else params
 
 
+def row_noise(seeds, shape_or_a, draw, slot=0, scale=None, row_scale=None, mult=1.0, out=None):
+    """Keyed standard normal noise, one seed per row (``k_row_noise``, DESIGN.md 4.8):
+    ``out[b, n] = a[b, n] + eps[b, n] * mult * scale * row_scale[b]``, eps[b, n] a function of (seeds[b], draw + slot,
+    n) alone.  ``seeds``: int64 CUDA tensor (B,) (read as uint64).  ``shape_or_a``: (B, T) for the bare noise (a = 0)
+    or the float32 (B, T) tensor a.  ``draw``: draw index, an int or a CUDA int32 tensor of one element (read by the
+    kernel at run time, so a captured graph replays with its current value).  ``scale``: optional CUDA float32 tensor
+    of one element; ``row_scale``: optional CUDA float32 (B,); ``mult``: host float.  ``out`` may be ``a``."""
+    if not torch.is_tensor(seeds):
+        raise TypeError("seeds must be an int64 tensor")
+    if not seeds.is_cuda:
+        raise BabeError(f"seeds is on {seeds.device}: babe_b200 runs on CUDA tensors only (there is no CPU fallback)")
+    if seeds.dtype != torch.int64 or seeds.dim() != 1:
+        raise ValueError(f"seeds must be a 1-D int64 tensor, got {seeds.dtype} of shape {tuple(seeds.shape)}")
+    seeds = seeds.contiguous()
+    dev = seeds.device
+    a = None
+    if torch.is_tensor(shape_or_a):
+        a = _cuda_f32(shape_or_a, "a")
+        shape = tuple(a.shape)
+    else:
+        shape = tuple(int(v) for v in shape_or_a)
+    if len(shape) != 2 or shape[0] != seeds.numel():
+        raise ValueError(f"noise of shape {shape}: must be (B, T) with B = {seeds.numel()} seeds")
+    B, T = shape
+    if torch.is_tensor(draw):
+        if not draw.is_cuda:
+            raise BabeError(f"draw is on {draw.device}: pass an int or a CUDA int32 tensor")
+        if draw.dtype != torch.int32 or draw.numel() != 1:
+            raise ValueError("draw must be an int or a CUDA int32 tensor of one element")
+    else:
+        draw = torch.full((1,), int(draw), dtype=torch.int32, device=dev)
+    if scale is not None:
+        scale = _cuda_f32(scale, "scale")
+        if scale.numel() != 1:
+            raise ValueError("scale must have one element")
+    if row_scale is not None:
+        row_scale = _cuda_f32(row_scale, "row_scale")
+        if row_scale.numel() != B:
+            raise ValueError(f"row_scale must have B = {B} entries, got {row_scale.numel()}")
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float32, device=dev)
+    else:
+        _cuda_f32(out, "out")
+        if tuple(out.shape) != shape or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous float32 tensor of shape {shape}")
+    if slot < 0:
+        raise ValueError("slot must be >= 0")
+    # algorithmic bytes: write the noise (+ read a)
+    with profiling.op("row_noise", 1, (8 if a is not None else 4) * B * T):
+        check(lib().babe_row_noise(_p(out), _p(a), _p(seeds), B, T, _p(draw), int(slot), _p(scale), _p(row_scale),
+                                   float(mult), _stream()), "row_noise")
+    return out
+
+
 # ---------------------------------------------------------------------------
 _FIR_TABLES = {}
 

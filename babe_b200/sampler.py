@@ -16,7 +16,11 @@ purely in execution:
   and H(fc, A) is never written to HBM;
 * noise may be drawn on the device (``device_noise=True``); the default keeps
   the reference's host generator stream so that outputs are comparable for a
-  fixed ``torch.manual_seed``.
+  fixed ``torch.manual_seed``;
+* with ``row_seeds`` (one 64-bit seed per row) every draw is keyed noise generated on
+  the device by ``k_row_noise`` (DESIGN.md 4.8): row r's noise is a function of its seed,
+  the draw index and the sample index alone, so a row restores the same whatever the
+  batch, its position in it or the number of ranks.
 
 One behaviour goes beyond the reference: with ``filter_per_row`` every row of ``y``
 is an independent restoration (its own fit statistics, filter fit, guidance
@@ -214,6 +218,11 @@ class BlindSamplerFused:
         self.device_noise = device_noise
         self.generator = None          # optional torch.Generator for device noise
         self.noise_fn = None           # optional callable(shape, device) -> tensor (benchmarks, parity runs)
+        # one seed per row of the next call (list of ints or an int64 tensor): keyed device noise for every draw,
+        # before device_noise / generator; None: the sources above
+        self.row_seeds = None
+        self._keyed = None             # during a call with row_seeds: the device seeds and the draw-index scalar
+        self._eval_slot = 1            # draw slot of the evaluation running (1: first, 4: Heun correction)
         self.joint = False             # True: ranks reproduce ONE reference call on the whole batch
         # True: every row of y is an independent restoration (own filter estimate and guidance scale); Hydra-style
         # configs switch it on with tester.blind_bwe.filter_per_row
@@ -257,9 +266,64 @@ class BlindSamplerFused:
         slot["events"][i] = ev
         return out
 
+    # -- keyed noise (row_seeds) -------------------------------------------------
+    # Draw index d of a call: 0 the initial state; schedule step i uses d = 1 + 8 i + slot with slot 0 the stochastic
+    # move, 1 / 2 / 3 the first evaluation's SNR observation noise (fit_params), sigma_den_estimate draw and SNR noise
+    # (get_rec_grads), 4 / 5 / 6 the same for the Heun evaluation, 7 reserved.  A call resumed at step i therefore
+    # draws what the uninterrupted call drew from step i on.
+    @staticmethod
+    def _seed_tensor(seeds):
+        """row_seeds -> int64 tensor (the bits of unsigned 64-bit seeds)."""
+        if torch.is_tensor(seeds):
+            if seeds.dtype != torch.int64 or seeds.dim() != 1:
+                raise ValueError(f"row_seeds must be a 1-D int64 tensor or a list of ints, got a {seeds.dtype} "
+                                 f"tensor of shape {tuple(seeds.shape)}")
+            return seeds
+        vals = []
+        for v in seeds:
+            if isinstance(v, bool) or not isinstance(v, int) and not hasattr(v, "__index__"):
+                raise ValueError(f"row_seeds entries must be ints, got {v!r}")
+            v = int(v)
+            if not -(1 << 63) <= v < (1 << 64):
+                raise ValueError(f"row seed {v} does not fit in 64 bits")
+            vals.append(v - (1 << 64) if v >= (1 << 63) else v)
+        return torch.tensor(vals, dtype=torch.int64)
+
+    def _keyed_begin(self, B, device):
+        """Start a call on B rows: keyed noise if ``row_seeds`` is set (checked here), else the other sources."""
+        self._keyed = None
+        if self.row_seeds is None:
+            return
+        if self.noise_fn is not None:
+            raise ValueError("row_seeds and noise_fn are both set: choose one noise source")
+        seeds = self._seed_tensor(self.row_seeds)
+        if seeds.numel() != B:
+            raise ValueError(f"row_seeds has {seeds.numel()} seeds for a call on {B} rows")
+        self._keyed = types.SimpleNamespace(seeds=seeds.to(device),
+                                            draw=torch.zeros(1, dtype=torch.int32, device=device))
+
+    def _keyed_step(self, i):
+        """Draw-index base of schedule step i (a device scalar, so captured kernels read it at replay)."""
+        if self._keyed is not None:
+            self._keyed.draw.fill_(1 + 8 * i)
+
+    def _keyed_noise(self, a_or_shape, slot, scale=None, row_scale=None, mult=1.0, out=None):
+        k = self._keyed
+        return ops.row_noise(k.seeds, a_or_shape, k.draw, slot, scale=scale, row_scale=row_scale, mult=mult, out=out)
+
+    def _initial_state(self, shape, device, t0, y=None):
+        """eps * t0, or y + eps * t0 (:640-644): draw 0."""
+        if self._keyed is not None:
+            return self._keyed_noise(shape if y is None else y, 0, scale=t0.reshape(1))
+        if y is None:
+            return self._randn(shape, device) * t0
+        return y + self._randn(shape, device) * t0
+
     def move_timestep(self, x, t, gamma, Snoise=1):
-        """testing/blind_bwe_sampler.py:509-516 (always draws)."""
+        """testing/blind_bwe_sampler.py:509-516 (always draws).  Keyed noise: draw and update in one launch."""
         t_hat = t + gamma * t
+        if self._keyed is not None:
+            return self._keyed_noise(x, 0, scale=((t_hat ** 2 - t ** 2) ** (1 / 2)).reshape(1), mult=Snoise), t_hat
         eps = self._randn(x.shape, x.device) * Snoise
         return x + ((t_hat ** 2 - t ** 2) ** (1 / 2)) * eps, t_hat
 
@@ -319,18 +383,25 @@ class BlindSamplerFused:
         H = bu.design_filter(filter_params[0], filter_params[1], self.freqs)
         return bu.apply_filter(x, H, self.args.tester.blind_bwe.NFFT)
 
-    def _maybe_noise_observations(self, y):
+    def _maybe_noise_observations(self, y, slot):
         ps = self.args.tester.posterior_sampling
         if ps.SNR_observations != "None":           # :80-86, :542-548 (in place on y)
             snr = 10 ** (ps.SNR_observations / 10)
             sigma = torch.sqrt(torch.var(y, -1) / snr).unsqueeze(-1)
-            y += sigma * self._randn(y.shape, y.device)
+            if self._keyed is None:
+                y += sigma * self._randn(y.shape, y.device)
+            elif y.is_contiguous():
+                self._keyed_noise(y, slot, row_scale=sigma.reshape(-1), out=y)
+            else:
+                y.copy_(self._keyed_noise(y, slot, row_scale=sigma.reshape(-1)))
 
     def fit_params(self, denoised_estimate, y, filter_params):
         """testing/blind_bwe_sampler.py:533-595."""
-        self._maybe_noise_observations(y)
+        self._maybe_noise_observations(y, self._eval_slot)
         sde = self.args.tester.blind_bwe.sigma_den_estimate
-        if sde:
+        if sde and self._keyed is not None:
+            denoised_estimate = self._keyed_noise(denoised_estimate, self._eval_slot + 1, mult=sde)
+        elif sde:
             denoised_estimate = denoised_estimate + self._randn(denoised_estimate.shape,
                                                                  denoised_estimate.device) * sde
         return self._fit(denoised_estimate, y, filter_params)
@@ -338,7 +409,7 @@ class BlindSamplerFused:
     def get_rec_grads(self, x_den, y, x, t_i, filter_params):
         """testing/blind_bwe_sampler.py:75-135."""
         ps = self.args.tester.posterior_sampling
-        self._maybe_noise_observations(y)
+        self._maybe_noise_observations(y, self._eval_slot + 2)
         nfft = self.args.tester.blind_bwe.NFFT
         if ps.norm == 2 and not ps.stft_distance.use:
             norm = rec_guidance_norms(x_den, y, self.freqs, filter_params, nfft)
@@ -377,8 +448,9 @@ class BlindSamplerFused:
         """testing/blind_bwe_sampler.py:63-73."""
         return y + x_hat - self.apply_filter_fcA(x_hat, filter_params)
 
-    def _evaluate(self, x_in, t_in, y, filter_params):
-        """Lines :689-:709 (and :733-:752 for the Heun correction)."""
+    def _evaluate(self, x_in, t_in, y, filter_params, slot=1):
+        """Lines :689-:709 (and :733-:752 for the Heun correction, keyed draw slot 4)."""
+        self._eval_slot = slot
         x_in.requires_grad_(True)
         x_den = self.get_denoised_estimate(x_in, t_in)
         x_den_2 = x_den.clone().detach()
@@ -425,16 +497,19 @@ class BlindSamplerFused:
 
     # -- one sampler step as a pure function of device tensors ----------------------------------------
     def _step_math(self, x, filter_params, eps, t_i, gamma_i, t_next, y, heun):
-        """Lines :686-:761 of the reference loop; all scalars are 0-d device tensors."""
+        """Lines :686-:761 of the reference loop; all scalars are 0-d device tensors.  eps None: keyed noise."""
         t_hat = t_i + gamma_i * t_i
-        x_hat = x + ((t_hat ** 2 - t_i ** 2) ** (1 / 2)) * eps
+        if eps is None:
+            x_hat = self._keyed_noise(x, 0, scale=((t_hat ** 2 - t_i ** 2) ** (1 / 2)).reshape(1))
+        else:
+            x_hat = x + ((t_hat ** 2 - t_i ** 2) ** (1 / 2)) * eps
         score, filter_params, x_den_2 = self._evaluate(x_hat, t_hat, y, filter_params)
         fp_mid = filter_params.clone()           # what rid logs (:724): the filter after the FIRST evaluation
         d = -t_hat * score
         h = t_next - t_hat
         if heun:
             x_prime = x_hat + h * d
-            score, filter_params, _ = self._evaluate(x_prime, t_next, y, filter_params)
+            score, filter_params, _ = self._evaluate(x_prime, t_next, y, filter_params, slot=4)
             x_new = x_hat + h * ((1 / 2) * d + (1 / 2) * (-t_next * score))
         else:
             x_new = x_hat + h * d
@@ -442,7 +517,11 @@ class BlindSamplerFused:
 
     def _step_graph_for(self, y, filter_params, heun):
         """Capture (once per shape / variant) and return the replayable step."""
-        key = (tuple(y.shape), y.device, tuple(filter_params.shape), self.filter_per_row, self._fit.cfg_key())
+        keyed = self._keyed
+        # keyed noise is generated inside the step from the graph's seed and draw-index buffers: the key records that
+        # it is on, not the seed values (new seeds are copied into the buffers, no recapture)
+        key = (tuple(y.shape), y.device, tuple(filter_params.shape), self.filter_per_row, keyed is not None,
+               self._fit.cfg_key())
         if self._step_key != key:
             self._step_key, self._step_graphs = key, {}
         if heun in self._step_graphs:
@@ -455,9 +534,20 @@ class BlindSamplerFused:
         # and re-installed on replaying calls
         st = types.SimpleNamespace(
             y=y.clone(), fit=self._fit, freqs=self.freqs,
-            x=torch.zeros_like(y), fp=filter_params.clone(), eps=torch.zeros_like(y),
+            x=torch.zeros_like(y), fp=filter_params.clone(), eps=None if keyed is not None else torch.zeros_like(y),
             t_i=torch.ones((), device=dev), gamma=torch.zeros((), device=dev), t_next=torch.ones((), device=dev) * 0.5,
-            graph=None, x_out=None, fp_out=None, den=None, launches=0)
+            seeds=None, draw=None, graph=None, x_out=None, fp_out=None, den=None, launches=0)
+        if keyed is not None:
+            st.seeds, st.draw = keyed.seeds.clone(), torch.zeros_like(keyed.draw)
+            self._keyed = types.SimpleNamespace(seeds=st.seeds, draw=st.draw)     # what the captured kernels read
+        try:
+            self._capture_step(st, heun)
+        finally:
+            self._keyed = keyed
+        self._step_graphs[heun] = st
+        return st
+
+    def _capture_step(self, st, heun):
         was_prof = profiling._enabled
         profiling.enable(False)                      # no event records inside a capture
         side = torch.cuda.Stream()
@@ -487,8 +577,6 @@ class BlindSamplerFused:
                 gc.enable()
         st.graph = g
         profiling.enable(was_prof)
-        self._step_graphs[heun] = st
-        return st
 
     # -- the sampling loop ---------------------------------------------------
     def predict_blind_bwe(self, y, rid=False, compute_sweep=False, max_steps=None, step_hook=None,
@@ -502,6 +590,7 @@ class BlindSamplerFused:
         ``init_params`` may be (2, K) (every row) or (B, 2, K), and with ``rid`` the logged filters are
         (T, B, 2, K)."""
         args = self.args
+        self._keyed_begin(y.shape[0], y.device)
         if self.filter_per_row:
             self._check_per_row(compute_sweep)
         device = y.device
@@ -535,10 +624,10 @@ class BlindSamplerFused:
 
         if self.start_sigma is None:
             t = self.diff_params.create_schedule(self.nb_steps).to(device)
-            x = self._randn(shape, device) * t[0] if init_x is None else init_x.to(device)
+            x = self._initial_state(shape, device, t[0]) if init_x is None else init_x.to(device)
         else:
             t = self.diff_params.create_schedule_from_initial_t(self.start_sigma, self.nb_steps).to(device)
-            x = y + self._randn(shape, device) * t[0] if init_x is None else init_x.to(device)
+            x = self._initial_state(shape, device, t[0], y) if init_x is None else init_x.to(device)
         gamma = self.diff_params.get_gamma(t).to(device)
         t_host = t.cpu()
         n_steps = self.nb_steps if max_steps is None else min(start_step + max_steps, self.nb_steps)
@@ -563,8 +652,13 @@ class BlindSamplerFused:
                 if i == start_step:
                     for sg in self._step_graphs.values():
                         sg.fp.copy_(filter_params)
+                        if self._keyed is not None:
+                            sg.seeds.copy_(self._keyed.seeds)
                 st.x.copy_(x)
-                st.eps.copy_(self._randn(shape, device) * Snoise, non_blocking=True)
+                if self._keyed is not None:
+                    st.draw.fill_(1 + 8 * i)               # the noise is generated inside the step
+                else:
+                    st.eps.copy_(self._randn(shape, device) * Snoise, non_blocking=True)
                 st.t_i.copy_(t[i]); st.gamma.copy_(gamma[i]); st.t_next.copy_(t[i + 1])
                 st.graph.replay()
                 profiling.add_launches(st.launches)
@@ -581,6 +675,7 @@ class BlindSamplerFused:
             n_steps = start_step                           # the eager loop below has nothing left to do
 
         for i in range(start_step, n_steps):
+            self._keyed_step(i)
             x_hat, t_hat = self.move_timestep(x, t[i], gamma[i])
             score, filter_params, x_den_2 = self._evaluate(x_hat, t_hat, y, filter_params)
             if compute_sweep:
@@ -596,7 +691,7 @@ class BlindSamplerFused:
             if float(t_host[i + 1]) != 0 and self.order == 2:
                 t_prime = t[i + 1]
                 x_prime = x_hat + h * d
-                score, filter_params, _ = self._evaluate(x_prime, t_prime, y, filter_params)
+                score, filter_params, _ = self._evaluate(x_prime, t_prime, y, filter_params, slot=4)
                 d_prime = -t_prime * score
                 x = x_hat + h * ((1 / 2) * d + (1 / 2) * d_prime)
             else:
@@ -604,6 +699,7 @@ class BlindSamplerFused:
             if step_hook is not None:
                 step_hook(i, x, filter_params)
 
+        self._keyed = None
         if rid:
             out = (x.detach(), filter_params.detach(), data_denoised.detach(), t.detach(), data_filters.detach())
             if compute_sweep:
@@ -613,14 +709,16 @@ class BlindSamplerFused:
 
     def predict_unconditional(self, shape, device, rid=False):
         """testing/blind_bwe_sampler.py:366-374,406-497 with y = None."""
+        self._keyed_begin(shape[0], device)
         t = self.diff_params.create_schedule(self.nb_steps).to(device)
-        x = self._randn(shape, device) * t[0]
+        x = self._initial_state(shape, device, t[0])
         gamma = self.diff_params.get_gamma(t).to(device)
         t_host = t.cpu()
         if rid:
             data_denoised = torch.zeros((self.nb_steps, shape[0], shape[1]))
             data_score = torch.zeros((self.nb_steps, shape[0], shape[1]))
         for i in range(self.nb_steps):
+            self._keyed_step(i)
             x_hat, t_hat = self.move_timestep(x, t[i], gamma[i], self.diff_params.Snoise)
             with torch.no_grad():
                 score = (self.get_denoised_estimate(x_hat, t_hat) - x_hat) / t_hat ** 2
@@ -637,6 +735,7 @@ class BlindSamplerFused:
                 x = x_hat + h * ((1 / 2) * d + (1 / 2) * (-t_prime * score))
             else:
                 x = x_hat + h * d
+        self._keyed = None
         if rid:
             return x.detach(), data_denoised.detach(), data_score.detach(), t.detach()
         return x.detach()
@@ -714,18 +813,20 @@ class BlindSamplerFused:
     def predict_conditional(self, y, degradation, rid=False, dc_step=None, fused_params=None):
         """testing/blind_bwe_sampler.py:387-497 (``predict`` with observations y)."""
         shape, device = y.shape, y.device
+        self._keyed_begin(shape[0], device)
         if self.start_sigma is None:
             t = self.diff_params.create_schedule(self.nb_steps).to(device)
-            x = self._randn(shape, device) * t[0]
+            x = self._initial_state(shape, device, t[0])
         else:
             t = self.diff_params.create_schedule_from_initial_t(self.start_sigma, self.nb_steps).to(device)
-            x = y + self._randn(shape, device) * t[0]
+            x = self._initial_state(shape, device, t[0], y)
         gamma = self.diff_params.get_gamma(t).to(device)
         t_host = t.cpu()
         if rid:
             data_denoised = torch.zeros((self.nb_steps, shape[0], shape[1]))
             data_score = torch.zeros((self.nb_steps, shape[0], shape[1]))
         for i in range(self.nb_steps):
+            self._keyed_step(i)
             x_hat, t_hat = self.move_timestep(x, t[i], gamma[i], self.diff_params.Snoise)
             score = self.get_score(x_hat, y, t_hat, degradation, dc_step, fused_params)
             d = -t_hat * score
@@ -740,6 +841,7 @@ class BlindSamplerFused:
                 x = x_hat + h * ((1 / 2) * d + (1 / 2) * (-t_prime * score))
             else:
                 x = x_hat + h * d
+        self._keyed = None
         if rid:
             return x.detach(), data_denoised.detach(), data_score.detach(), t.detach()
         return x.detach()

@@ -10,9 +10,40 @@ filter estimate, :433,:477,:543) and the predictions are cross-faded with a
 ranks with no data-path collective (SURVEY 8e); ``restore_recording`` gathers
 predictions and per-segment filters with NCCL at the end.
 """
+import contextlib
+
 import torch
 
 from . import distributed as bd
+
+_MASK64 = (1 << 64) - 1
+_GOLDEN64 = 0x9E3779B97F4A7C15
+
+
+def row_seed(seed, k):
+    """Seed of unit ``k`` (segment, window or row) of a run seeded with ``seed``: SplitMix64 of
+    ``seed + (k + 1) * 0x9E3779B97F4A7C15`` (mod 2**64), i.e. output k of the SplitMix64 stream started at
+    ``seed``.  An unsigned 64-bit int, for ``BlindSamplerFused.row_seeds``.  A pure function: every rank derives
+    the seed of a unit from its global index alone."""
+    z = (int(seed) + (int(k) + 1) * _GOLDEN64) & _MASK64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _MASK64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _MASK64
+    return z ^ (z >> 31)
+
+
+@contextlib.contextmanager
+def _row_seeds(sampler, seeds):
+    """Install ``row_seeds`` on the sampler for one call and restore the previous value afterwards
+    (``seeds`` None: leave the sampler as it is)."""
+    if seeds is None:
+        yield
+        return
+    was = sampler.row_seeds
+    sampler.row_seeds = list(seeds)
+    try:
+        yield
+    finally:
+        sampler.row_seeds = was
 
 
 def segment_spans(L, seg_len, ola=256, discard_end=200, discard_start=0):
@@ -59,7 +90,7 @@ def merge(preds, spans, L, ola=256, discard_end=200):
     return out
 
 
-def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, joint=False, batched=False):
+def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, joint=False, batched=False, seed=None):
     """Blind restoration of a whole recording, segments sharded over the ranks of the
     current process group.  Returns (final_pred (1, L), filter_data) on every rank,
     ``filter_data`` being the list [((ix0, ix1), filter_params), ...] the reference
@@ -72,7 +103,13 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
     noise is drawn for the whole batch at each step, so the host noise stream is consumed in a
     different order than by the loop of B = 1 calls: the two restorations agree statistically,
     not bitwise (they agree to rounding when every segment gets the same noise either way, e.g.
-    through ``sampler.noise_fn``)."""
+    through ``sampler.noise_fn``).
+
+    ``seed`` (an int) switches the sampler to keyed per-row noise: segment s, counted over the whole
+    recording, draws with ``row_seed(seed, s)`` in all three modes, so the noise each segment sees
+    depends neither on the mode nor on how the segments are sharded over ranks (the sequential and
+    batched restorations then agree to the rounding of the per-row kernels).  ``seed=None`` keeps the
+    sampler's own noise source."""
     import torch.distributed as dist
     if joint and batched:
         raise ValueError("batched=True restores every segment with its own filter; joint=True shares one")
@@ -84,21 +121,25 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
                          "(an empty shard would enter the NCCL gathers with a different shape)")
     lo, hi = bd.shard_rows(segs.shape[0], rank, world)
     mine = segs[lo:hi]
+    seeds = None if seed is None else [row_seed(seed, k) for k in range(lo, hi)]
     if joint:
         sampler.joint = True
-        pred, filt = sampler.predict_blind_bwe(mine, rid=False)
+        with _row_seeds(sampler, seeds):
+            pred, filt = sampler.predict_blind_bwe(mine, rid=False)
         filts = filt.unsqueeze(0).expand(mine.shape[0], -1, -1).contiguous()
     elif batched:
         was = sampler.filter_per_row
         sampler.filter_per_row = True
         try:
-            pred, filts = sampler.predict_blind_bwe(mine.clone(), rid=False)
+            with _row_seeds(sampler, seeds):
+                pred, filts = sampler.predict_blind_bwe(mine.clone(), rid=False)
         finally:
             sampler.filter_per_row = was
     else:
         preds, fl = [], []
         for s in range(mine.shape[0]):
-            p, f = sampler.predict_blind_bwe(mine[s:s + 1].clone(), rid=False)
+            with _row_seeds(sampler, None if seeds is None else seeds[s:s + 1]):
+                p, f = sampler.predict_blind_bwe(mine[s:s + 1].clone(), rid=False)
             preds.append(p)
             fl.append(f)
         pred = torch.cat(preds, 0) if preds else mine.new_zeros((0, seg_len))
@@ -111,7 +152,7 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
 
 def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25, n_segments_blindstep=2,
                          ix_start_s=0, std=0.1, typefilter="fc_A", discard_end=200, discard_start=0,
-                         rng=None, estimated_filter=None):
+                         rng=None, estimated_filter=None, seed=None):
     """Autoregressive restoration of a whole recording with ONE filter estimated once:
     ``BlindTester.test_real_blind_bwe_complete`` (testing/blind_bwe_tester.py:710-867) without file
     I/O, resampling and wandb.
@@ -126,7 +167,12 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
 
     Sequential by construction (each window needs the previous prediction): replicas only across
     recordings (SURVEY 8e).  ``degraded``: (1, L) tensor on the sampler's device.  Returns
-    (restored (1, L), filter (2, K))."""
+    (restored (1, L), filter (2, K)).
+
+    ``seed`` (an int) switches the sampler to keyed per-row noise: window w draws with ``row_seed(seed, w)``
+    (w = 0 is the first ``predict_bwe`` window, then the autoregressive windows, then the padded last one) and
+    row j of the blind step with ``row_seed(seed, 2**32 + j)``, so the restoration is a function of the
+    recording and the seed alone.  ``seed=None`` keeps the sampler's own noise source."""
     import numpy as np
     segL = int(seg_len)
     L = degraded.shape[-1]
@@ -143,13 +189,23 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
             for j in range(n_segments_blindstep):
                 ix = int(rng.randint(0, L - segL))
                 y[j] = degraded[0, ix:ix + segL]
-        pred, estimated_filter = sampler.predict_blind_bwe(y, rid=False)
+        blind = None if seed is None else [row_seed(seed, (1 << 32) + j) for j in range(y.shape[0])]
+        with _row_seeds(sampler, blind):
+            pred, estimated_filter = sampler.predict_blind_bwe(y, rid=False)
         final[0, ix_first:ix_first + segL] = pred[0]
     overlap = int(overlap_s * sample_rate)
     keep = segL - discard_end
     ix = 0
+    window = [0]
+
+    def keyed():                                             # the seeds of the next window
+        w = window[0]
+        window[0] += 1
+        return _row_seeds(sampler, None if seed is None else [row_seed(seed, w)])
+
     seg = degraded[..., ix:ix + segL]
-    pred = sampler.predict_bwe(seg, estimated_filter, typefilter, rid=False)
+    with keyed():
+        pred = sampler.predict_bwe(seg, estimated_filter, typefilter, rid=False)
     previous = pred[..., :keep]
     final[..., ix:ix + keep] = previous
     ix += segL - overlap - discard_end
@@ -161,7 +217,8 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
     while ix < L - segL - discard_end - discard_start or L - ix > segL:
         y_masked[..., :overlap] = previous[..., segL - overlap - discard_end:]
         seg = degraded[..., ix:ix + segL]
-        pred = sampler.predict_bwe_AR(seg, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
+        with keyed():
+            pred = sampler.predict_bwe_AR(seg, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
         previous = pred[..., :keep]
         final[..., ix:ix + keep] = previous
         ix += segL - overlap - discard_end
@@ -174,6 +231,7 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
         mask[..., n:segL] = 0
     else:
         seg_zp = seg[..., :segL]
-    pred = sampler.predict_bwe_AR(seg_zp, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
+    with keyed():
+        pred = sampler.predict_bwe_AR(seg_zp, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
     final[..., ix:ix + n] = pred[..., :n]
     return final * scale.unsqueeze(-1) / std, estimated_filter

@@ -339,6 +339,16 @@ int babe_gn_film_gelu_bwd(const float* gh, const float* x, const float* gy, floa
 int babe_resample2(const float* in, float* out, long long rows, int T, int mode,
                    const float* taps_host, int L, void* stream);
 
+/* ---- keyed per-row noise (sampler draws with BlindSamplerFused.row_seeds) ---- */
+/* out[b,n] = a[b,n] + eps[b,n] * mult * (*scale) * row_scale[b] on B rows of T samples, where eps[b,n] is the
+ * standard normal sample n of row seed seeds[b] (int64 read as uint64) at draw index *draw + slot: Philox4x32-10
+ * with key (seed low, seed high) and counter (n/4, draw index, 0, 0), uniforms (2 (x >> 9) + 1) 2^-24, Box-Muller
+ * (DESIGN.md 4.8).  eps depends on (seed, draw index, n) only, never on B, the row's position, T or alignment.
+ * a (may be NULL = 0, may equal out), scale (one device float) and row_scale (B device floats) are optional; draw is
+ * one device int, read at run time, so a captured graph replays with the value it holds then. */
+int babe_row_noise(float* out, const float* a, const long long* seeds, int B, int T, const int* draw, int slot,
+                   const float* scale, const float* row_scale, float mult, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
