@@ -378,7 +378,10 @@ class CQT_nsgt:
                             f"cuda:{torch.cuda.current_device()}: they must agree")
         if x.shape[-1] != self.Ls:
             raise ValueError(f"input length {x.shape[-1]} != audio_len {self.Ls}")
-        return x.reshape(-1, self.Ls).contiguous()
+        rows = x.reshape(-1, self.Ls).contiguous()
+        # the kernels read the rows as float2 / float4: a contiguous view at an odd float offset (a slice of a longer
+        # buffer) is copied into fresh, aligned storage
+        return rows if rows.data_ptr() % 16 == 0 else rows.clone()
 
     def fwd(self, x):
         """x (B,C,T) -> list of numocts complex64 tensors (B,C,binsoct,T_o),

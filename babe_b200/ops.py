@@ -38,6 +38,18 @@ def _cuda_f32(t, name):
     return t.detach().contiguous()
 
 
+def _filter_out(out, x):
+    """The output tensor of the filter ops: new, or ``out`` once it is known to hold exactly x's B * T floats (the
+    kernels write them from its base pointer, so a smaller, strided or other-typed ``out`` would be overrun)."""
+    if out is None:
+        return torch.empty_like(x)
+    if not (torch.is_tensor(out) and out.is_cuda and out.dtype == torch.float32 and out.device == x.device
+            and out.shape == x.shape and out.is_contiguous()):
+        what = f"{out.dtype} {tuple(out.shape)} on {out.device}" if torch.is_tensor(out) else type(out).__name__
+        raise ValueError(f"out must be a contiguous float32 tensor of shape {tuple(x.shape)} on {x.device}, got {what}")
+    return out
+
+
 def num_frames(T, nfft):
     """utils/blind_bwe_utils.py:22-23: padded by NFFT, hop NFFT/2, center=False."""
     return 1 + T // (nfft // 2)
@@ -123,9 +135,11 @@ def apply_filter(x, nfft, H=None, freqs=None, fc=None, A=None, adjoint=False, su
             raise ValueError("sub must match x")
     if row_scale is not None:
         row_scale = _cuda_f32(row_scale, "row_scale")
+        if row_scale.numel() != B:
+            raise ValueError("row_scale must have B entries")
     if row_sumsq is not None and (row_sumsq.dtype != torch.float64 or row_sumsq.numel() != B):
         raise ValueError("row_sumsq must be float64[B]")
-    y = torch.empty_like(x) if out is None else out
+    y = _filter_out(out, x)
     ws, nbytes = None, 0
     if row_sumsq is not None:
         nbytes = lib().babe_apply_filter_workspace(B, T, int(nfft))
@@ -176,7 +190,7 @@ def apply_filter_rows(x, nfft, freqs, fc, A, adjoint=False, sub=None, row_scale=
         raise ValueError("row_sumsq must be float64[B]")
     if status is not None and (status.dtype != torch.int32 or status.numel() != B):
         raise ValueError("status must be int32[B]")
-    y = torch.empty_like(x) if out is None else out
+    y = _filter_out(out, x)
     ws, nbytes = None, 0
     if row_sumsq is not None:
         nbytes = lib().babe_apply_filter_workspace(B, T, int(nfft))
@@ -205,6 +219,8 @@ def stft(x, nfft, frames=0, in_env_div=False, bin_scale=None):
 
 def istft(X, nfft, out_len=None, bin_scale=None, out_env_div=True):
     X = _cuda_f32(X, "X")
+    if X.data_ptr() % 8:
+        X = X.clone()           # k_istft reads the bins as float2: a view at an odd float offset goes to fresh storage
     B, F, M, two = X.shape
     if F != nfft // 2 + 1 or two != 2:
         raise ValueError("X must be (B, NFFT/2+1, frames, 2)")

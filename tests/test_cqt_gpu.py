@@ -223,3 +223,25 @@ def test_programmatic_launch_is_bitwise_neutral(CQT):
     assert len(ref) == len(got)
     for a, b in zip(ref, got):
         assert torch.equal(torch.view_as_real(a) if a.is_complex() else a, torch.view_as_real(b) if b.is_complex() else b)
+
+
+@pytest.mark.parametrize("numocts,binsoct,fs,Ls,B", [CONFIGS[0], CONFIGS[2]])
+def test_rows_at_odd_float_offset_are_realigned(CQT, numocts, binsoct, fs, Ls, B):
+    """The CQT kernels read their input rows as float2 / float4.  A contiguous view that starts at an odd float (a slice
+    of a longer buffer) is copied into aligned storage first -- checked before anything is launched on it -- and then
+    gives the aligned call's results bit for bit."""
+    cq = CQT(numocts, binsoct, mode="oct", window=("kaiser", 1), fs=fs, audio_len=Ls, device="cuda")
+    g = torch.Generator().manual_seed(Ls + 1)
+    x = (torch.randn(B, Ls, generator=g) * 0.063).cuda()
+    buf = torch.empty(B * Ls + 4, device="cuda")
+    view = buf[1:1 + B * Ls].view(B, Ls)
+    view.copy_(x)
+    assert view.is_contiguous() and view.data_ptr() % 8 == 4
+    assert cq._rows(view).data_ptr() % 16 == 0
+    assert cq._rows(view.unsqueeze(1)).data_ptr() % 16 == 0
+    c, c_ref = cq.fwd(view.unsqueeze(1)), cq.fwd(x.unsqueeze(1))
+    assert all(torch.equal(a, b) for a, b in zip(c, c_ref))
+    assert torch.equal(cq.bwd(c), cq.bwd(c_ref))
+    assert torch.equal(cq.apply_hpf_DC(view), cq.apply_hpf_DC(x))
+    assert torch.equal(cq.rfft(view), cq.rfft(x))
+    assert torch.equal(view, x)                             # the view itself is left alone

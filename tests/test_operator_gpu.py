@@ -131,25 +131,36 @@ def test_apply_filter_vs_oracle(bu, sf, nfft, B, T):
 
 @pytest.mark.parametrize("nfft", [1024, 4096])
 def test_fused_design_and_epilogues(bu, sf, nfft):
+    """In-kernel filter design and the guidance epilogues (residual + sum of squares, adjoint with row scale) against
+    the oracle.  At NFFT 4096, T = 30012 runs them on k_filter_fused (<false, 1> and <true, 2>); T = 30011 cannot be
+    bulk-copied and runs the round-1 k_apply_filter, as does every NFFT 1024 call."""
     from babe_b200 import ops
-    torch.manual_seed(5)
-    B, T = 4, 30011
-    x, yobs = torch.randn(B, T) * 0.05, torch.randn(B, T) * 0.05
-    f = torch.fft.rfftfreq(nfft, d=1 / 22050)
-    fc, A = torch.tensor([300.0, 310.0, 900.0, 5000.0]), torch.tensor([-12.0, -14.0, -30.0, -31.0])
-    H = sf.design_filter(fc, A, f)
-    y = ops.apply_filter(x.cuda(), nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda())
-    assert rel_l2(y.cpu(), sf.apply_filter(x, H, nfft)) < TOL
-    ss = torch.zeros(B, dtype=torch.float64, device="cuda")
-    r = ops.apply_filter(x.cuda(), nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda(), sub=yobs.cuda(), row_sumsq=ss)
-    r_ref = sf.apply_filter(x, H, nfft) - yobs
-    assert rel_l2(r.cpu(), r_ref) < TOL
-    assert rel_l2(ss.cpu(), (r_ref.double() ** 2).sum(1)) < TOL
-    n_ref, g_ref = sf.rec_guidance_operator(x, yobs, H, nfft)
-    scale = (1.0 / torch.sqrt(ss)).float()
-    g = ops.apply_filter(r, nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda(), adjoint=True, row_scale=scale)
-    assert rel_l2(torch.sqrt(ss).cpu(), n_ref) < TOL
-    assert rel_l2(g.cpu(), g_ref) < 2e-5
+    from kernel_trace import assert_path, filter_variants, launched
+    for T in (30011, 30012):
+        torch.manual_seed(5)
+        B = 4
+        x, yobs = torch.randn(B, T) * 0.05, torch.randn(B, T) * 0.05
+        f = torch.fft.rfftfreq(nfft, d=1 / 22050)
+        fc, A = torch.tensor([300.0, 310.0, 900.0, 5000.0]), torch.tensor([-12.0, -14.0, -30.0, -31.0])
+        H = sf.design_filter(fc, A, f)
+        with launched() as names:
+            y = ops.apply_filter(x.cuda(), nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda())
+            ss = torch.zeros(B, dtype=torch.float64, device="cuda")
+            r = ops.apply_filter(x.cuda(), nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda(), sub=yobs.cuda(),
+                                 row_sumsq=ss)
+            scale = (1.0 / torch.sqrt(ss)).float()
+            g = ops.apply_filter(r, nfft, freqs=f.cuda(), fc=fc.cuda(), A=A.cuda(), adjoint=True, row_scale=scale)
+        fused = nfft == 4096 and T % 4 == 0
+        assert_path(names, fused=fused, kernel="k_filter_fused" if fused else "k_apply_filter")
+        if fused:
+            assert filter_variants(names) == {(False, 0, False), (False, 1, False), (True, 2, False)}
+        assert rel_l2(y.cpu(), sf.apply_filter(x, H, nfft)) < TOL
+        r_ref = sf.apply_filter(x, H, nfft) - yobs
+        assert rel_l2(r.cpu(), r_ref) < TOL
+        assert rel_l2(ss.cpu(), (r_ref.double() ** 2).sum(1)) < TOL
+        n_ref, g_ref = sf.rec_guidance_operator(x, yobs, H, nfft)
+        assert rel_l2(torch.sqrt(ss).cpu(), n_ref) < TOL
+        assert rel_l2(g.cpu(), g_ref) < 2e-5
 
 
 @pytest.mark.parametrize("nfft", [512, 1024, 2048, 4096])
