@@ -2,8 +2,8 @@
 // two-wide FADD2 / FFMA2 / FMUL2: one issue slot per complex add), forward or inverse selected at compile time (no
 // conjugation passes), with the window / dual-window multiply folded into the first butterflies.
 //
-// BandCoreV<R3, INV>: M = 256 R3 points (R3 = 1..16) by TPB = 16 R3 threads, 16 points per thread, same index
-// scheme as round 1's BandCore (bandfft.cuh) -- coalesced on both sides without staging:
+// BandCoreV<R3, INV>: M = 256 R3 points (R3 = 1..16) by TPB = 16 R3 threads, 16 points per thread, three passes
+// 16 x 16 x R3 with two exchanges (rows of TPB + 1 float2: conflict-free) -- coalesced on both sides without staging:
 //   n = 16 R3 n1 + R3 n2 + n3,   k = k1 + 16 k2 + 256 k3,   t = R3 n2 + n3
 //   P1  thread t: FFT16 n1 -> k1, * W_M^{-+ t k1} -> ex[k1][t]            (input slot of register n1: TPB n1 + t)
 //   P2  thread (k1 = t & 15, n3 = t >> 4): FFT16 n2 -> k2, in place
@@ -14,7 +14,7 @@
 //
 // The exchanges are synchronised per BAND (named barrier of TPB threads, __syncwarp for TPB <= 32), never per CTA:
 // the bands of a CTA run independently.  Every thread of a band group must call fwd().
-// __host__ __device__ passes: tests/host/bandfft_host_check.cu.
+// __host__ __device__ passes: tests/host/bandfft_v_host_check.cu.
 #pragma once
 #include "common.cuh"
 #include "fft16v.cuh"

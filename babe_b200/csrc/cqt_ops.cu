@@ -19,19 +19,17 @@
 #include <algorithm>
 
 #include "common.cuh"
-#include "bandfft.cuh"
 #include "bandfft_v.cuh"
 #include "tma.cuh"
 #include "smemfft.cuh"
 #include "rfft_pairs.cuh"
-#include "cqt_fft.cuh"
 #include "cqt_pfa.cuh"
 
 namespace babe {
 
 constexpr int CQT_THREADS = 256;
 constexpr int MAX_TB = 64;          // bands per CTA (tb <= 2048 / 32)
-constexpr int BAND_THREADS = 256;   // band kernels: 16 points per thread, 4096-point tiles (bandfft.cuh)
+constexpr int BAND_THREADS = 256;   // band kernels: 16 points per thread, 4096-point tiles (bandfft_v.cuh)
 constexpr int TILE_SEQ = 8;          // sequences per CTA in the two big-FFT passes
 constexpr int TW_LO = 1024;          // low part of the two-level twiddle tables
 
@@ -209,11 +207,10 @@ __device__ __forceinline__ int find_octave(const BandArgs& a, int item) {
   return o;
 }
 
-// --- octaves with M = 256 * R3: register FFT (bandfft.cuh), 16 / R3 bands per CTA ----------
-// The 16 input values of a thread for row r+1 (a window slice of the half spectrum, or a coefficient row) are
-// copied global -> shared with 8-byte cp.async while row r is transformed: round 1's version loaded them straight
-// into registers at the top of every row and sat on the scoreboard (long_scoreboard 7.7 of 13 stall cycles per
-// issue, profiles/r01_cqt_B64.md).
+// cp.async staging of the band kernels: the 16 input values of a thread for row r+1 (a window slice of the half
+// spectrum, or a coefficient row) are copied global -> shared with 8-byte cp.async while row r is transformed.  Loaded
+// straight into registers at the top of every row they sat on the scoreboard (long_scoreboard 7.7 of 13 stall cycles
+// per issue, profiles/r01_cqt_B64.md).
 __device__ __forceinline__ void cp_async8(void* dst, const void* src) {
   const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(src) : "memory");
@@ -226,152 +223,19 @@ __device__ __forceinline__ void cp_async_commit_wait() {
   asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
 }
 
-template <int R3, bool SYNTH>
-__device__ __forceinline__ void band_tile_fast(const BandArgs& a, int o, int tile, int row0, int row_end,
-                                               unsigned char* smem_raw) {
-  using C = BandCore<R3>;
-  constexpr int NB = BAND_THREADS / C::TPB, M = C::M;
-  float2* exs = reinterpret_cast<float2*>(smem_raw);
-  float2* tw = exs + NB * C::EX;
-  float2* stage = tw + C::TPB;                         // [16][BAND_THREADS]: slot n1 of thread tid
-  const int tid = threadIdx.x, bl = tid / C::TPB, t = tid % C::TPB;
-  const float2* roots_m = a.rootsm[o];
-  C::load_twiddles(tw, roots_m);
-  typename C::Regs rg;
-  C::init_regs(rg, roots_m, t);
-  const int band = tile * NB + bl;
-  const bool active = band < a.binsoct;
-  int p = 0, lg = 0, off = 0;
-  if (active) {
-    const int j = o * a.binsoct + band;
-    p = a.band_p[j]; lg = a.band_lg[j]; off = a.band_off[j];
-  }
-  const int half = lg / 2;
-  float2* ex = exs + bl * C::EX;
-  const float inv_m = 1.0f / (float)M;
-  // analysis: window samples (times the optional bin scale) and validity of this thread's 16 slots are
-  // row-independent: kept in shared memory next to the prefetch slots (zero = slot outside the window; those
-  // slots are never copied into, so they are zeroed once)
-  float* wst = reinterpret_cast<float*>(stage + 16 * BAND_THREADS);
-  unsigned valid = 0;
-  if (!SYNTH) {
-#pragma unroll
-    for (int n1 = 0; n1 < 16; ++n1) {
-      int i = C::TPB * n1 + t + half;
-      if (i >= M) i -= M;
-      float w = 0.f;
-      const int k = p - half + i;
-      if (active && i < lg && k >= 0 && k <= a.Nc) {
-        w = a.win[off + i];
-        if (a.scale) w *= a.scale[k];
-        valid |= 1u << n1;
-      }
-      wst[n1 * BAND_THREADS + tid] = w;
-      stage[n1 * BAND_THREADS + tid] = make_float2(0.f, 0.f);
-    }
-  } else {
-    // synthesis: the dual-window samples of this thread's 16 OUTPUT slots (zero = outside the band's window)
-#pragma unroll
-    for (int r = 0; r < 16; ++r) {
-      int i = C::out_slot(r, t) + half;
-      if (i >= M) i -= M;
-      wst[r * BAND_THREADS + tid] = (active && i < lg) ? a.win[off + i] : 0.f;
-    }
-  }
-  auto prefetch = [&](int row) {
-    if (!SYNTH) {
-      const float2* X = a.X + (size_t)row * a.xpitch + (p - half);
-#pragma unroll
-      for (int n1 = 0; n1 < 16; ++n1) {
-        int i = C::TPB * n1 + t + half;
-        if (i >= M) i -= M;
-        if (valid & (1u << n1)) cp_async8(stage + n1 * BAND_THREADS + tid, X + i);
-      }
-    } else if (active) {
-      if (!a.planar) {
-        const float2* in = a.coef[o] + ((size_t)row * a.binsoct + band) * M;
-#pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) cp_async8(stage + n1 * BAND_THREADS + tid, in + C::TPB * n1 + t);
-      } else {
-        const float* ire = reinterpret_cast<const float*>(a.coef[o]) + (((size_t)row * 2) * a.binsoct + band) * M;
-        const float* iim = ire + (size_t)a.binsoct * M;
-#pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) {
-          float* d = reinterpret_cast<float*>(stage + n1 * BAND_THREADS + tid);
-          cp_async4f(d, ire + C::TPB * n1 + t);
-          cp_async4f(d + 1, iim + C::TPB * n1 + t);
-        }
-      }
-    }
-  };
-  if (row0 < row_end) prefetch(row0);
-  __syncthreads();
-  for (int row = row0; row < row_end; ++row) {
-    float re[16], im[16];
-    cp_async_commit_wait();                       // this thread's own copies: no barrier needed to read them
-    if (!SYNTH) {
-      // slot m holds window sample i with (i - half) mod M == m, conjugated (inverse FFT via forward)
-#pragma unroll
-      for (int n1 = 0; n1 < 16; ++n1) {
-        const float2 xv = stage[n1 * BAND_THREADS + tid];
-        const float w = wst[n1 * BAND_THREADS + tid];
-        re[n1] = xv.x * w;
-        im[n1] = -xv.y * w;
-      }
-    } else if (active) {
-#pragma unroll
-      for (int n1 = 0; n1 < 16; ++n1) { const float2 v = stage[n1 * BAND_THREADS + tid]; re[n1] = v.x; im[n1] = v.y; }
-    } else {
-#pragma unroll
-      for (int n1 = 0; n1 < 16; ++n1) { re[n1] = 0.f; im[n1] = 0.f; }
-    }
-    if (row + 1 < row_end) prefetch(row + 1);     // the staged values are in registers: the slots are free
-    C::fwd(re, im, ex, tw, rg, t);
-    if (active) {
-      if (!SYNTH) {
-        if (!a.planar) {
-          float2* out = a.coef[o] + ((size_t)row * a.binsoct + band) * M;
-#pragma unroll
-          for (int r = 0; r < 16; ++r) out[C::out_slot(r, t)] = make_float2(re[r] * inv_m, -im[r] * inv_m);
-        } else {   // the layout the denoiser consumes (networks/cqtdiff+.py:750-753) without the transposing copy
-          float* ore = reinterpret_cast<float*>(a.coef[o]) + (((size_t)row * 2) * a.binsoct + band) * M;
-          float* oim = ore + (size_t)a.binsoct * M;
-#pragma unroll
-          for (int r = 0; r < 16; ++r) {
-            ore[C::out_slot(r, t)] = re[r] * inv_m;
-            oim[C::out_slot(r, t)] = -im[r] * inv_m;
-          }
-        }
-      } else {
-        float2* BS = a.BS + (size_t)row * a.sum_lg + off;
-#pragma unroll
-        for (int r = 0; r < 16; ++r) {
-          int i = C::out_slot(r, t) + half;
-          if (i >= M) i -= M;
-          if (i < lg) {
-            const float w = wst[r * BAND_THREADS + tid];
-            BS[i] = make_float2(re[r] * w, im[r] * w);
-          }
-        }
-      }
-    }
-    __syncthreads();                             // ex is reused by the next row
-  }
-}
-
 // --- octaves with M = 32 ... 4096: packed register FFT (bandfft_v.cuh), 4096 / M bands per CTA (M >= 256) ----------
 // The transform works on float2 register pairs with the two-wide instructions, runs forward or inverse directly (no
 // conjugations), takes the window (and 1 / M) multiply in its first butterflies, and synchronises per band.
 // Inputs of a row are staged one row ahead:
-//   TMA = true : by the TMA engine -- per band ONE 1-D bulk copy (cp.async.bulk + mbarrier, SASS UBLKCP) of the
-//                contiguous window slice X[p - lg/2 .. p + lg/2) (analysis; start rounded down / length rounded up to
-//                16 bytes, the row pitch of X is even) or of the coefficient row (synthesis; two copies for the planar
-//                layout), issued by one thread per synchronisation group right behind the band's first barrier;
-//                no per-thread address / predicate / LDGSTS work in the row loop;
-//   TMA = false: by 16 8-byte cp.async per thread (round 2, first session): any alignment / pitch.
+//   TMA = true : (analysis only) by the TMA engine -- per band ONE 1-D bulk copy (cp.async.bulk + mbarrier, SASS
+//                UBLKCP) of the contiguous window slice X[p - lg/2 .. p + lg/2) (start rounded down / length rounded up
+//                to 16 bytes, the row pitch of X is even), issued by one thread per synchronisation group right behind
+//                the band's first barrier; no per-thread address / predicate / LDGSTS work in the row loop;
+//   TMA = false: by 16 8-byte cp.async per thread: any alignment / pitch.
 template <class C, bool SYNTH, bool TMA>
 __device__ __forceinline__ void band_tile_v(const BandArgs& a, int o, int tile, int row0, int row_end,
                                             unsigned char* smem_raw) {
+  static_assert(!(SYNTH && TMA), "the synthesis stages its coefficient rows with cp.async");
   constexpr int NB = BAND_THREADS / C::TPB, M = C::M, NTWP = (C::NTW + 1) & ~1;
   constexpr int GT = C::TPB < 32 ? 32 : C::TPB;            // threads per synchronisation group (>= one warp)
   constexpr int NG = BAND_THREADS / GT, BPG = GT / C::TPB; // groups per CTA, bands per group
@@ -434,7 +298,6 @@ __device__ __forceinline__ void band_tile_v(const BandArgs& a, int o, int tile, 
       if (i >= M) i -= M;
       wst[r * BAND_THREADS + tid] = (active && i < lg) ? a.win[off + i] : 0.f;
     }
-    if (TMA && t == 0) { s_src[bl] = band; s_cnt[bl] = active ? M : 0; }
   }
   if (TMA && tid < NG) tma::mbar_init(mbar + tid, 1);
   if (TMA) tma::fence_proxy_async();                   // zeros / barrier inits before the first bulk copy
@@ -452,16 +315,7 @@ __device__ __forceinline__ void band_tile_v(const BandArgs& a, int o, int tile, 
       for (int b = 0; b < BPG; ++b) {
         const int bb = grp * BPG + b, cnt = s_cnt[bb];
         if (cnt == 0) continue;
-        float2* dst = stage + bb * SB;
-        if (!SYNTH) {
-          tma::bulk_g2s(dst, a.X + (size_t)row * a.xpitch + s_src[bb], cnt * 8u, bar);
-        } else if (!a.planar) {
-          tma::bulk_g2s(dst, a.coef[o] + ((size_t)row * a.binsoct + s_src[bb]) * M, cnt * 8u, bar);
-        } else {
-          const float* ire = reinterpret_cast<const float*>(a.coef[o]) + (((size_t)row * 2) * a.binsoct + s_src[bb]) * M;
-          tma::bulk_g2s(dst, ire, cnt * 4u, bar);                                          // real plane -> floats [0, M)
-          tma::bulk_g2s(reinterpret_cast<float*>(dst) + M, ire + (size_t)a.binsoct * M, cnt * 4u, bar);   // imaginary
-        }
+        tma::bulk_g2s(stage + bb * SB, a.X + (size_t)row * a.xpitch + s_src[bb], cnt * 8u, bar);
       }
       return;
     }
@@ -501,22 +355,12 @@ __device__ __forceinline__ void band_tile_v(const BandArgs& a, int o, int tile, 
     if (TMA) {
       tma::mbar_wait(mbar + grp, phase);
       phase ^= 1u;
-      if (!SYNTH) {
 #pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) {
-          int i = C::in_slot(n1, t) + half;
-          if (i >= M) i -= M;
-          i = min(max(i + sdelta, 0), SB - 1);           // slots outside the slice carry weight 0
-          z[n1] = stage_b[i];
-        }
-      } else if (!a.planar) {
-#pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) z[n1] = active ? stage_b[C::in_slot(n1, t)] : make_float2(0.f, 0.f);
-      } else {
-        const float* sf = reinterpret_cast<const float*>(stage_b);
-#pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1)
-          z[n1] = active ? make_float2(sf[C::in_slot(n1, t)], sf[M + C::in_slot(n1, t)]) : make_float2(0.f, 0.f);
+      for (int n1 = 0; n1 < 16; ++n1) {
+        int i = C::in_slot(n1, t) + half;
+        if (i >= M) i -= M;
+        i = min(max(i + sdelta, 0), SB - 1);             // slots outside the slice carry weight 0
+        z[n1] = stage_b[i];
       }
     } else {
       cp_async_commit_wait();                         // this thread's own copies: no barrier needed to read them
@@ -661,22 +505,9 @@ __device__ __forceinline__ void band_tile_generic(const BandArgs& a, int o, int 
   }
 }
 
-// V: packed per-band cores (bandfft_v.cuh, default) / round 2's cores (A/B: babe_set_cqt_band_variant(0)).  Separate
-// kernels: one body with both sets inlined is 32 K SASS instructions.
-template <bool SYNTH, bool V, bool TMA>
+template <bool SYNTH, bool TMA>
 __device__ __forceinline__ void band_segment(const BandArgs& a, int o, int tile, int row0, int row_end,
                                              unsigned char* smem_raw) {
-  if (!V) {
-    switch (a.M[o]) {
-      case 256: band_tile_fast<1, SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-      case 512: band_tile_fast<2, SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-      case 1024: band_tile_fast<4, SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-      case 2048: band_tile_fast<8, SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-      case 4096: band_tile_fast<16, SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-      default: band_tile_generic<SYNTH>(a, o, tile, row0, row_end, smem_raw); break;
-    }
-    return;
-  }
   switch (a.M[o]) {                  // analysis = inverse transform of the windowed slice, synthesis = forward
     case 32: band_tile_v<BandCoreS<2, !SYNTH>, SYNTH, TMA>(a, o, tile, row0, row_end, smem_raw); break;
     case 64: band_tile_v<BandCoreS<4, !SYNTH>, SYNTH, TMA>(a, o, tile, row0, row_end, smem_raw); break;
@@ -690,7 +521,7 @@ __device__ __forceinline__ void band_segment(const BandArgs& a, int o, int tile,
   }
 }
 
-template <bool SYNTH, bool V, bool TMA>
+template <bool SYNTH, bool TMA>
 __device__ __forceinline__ void band_tile(const BandArgs& a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // The successor of a band kernel is triggered when a CTA is DONE, not when it starts: the grid is one wave of
@@ -698,8 +529,7 @@ __device__ __forceinline__ void band_tile(const BandArgs& a) {
   // (synthesis 0.155 -> 0.178 ms at B = 64 with the early trigger).
   const int o = find_octave(a, blockIdx.x);
   const int row0 = blockIdx.y * a.rows_per_cta, row_end = min(a.B, row0 + a.rows_per_cta);
-  if (!V) pfa::pdl_wait();                                  // the packed tiles wait behind their own preamble
-  band_segment<SYNTH, V, TMA>(a, o, blockIdx.x - a.tile0[o], row0, row_end, smem_raw);
+  band_segment<SYNTH, TMA>(a, o, blockIdx.x - a.tile0[o], row0, row_end, smem_raw);
   pfa::pdl_launch_dependents();
   if (SYNTH && blockIdx.x == 0 && threadIdx.x < 2)          // the "no band" entries of the rows (a.sum_lg = pitch)
     for (int row = row0; row < row_end; ++row)
@@ -708,14 +538,10 @@ __device__ __forceinline__ void band_tile(const BandArgs& a) {
 
 // analysis: window multiply + fold + per-band inverse FFT of the half spectrum X
 // synthesis, first half: per-band FFT of the coefficients, dual-window multiply -> band spectra BS
-// TMA: inputs staged by bulk copies (default); the cp.async variants serve misaligned inputs and the A/B knob
+// TMA: window slices staged by bulk copies (default); the cp.async analysis serves spectra that cannot be bulk-copied
 template <bool TMA>
-__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_analysis(const BandArgs a) { band_tile<false, true, TMA>(a); }
-template <bool TMA>
-__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_synth_bands(const BandArgs a) { band_tile<true, true, TMA>(a); }
-// the same on round 2's cores
-__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_analysis_r2(const BandArgs a) { band_tile<false, false, false>(a); }
-__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_synth_bands_r2(const BandArgs a) { band_tile<true, false, false>(a); }
+__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_analysis(const BandArgs a) { band_tile<false, TMA>(a); }
+__global__ void __launch_bounds__(BAND_THREADS, 2) k_cqt_synth_bands(const BandArgs a) { band_tile<true, false>(a); }
 
 // overlap-add of the band spectra as a gather, fused with the c2r pre-processing
 struct GatherArgs {
@@ -795,9 +621,8 @@ static int validate_plan(const babe_cqt_plan* p, bool bands) {
   BABE_REQUIRE(p->roots1 && p->roots2 && p->tw_nc && p->tw_ls, BABE_EBADARG, "plan tables missing");
   const size_t smem1 = sizeof(float2) * ((size_t)2 * TILE_SEQ * odd_stride(p->f1.n) + p->f1.n + TW_LO + (p->Nc >> 10) + 1);
   const size_t smem2 = sizeof(float2) * ((size_t)2 * TILE_SEQ * odd_stride(p->f2.n) + p->f2.n);
-  BABE_REQUIRE((smem1 <= 220 * 1024 && smem2 <= 220 * 1024) ||
-                   (tile_fft_smem(p->f1.n) <= 220 * 1024 && tile_fft_smem(p->f2.n) <= 220 * 1024),
-               BABE_EUNSUPPORTED, "pass lengths %d x %d do not fit shared memory", p->f1.n, p->f2.n);
+  BABE_REQUIRE(smem1 <= 220 * 1024 && smem2 <= 220 * 1024, BABE_EUNSUPPORTED,
+               "pass lengths %d x %d do not fit shared memory", p->f1.n, p->f2.n);
   if (bands) {
     BABE_REQUIRE(p->numocts >= 1 && p->numocts <= BABE_MAX_OCTAVES && p->binsoct >= 1, BABE_EBADARG,
                  "bad octave layout");
@@ -861,17 +686,9 @@ static int big_fft(const babe_cqt_plan* p, const float2* in, float2* tmp, float2
 }
 
 
-// ---- second-generation length-Ls transform (cqt_fft.cuh) ---------------------------------------------------
-// 0: tiled passes with fused r2c / c2r / gather (cqt_fft.cuh); -1: round-1 passes.  Measured on B200 (profiles/
-// r02_cqt.md): the tiled passes need 128 registers for the radix-13 / 23 butterflies (2 CTAs per SM) and come out
-// 7-40 % SLOWER than the round-1 passes (80 registers, 3 CTAs per SM) despite two launches fewer, so round 1's are
-// the default.
-//  2 (default): prime-factor passes (cqt_pfa.cuh) for the instantiated lengths, round-1 passes otherwise.
+// 2 (default): prime-factor passes (cqt_pfa.cuh) for the instantiated lengths, round-1 passes otherwise;
+// -1: round-1 passes for every length.
 static int g_cqt_variant = 2;
-static bool tiled_ok(const babe_cqt_plan* p) {
-  return (g_cqt_variant == 0 || g_cqt_variant == 1) && tile_fft_smem(p->f1.n) <= 220 * 1024 &&
-         tile_fft_smem(p->f2.n) <= 220 * 1024;
-}
 
 // ---- programmatic dependent launch of the kernels of a CQT chain (device side: cqt_pfa.cuh) -------------------------
 static int g_cqt_pdl = 15;     // bit mask, A/B: babe_set_cqt_pdl (1: pass-1 kernels, 2: pass-2 kernels, 4: band kernels,
@@ -1000,95 +817,10 @@ static int pfa_filter(const babe_cqt_plan* p, const float2* x, float2* tmpA, flo
 #undef BABE_PFA_DISPATCH
 #undef BABE_PFA_DISPATCH_PLAN
 
-static int launch_f1(const babe_cqt_plan* p, const float2* in, float2* out, int B, int twiddle, int conj_out,
-                     cudaStream_t st) {
-  F1Args a{};
-  a.in = in; a.out = out; a.Nc = p->Nc; a.N1 = p->f1.n; a.N2 = p->f2.n;
-  a.f = to_dev(p->f1); a.roots = reinterpret_cast<const float2*>(p->roots1);
-  a.tw_nc = reinterpret_cast<const float2*>(p->tw_nc);
-  a.twiddle = twiddle; a.conj_out = conj_out;
-  if (g_cqt_variant == 1) {
-    const size_t smem = tile_fft_smem(a.N1, 8);
-    cudaFuncSetAttribute(k_fft_n1<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_fft_n1<8><<<dim3((a.N2 + 7) / 8, B), TF_THREADS, smem, st>>>(a);
-  } else {
-    const size_t smem = tile_fft_smem(a.N1, 16);
-    cudaFuncSetAttribute(k_fft_n1<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_fft_n1<16><<<dim3((a.N2 + 15) / 16, B), TF_THREADS, smem, st>>>(a);
-  }
-  return check_launch("k_fft_n1");
-}
-
-static F2Args f2_args(const babe_cqt_plan* p, const float* scale) {
-  F2Args a{};
-  a.Nc = p->Nc; a.N1 = p->f1.n; a.N2 = p->f2.n;
-  a.f = to_dev(p->f2); a.roots = reinterpret_cast<const float2*>(p->roots2);
-  a.tw_nc = reinterpret_cast<const float2*>(p->tw_nc);
-  a.tw_ls = reinterpret_cast<const float2*>(p->tw_ls);
-  a.scale = scale;
-  return a;
-}
-static int f2_grid(int N1, int half) { return ((N1 - 1) / 2 + half - 1) / half + 1; }
-
-// Y[N1][N2] -> half spectrum X[Nc+1] (times scale)
-static int launch_f2_fwd(const babe_cqt_plan* p, const float2* Y, float2* X, const float* scale, int B,
-                         cudaStream_t st) {
-  F2Args a = f2_args(p, scale);
-  a.Y = Y; a.Xout = X;
-  if (g_cqt_variant == 1) {
-    const size_t smem = tile_fft_smem(a.N2, 8);
-    cudaFuncSetAttribute(k_fft_n2_fwd<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_fft_n2_fwd<8><<<dim3(f2_grid(a.N1, 4), B), TF_THREADS, smem, st>>>(a);
-  } else {
-    const size_t smem = tile_fft_smem(a.N2, 16);
-    cudaFuncSetAttribute(k_fft_n2_fwd<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_fft_n2_fwd<16><<<dim3(f2_grid(a.N1, 8), B), TF_THREADS, smem, st>>>(a);
-  }
-  return check_launch("k_fft_n2_fwd");
-}
-
-// half spectrum X[Nc+1] (times scale), or the synthesis band spectra BS (gather), -> Y[N1][N2]
-static int launch_f2_inv(const babe_cqt_plan* p, const float2* X, const float2* BS, float2* Y, const float* scale,
-                         int B, cudaStream_t st) {
-  F2Args a = f2_args(p, scale);
-  a.X = X; a.Yout = Y;
-  const bool s8 = g_cqt_variant == 1;
-  const size_t smem = tile_fft_smem(a.N2, s8 ? 8 : 16);
-  const dim3 grid(f2_grid(a.N1, s8 ? 4 : 8), B);
-  if (BS != nullptr) {
-    a.BS = BS; a.sum_lg = bs_pitch(p);
-    a.band_p = p->band_p; a.band_lg = p->band_lg; a.band_off = p->band_off; a.jlo = p->bin_jlo; a.jhi = p->bin_jhi;
-  }
-#define BABE_LAUNCH_INV(G, S)                                                                          \
-  do {                                                                                                 \
-    cudaFuncSetAttribute(k_fft_n2_inv<G, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);  \
-    k_fft_n2_inv<G, S><<<grid, TF_THREADS, smem, st>>>(a);                                             \
-  } while (0)
-  if (BS != nullptr) { if (s8) BABE_LAUNCH_INV(true, 8); else BABE_LAUNCH_INV(true, 16); }
-  else { if (s8) BABE_LAUNCH_INV(false, 8); else BABE_LAUNCH_INV(false, 16); }
-#undef BABE_LAUNCH_INV
-  return check_launch("k_fft_n2_inv");
-}
-
-// x[B, Ls] real -> X[B, Nc+1]  (two launches)
-static int tiled_rfft(const babe_cqt_plan* p, const float2* x, float2* tmp, float2* X, const float* scale, int B,
-                      cudaStream_t st) {
-  int rc = launch_f1(p, x, tmp, B, 1, 0, st);
-  if (rc) return rc;
-  return launch_f2_fwd(p, tmp, X, scale, B, st);
-}
-// X[B, Nc+1] (or band spectra) -> x[B, Ls] real  (two launches)
-static int tiled_irfft(const babe_cqt_plan* p, const float2* X, const float2* BS, float2* tmp, float2* x,
-                       const float* scale, int B, cudaStream_t st) {
-  int rc = launch_f2_inv(p, X, BS, tmp, scale, B, st);
-  if (rc) return rc;
-  return launch_f1(p, tmp, x, B, 0, 1, st);
-}
-
-// 1 (default): packed band cores (bandfft_v.cuh), analysis slices staged by TMA bulk copies, synthesis rows by
-// cp.async; 2: cp.async for both; 3: TMA for both; 0: round 2's BandCore / generic Stockham
+// Staging of the analysis band kernel: 1 (default) window slices by TMA bulk copies where the spectrum allows it;
+// 2: cp.async.  The synthesis always stages by cp.async.
 static int g_band_variant = 1;
-static inline int band_r3(int M) {     // M = 256 * R3 handled by BandCore<R3>, else 0
+static inline int band_r3(int M) {     // M = 256 * R3 handled by BandCoreV<R3>, else 0
   switch (M) { case 256: return 1; case 512: return 2; case 1024: return 4; case 2048: return 8;
                case 4096: return 16; default: return 0; }
 }
@@ -1103,7 +835,7 @@ static int fill_band_args(const babe_cqt_plan* p, BandArgs& a, size_t& smem, int
     const int r3 = band_r3(M);
     int tb;
     size_t need;
-    if (g_band_variant != 0 && (M == 32 || M == 64 || M == 128)) {   // BandCoreS<R2>: R2 threads per band
+    if (M == 32 || M == 64 || M == 128) {      // BandCoreS<R2>: R2 threads per band
       const int r2 = M / 16;
       tb = BAND_THREADS / r2;
       need = sizeof(float2) * ((size_t)((tb * (16 * (r2 + 1) + r2) + 1) & ~1) + 2 + 16 * BAND_THREADS + 2 * tb) +
@@ -1155,8 +887,6 @@ extern "C" int babe_rfft(const babe_cqt_plan* plan, const float* x, float* X, in
   if (pfa_id(plan))
     return pfa_rfft(plan, reinterpret_cast<const float2*>(x), w.bufA, reinterpret_cast<float2*>(X), bin_scale, B,
                     plan->Nc + 1, st);
-  if (tiled_ok(plan))
-    return tiled_rfft(plan, reinterpret_cast<const float2*>(x), w.bufA, reinterpret_cast<float2*>(X), bin_scale, B, st);
   rc = big_fft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufB, B, 0, st);
   if (rc) return rc;
   const int n = plan->Nc / 2 + 1;
@@ -1179,9 +909,6 @@ extern "C" int babe_irfft(const babe_cqt_plan* plan, const float* X, float* x, i
   if (pfa_id(plan))
     return pfa_irfft(plan, reinterpret_cast<const float2*>(X), nullptr, w.bufA, reinterpret_cast<float2*>(x),
                      bin_scale, B, st);
-  if (tiled_ok(plan))
-    return tiled_irfft(plan, reinterpret_cast<const float2*>(X), nullptr, w.bufA, reinterpret_cast<float2*>(x),
-                       bin_scale, B, st);
   const int n = plan->Nc / 2 + 1;
   k_irfft_pre<<<dim3((n + 255) / 256, B), 256, 0, st>>>(reinterpret_cast<const float2*>(X), w.bufA,
                                                         plan->Nc,
@@ -1204,11 +931,6 @@ extern "C" int babe_spectral_filter(const babe_cqt_plan* plan, const float* x, f
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (pfa_id(plan))
     return pfa_filter(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufB, reinterpret_cast<float2*>(y), H, B, st);
-  if (tiled_ok(plan)) {
-    rc = tiled_rfft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufX, H, B, st);
-    if (rc) return rc;
-    return tiled_irfft(plan, w.bufX, nullptr, w.bufA, reinterpret_cast<float2*>(y), nullptr, B, st);
-  }
   rc = big_fft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufB, B, 0, st);
   if (rc) return rc;
   const int n = plan->Nc / 2 + 1;
@@ -1235,9 +957,6 @@ extern "C" int babe_cqt_analysis(const babe_cqt_plan* plan, const float* x,
     xpitch = plan->Nc + 2;       // even: rows of the internal spectrum are 16-byte aligned (bulk-copied slices)
     rc = pfa_rfft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufX, nullptr, B, xpitch, st);
     if (rc) return rc;
-  } else if (tiled_ok(plan)) {
-    rc = tiled_rfft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufX, nullptr, B, st);
-    if (rc) return rc;
   } else {
     rc = big_fft(plan, reinterpret_cast<const float2*>(x), w.bufA, w.bufB, B, 0, st);
     if (rc) return rc;
@@ -1259,17 +978,13 @@ extern "C" int babe_cqt_analysis(const babe_cqt_plan* plan, const float* x,
   a.win = win; a.scale = bin_scale; a.X = w.bufX; a.planar = planar ? 1 : 0; a.xpitch = xpitch;
   const dim3 grid(items, (B + a.rows_per_cta - 1) / a.rows_per_cta);
   // bulk-copied window slices need 16-byte aligned rows of X: the internal spectrum buffer of the prime-factor path
-  const bool tma_ok = (a.band_variant == 1 || a.band_variant == 3) && (a.xpitch % 2 == 0) &&
-                      (reinterpret_cast<uintptr_t>(a.X) % 16 == 0);
+  const bool tma_ok = a.band_variant == 1 && (a.xpitch % 2 == 0) && (reinterpret_cast<uintptr_t>(a.X) % 16 == 0);
   if (tma_ok) {
     cudaFuncSetAttribute(k_cqt_analysis<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     launch_chain<4>(k_cqt_analysis<true>, grid, BAND_THREADS, smem, st, a);
-  } else if (a.band_variant) {
+  } else {
     cudaFuncSetAttribute(k_cqt_analysis<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     launch_chain<4>(k_cqt_analysis<false>, grid, BAND_THREADS, smem, st, a);
-  } else {
-    cudaFuncSetAttribute(k_cqt_analysis_r2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_chain<4>(k_cqt_analysis_r2, grid, BAND_THREADS, smem, st, a);
   }
   return check_launch("k_cqt_analysis");
 }
@@ -1295,27 +1010,14 @@ extern "C" int babe_cqt_synthesis(const babe_cqt_plan* plan, const float* const*
   }
   a.win = win; a.scale = nullptr; a.BS = w.bufS; a.planar = planar ? 1 : 0;
   const dim3 grid(items, (B + a.rows_per_cta - 1) / a.rows_per_cta);
-  // bulk-copied coefficient rows (16-byte aligned octave tensors) only on request (variant 3): measured against the
-  // cp.async staging, 68.3 vs 69.8 us at B = 64 but 18.2 vs 16.2 us at B = 8 and 20.2 vs 17.1 us for the planar layout
-  // the sampler uses (two copies per band) -- profiles/r02_cqt.md
-  bool tma_ok = a.band_variant == 3;
-  for (int o = 0; o < plan->numocts; ++o) tma_ok = tma_ok && reinterpret_cast<uintptr_t>(a.coef[o]) % 16 == 0;
-  if (tma_ok) {
-    cudaFuncSetAttribute(k_cqt_synth_bands<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_chain<4>(k_cqt_synth_bands<true>, grid, BAND_THREADS, smem, st, a);
-  } else if (a.band_variant) {
-    cudaFuncSetAttribute(k_cqt_synth_bands<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_chain<4>(k_cqt_synth_bands<false>, grid, BAND_THREADS, smem, st, a);
-  } else {
-    cudaFuncSetAttribute(k_cqt_synth_bands_r2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_chain<4>(k_cqt_synth_bands_r2, grid, BAND_THREADS, smem, st, a);
-  }
+  // coefficient rows staged by cp.async: bulk copies measured 68.3 vs 69.8 us at B = 64 but 18.2 vs 16.2 us at B = 8
+  // and 20.2 vs 17.1 us for the planar layout the sampler uses (two copies per band) -- profiles/r02_cqt.md
+  cudaFuncSetAttribute(k_cqt_synth_bands, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  launch_chain<4>(k_cqt_synth_bands, grid, BAND_THREADS, smem, st, a);
   rc = check_launch("k_cqt_synth_bands");
   if (rc) return rc;
   if (pfa_id(plan) && plan->bin_src != nullptr)   // table-driven overlap-add gather in the prologue of the inverse pass 2
     return pfa_irfft(plan, nullptr, w.bufS, w.bufA, reinterpret_cast<float2*>(x), bin_scale, B, st);
-  if (tiled_ok(plan))       // overlap-add gather + c2r pre-processing in the prologue of the inverse's first pass
-    return tiled_irfft(plan, nullptr, w.bufS, w.bufA, reinterpret_cast<float2*>(x), bin_scale, B, st);
   GatherArgs g{};
   g.BS = w.bufS; g.Zc = w.bufA; g.Nc = plan->Nc; g.sum_lg = bs_pitch(plan);
   g.band_p = plan->band_p; g.band_lg = plan->band_lg; g.band_off = plan->band_off;
@@ -1330,7 +1032,7 @@ extern "C" int babe_cqt_synthesis(const babe_cqt_plan* plan, const float* const*
 
 // profiling / A-B knob (profiles/probe_r02.py): which implementation computes the length-Ls transform
 extern "C" int babe_set_cqt_variant(int v) {
-  if (v < -1 || v > 2) return BABE_EBADARG;
+  if (v != 2 && v != -1) return BABE_EBADARG;
   babe::g_cqt_variant = v;
   return BABE_OK;
 }
@@ -1340,7 +1042,7 @@ extern "C" int babe_set_cqt_pdl(int on) {
   return BABE_OK;
 }
 extern "C" int babe_set_cqt_band_variant(int v) {
-  if (v < 0 || v > 3) return BABE_EBADARG;
+  if (v != 1 && v != 2) return BABE_EBADARG;
   babe::g_band_variant = v;
   return BABE_OK;
 }

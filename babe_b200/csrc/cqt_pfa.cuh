@@ -16,7 +16,7 @@
 // float2 and every stage works IN PLACE with compile-time strides (one buffer, no twiddle tables, no Stockham index
 // arithmetic); the input / output permutations are two small tables built by every CTA.  The odd-prime DFTs keep the
 // (R-1)/2 sums and differences of the mirrored inputs in registers and store every output pair as soon as it is
-// complete, which fits the radix-23 butterfly into 64 registers (round 2's tiled passes kept all R outputs: 128).
+// complete, which fits the radix-23 butterfly into 64 registers (keeping all R outputs takes 128).
 //
 // apply_hpf_DC needs 3 launches instead of 5 (pass 2 runs forward, multiplies by H in the r2c / c2r pair processing
 // and runs backward without leaving shared memory), analysis 2 + 1, synthesis 1 + 2 (the overlap-add of the band

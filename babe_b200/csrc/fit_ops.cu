@@ -265,22 +265,24 @@ __global__ void __launch_bounds__(FIT_THREADS, 1) k_fit_params(const FitArgs a) 
 }
 
 // ---------------------------------------------------------------------------
-// device-resident fit loop, second generation (same arithmetic as k_fit_params above; ~5x less latency per
-// iteration).  Round-1 profile (profiles/r01_fit_params.md): 19.8 K cycles per iteration, half of it a serial
-// section on one lane (chain rule walk, sequential clamps, 11-step binary searches, a K-step chain of
-// log2 / exp10 for the anchors), 40 % the per-bin evaluation with its second log2 and per-bin owner search, the
-// rest three CTA barriers and segment-wise shared-memory reductions.  Here
-//  * every thread owns <= 5 CONTIGUOUS bins whose static data (f, w^2 a, w^2 b) stay in registers; per-segment sums
-//    accumulate in registers and are reduced with one multi-value butterfly per warp (16 double shuffles for 16
-//    values instead of 5 per value) + one pass over the 16 warp partials;
-//  * warp 0 keeps the breakpoint state in the registers of lanes 0..K-1: chain rule from a precomputed
-//    child-of-ancestor table, gradient step, the SEQUENTIAL clamps as shuffle scans (bit-identical to the
-//    reference's order, testing/blind_bwe_sampler.py:576-583), closed-form first-bin search with a table fix-up,
-//    parents by shuffles, gains in parallel and only the anchor products chained;
-//  * two CTA barriers per iteration.
+// device-resident fit loop, cluster kernel (same arithmetic per bin and per breakpoint as k_fit_params above).
+// Round-1 profile (profiles/r01_fit_params.md): 19.8 K cycles per iteration, half of it a serial section on one lane
+// (chain rule walk, sequential clamps, 11-step binary searches, a K-step chain of log2 / exp10 for the anchors), 40 %
+// the per-bin evaluation with its second log2 and per-bin owner search, the rest three CTA barriers and segment-wise
+// shared-memory reductions.  Here
+//  * a thread-block CLUSTER of 4 CTAs shares the bins: every CTA evaluates a quarter of them, and every thread's <= 2
+//    bins keep their static data (f, w^2 a, w^2 b) in registers; per-segment sums accumulate in registers and are
+//    reduced with one multi-value butterfly per warp (16 double shuffles for 16 values instead of 5 per value) + one
+//    pass over the 16 warp partials;
+//  * the 17 per-CTA sums travel to rank 0 through distributed shared memory; rank 0's warp 0 keeps the breakpoint
+//    state in the registers of lanes 0..K-1: chain rule from a precomputed child-of-ancestor table, gradient step, the
+//    SEQUENTIAL clamps as shuffle scans (bit-identical to the reference's order, testing/blind_bwe_sampler.py:576-583),
+//    closed-form first-bin search with a table fix-up, parents by shuffles, gains in parallel and only the anchor
+//    products chained; it writes the next segment tables into every CTA's shared memory;
+//  * two cluster barriers per iteration.
+// Only the association of the fp64 sums over bins differs from k_fit_params (per CTA, then over the 4 CTAs in rank
+// order -- fixed, bitwise reproducible).
 // ---------------------------------------------------------------------------
-constexpr int FIT2_NB = 5;            // bins per thread (F <= 2560)
-
 // sum of NV = 16 doubles per lane over the 32 lanes of a warp with 16 shuffles: after the call lane L holds the
 // total of value (L >> 1) (both lanes of a pair hold it)
 __device__ __forceinline__ double warp_reduce16(double (&v)[16], int lane) {
@@ -319,238 +321,6 @@ __device__ __forceinline__ int reduce16_index(int lane) {
   return ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1);
 }
 
-template <int K>      // exact number of breakpoints (1..8): every loop over breakpoints unrolls, lane tests are predicates
-__global__ void __launch_bounds__(FIT_THREADS, 1) k_fit_params2(const FitArgs a) {
-  constexpr int KP = K;
-  const int F = a.F;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* sf = reinterpret_cast<float*>(smem_raw);                       // bin frequencies
-  __shared__ int s_kf[KMAX];
-  __shared__ float s_fc[KMAX], s_A[KMAX], s_anchor[KMAX];
-  __shared__ double red[FIT_WARPS][17];
-  __shared__ double gS[KMAX], gL[KMAX];
-  __shared__ signed char child[KMAX][KMAX];       // child[i][j]: the ancestor-or-self of i whose parent is j (-1: none)
-  __shared__ float s_lgc[KMAX];                   // log2(f[kf[c]] / fc[parent[c]]) of breakpoint c
-  __shared__ int stop_flag;
-  __shared__ double c_total_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-  // ---- static per-bin data of this thread's contiguous bins ----------------------------------------------
-  const int base = F / FIT_THREADS, rem = F - base * FIT_THREADS;
-  const int nb = base + (tid < rem ? 1 : 0);
-  const int k0 = tid * base + min(tid, rem);
-  float fk[FIT2_NB];
-  double wa[FIT2_NB], wb[FIT2_NB];
-  double ct = 0.0;
-#pragma unroll
-  for (int i = 0; i < FIT2_NB; ++i) {
-    fk[i] = 1.0f; wa[i] = 0.0; wb[i] = 0.0;
-    if (i < nb) {
-      const int k = k0 + i;
-      const double w2 = (double)a.w[k] * (double)a.w[k];
-      fk[i] = a.freqs[k];
-      wa[i] = w2 * a.abc[k];
-      wb[i] = w2 * a.abc[F + k];
-      ct += w2 * a.abc[2 * F + k];
-    }
-  }
-  for (int k = tid; k < F; k += FIT_THREADS) sf[k] = a.freqs[k];
-  ct = warp_sum(ct);
-  if (lane == 0) red[warp][16] = ct;
-  if (tid == 0) stop_flag = 0;
-  __syncthreads();
-  // ---- breakpoint state in the registers of warp 0, lanes 0..K-1 --------------------------------------------
-  const bool bp = warp == 0 && lane < K;
-  float fc = 0.f, A = 0.f, fc_prev = 0.f, A_prev = 0.f;
-  if (bp) { fc = a.params[lane]; A = a.params[K + lane]; }
-  const float df = F > 1 ? (sf[F - 1] - sf[0]) / (float)(F - 1) : 1.0f;
-  const float inv_df = 1.0f / df;
-  double c_total = 0.0;
-
-  // segments of the current (fc, A): kf, parent, gains, anchors, child table -> shared memory (warp 0 only)
-  auto build = [&]() {
-    __syncwarp();                                                // the chain rule has read the previous tables
-    int kf = F, par = -1;
-    float fkf = 0.f, lgc = 0.f, anchor = 1.0f;
-    if (lane < K) {
-      if (fc == fc) {                                           // NaN -> F, like first_bin_ge
-        int k = (int)fminf(fmaxf((fc - sf[0]) * inv_df, 0.f), (float)F);
-        while (k > 0 && sf[k - 1] >= fc) --k;
-        while (k < F && sf[k] < fc) ++k;
-        kf = k;
-      }
-      fkf = kf < F ? sf[kf] : 0.f;
-    }
-#pragma unroll
-    for (int i = 0; i < K; ++i) {                                // parent = last earlier breakpoint at or below
-      const int kfi = __shfl_sync(0xffffffffu, kf, i);
-      if (lane < K && i < lane && kfi <= kf) par = i;
-    }
-    const float fc_p = __shfl_sync(0xffffffffu, fc, par >= 0 ? par : 0);
-    const float A_p = __shfl_sync(0xffffffffu, A, par >= 0 ? par : 0);
-    float g = 1.0f;
-    const bool chained = lane < K && lane > 0 && par >= 0 && kf < F;
-    if (chained) {
-      lgc = log2f(rn_div(fkf, fc_p));
-      g = exp10f(rn_div(rn_mul(A_p, lgc), 20.0f));               // seg_gain(A_p, fc_p, fkf)
-    }
-#pragma unroll
-    for (int i = 1; i < K; ++i) {                                // anchors along the parent chain, in order
-      const float ap = __shfl_sync(0xffffffffu, anchor, par >= 0 ? par : 0);
-      if (lane == i && chained) anchor = rn_mul(g, ap);
-    }
-    if (lane < K) {
-      s_kf[lane] = kf; s_fc[lane] = fc; s_A[lane] = A; s_anchor[lane] = anchor; s_lgc[lane] = lgc;
-#pragma unroll
-      for (int j = 0; j < K; ++j) child[lane][j] = (signed char)(j == lane ? lane : -1);
-    }
-    __syncwarp();
-    int c = lane, q = (lane < K && kf < F) ? par : -1;           // walk this breakpoint's ancestors
-#pragma unroll
-    for (int s2 = 0; s2 < K - 1; ++s2) {
-      if (q >= 0) child[lane][q] = (signed char)c;
-      const int nq = __shfl_sync(0xffffffffu, par, q >= 0 ? q : 0);
-      if (q >= 0) { c = q; q = nq; }
-    }
-    return kf;
-  };
-  int my_kf = F;
-  if (warp == 0) {
-    double s = 0.0;
-    if (lane < FIT_WARPS) s = red[lane][16];
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);     // 16 partials, fixed order
-    if (lane == 0) c_total_s = s;
-    my_kf = build();
-  }
-  __syncthreads();
-  c_total = c_total_s;
-
-  int it = 0;
-  for (int iter = 0; iter < a.cfg.max_iter; ++iter) {
-    // ---- (A) per-bin evaluation, per-segment sums in registers ------------------------------------------
-    double v[16], loss = 0.0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = 0.0;
-    int kfr[KP];
-#pragma unroll
-    for (int i = 0; i < KP; ++i) kfr[i] = i < K ? s_kf[i] : 0x7fffffff;
-    // owners are non-decreasing along a thread's contiguous bins: sums of a run of equal owners are flushed into
-    // the per-segment accumulators only when the owner changes
-    int run_o = -1;
-    double run_u = 0.0, run_l = 0.0;
-#pragma unroll
-    for (int b = 0; b < FIT2_NB; ++b) {
-      if (b < nb) {
-        const int k = k0 + b;
-        int o = -1;
-#pragma unroll
-        for (int i = 0; i < KP; ++i) if (kfr[i] <= k) o = i;
-        float h = 1.0f, lg = 0.f;
-        if (o >= 0) {
-          lg = log2f(rn_div(fk[b], s_fc[o]));
-          const float g = exp10f(rn_div(rn_mul(s_A[o], lg), 20.0f));
-          h = (o == 0) ? g : rn_mul(g, s_anchor[o]);
-        }
-        const double hd = (double)h;
-        loss += hd * (hd * wa[b] - 2.0 * wb[b]);
-        if (o != run_o) {
-#pragma unroll
-          for (int i = 0; i < KP; ++i) if (i == run_o) { v[i] += run_u; v[KP + i] += run_l; }
-          run_o = o; run_u = 0.0; run_l = 0.0;
-        }
-        if (o >= 0) {
-          const double u = (hd * wa[b] - wb[b]) * hd;
-          run_u += u;
-          run_l += u * (double)lg;
-        }
-      }
-    }
-#pragma unroll
-    for (int i = 0; i < KP; ++i) if (i == run_o) { v[i] += run_u; v[KP + i] += run_l; }
-    // ---- (B) block reduction: 2 KP segment sums with one butterfly, the loss with a plain warp sum ----------
-    const double tot = warp_reduce16(v, lane);
-    loss = warp_sum(loss);
-    if ((lane & 1) == 0) red[warp][reduce16_index(lane)] = tot;
-    if (lane == 0) red[warp][16] = loss;
-    __syncthreads();
-    // ---- (C) warp 0: totals, chain rule, step, clamps, stopping test, next segments --------------------------
-    if (warp == 0) {
-      {
-        const int q = lane & 15, hhalf = lane >> 4;              // value q, warps [8 hhalf, 8 hhalf + 8)
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += red[8 * hhalf + w][q];
-        s += __shfl_xor_sync(0xffffffffu, s, 16);
-        if (lane < KP) gS[lane] = s; else if (lane < 2 * KP) gL[lane - KP] = s;
-        double ls = lane < FIT_WARPS ? red[lane][16] : 0.0;
-#pragma unroll
-        for (int o = 8; o > 0; o >>= 1) ls += __shfl_xor_sync(0xffffffffu, ls, o);
-        loss = __shfl_sync(0xffffffffu, ls, 0);
-      }
-      __syncwarp();
-      const double alpha = 0.11512925464970229, ln2 = 0.6931471805599453;
-      if (lane < K) {
-        const int j = lane;
-        double ssum = 0.0, gA = 0.0;
-#pragma unroll
-        for (int i = 0; i < K; ++i) {
-          const int c = child[i][j];
-          if (c < 0 || s_kf[i] >= F) continue;
-          const double Si = gS[i];
-          ssum += Si;
-          gA += (i == j) ? alpha * gL[i] : alpha * (double)s_lgc[c] * Si;
-        }
-        const double gfc = -alpha * (double)A / ((double)fc * ln2) * ssum;
-        const double S = loss + c_total;
-        const double inv_norm = 1.0 / sqrt(S > 0.0 ? S : 0.0);
-        fc = __fsub_rn(fc, __fmul_rn(a.cfg.mu_fc, (float)(gfc * inv_norm)));       // fp32 step (:569)
-        A = __fsub_rn(A, __fmul_rn(a.cfg.mu_A, (float)(gA * inv_norm)));
-      }
-      // sequential clamps (:576-583) as shuffle scans: lane k needs lane k-1's CLAMPED value
-      if (a.cfg.clamp_fc) {
-        if (lane == 0) fc = fminf(fmaxf(fc, a.cfg.fcmin), a.cfg.fcmax);
-#pragma unroll
-        for (int k = 1; k < K; ++k) {
-          const float pv = __shfl_sync(0xffffffffu, fc, k - 1);
-          if (lane == k) fc = fminf(fmaxf(fc, __fadd_rn(pv, 1.0f)), a.cfg.fcmax);
-        }
-      }
-      if (a.cfg.clamp_A) {
-        if (lane == 0) A = fminf(fmaxf(A, a.cfg.Amin), a.cfg.only_negative_A ? -1.0f : a.cfg.Amax);
-#pragma unroll
-        for (int k = 1; k < K; ++k) {
-          const float pv = __shfl_sync(0xffffffffu, A, k - 1);
-          if (lane == k) A = fminf(fmaxf(A, a.cfg.Amin), a.cfg.only_negative_A ? pv : a.cfg.Amax);
-        }
-      }
-      // stopping test (:586-588): mean |delta| of fc and of A, summed in breakpoint order like fit_converged
-      float d0 = lane < K ? fabsf(fc - fc_prev) : 0.f, d1 = lane < K ? fabsf(A - A_prev) : 0.f;
-      float t0 = 0.f, t1 = 0.f;
-#pragma unroll
-      for (int k = 0; k < K; ++k) { t0 += __shfl_sync(0xffffffffu, d0, k); t1 += __shfl_sync(0xffffffffu, d1, k); }
-      if (lane == 0 && iter > 0 && t0 / (float)K < a.cfg.tol_fc && t1 / (float)K < a.cfg.tol_A) stop_flag = 1;
-      fc_prev = fc; A_prev = A;
-      my_kf = build();
-    }
-    __syncthreads();
-    it = iter + 1;
-    if (stop_flag) break;
-  }
-  if (bp) { a.params[lane] = fc; a.params[K + lane] = A; }
-  if (tid == 0 && a.iters_out != nullptr) *a.iters_out = it;
-  (void)my_kf;
-}
-
-// ---------------------------------------------------------------------------
-// device-resident fit loop, third generation: a thread-block CLUSTER of 4 CTAs.  clock64 inside k_fit_params2
-// (profiles/r02_summary.md): the per-bin evaluation + reduction of an iteration is ISSUE-bound on its one SM
-// (16 warps x ~650 instructions in ~2.6 K cycles), the other half is warp 0's serial section.  Here every CTA
-// evaluates a quarter of the bins, the 17 per-CTA sums travel to rank 0 through distributed shared memory, rank 0's
-// warp 0 runs the unchanged serial section and writes the next segment tables into every CTA's shared memory; two
-// cluster barriers per iteration.  Same arithmetic per bin and per breakpoint; only the association of the fp64 sums
-// over bins differs (per CTA, then over the 4 CTAs in rank order -- fixed, bitwise reproducible).
-// ---------------------------------------------------------------------------
 constexpr int FIT3_NC = 4;            // CTAs per cluster
 constexpr int FIT3_NB = 2;            // bins per thread: F <= 4 * 512 * 2
 
@@ -1053,7 +823,7 @@ static int launch_fit3(const FitArgs& a, int B, cudaStream_t st) {
   return check_launch("k_fit_params3");
 }
 
-static int g_fit_variant = 0;     // 0: k_fit_params3 (4-CTA cluster), 1: k_fit_params2 (one CTA), -1: round-1 k_fit_params
+static int g_fit_variant = 0;     // 0: k_fit_params3 (4-CTA cluster) where it applies, -1: round-1 k_fit_params
                                   // (A/B: babe_set_fit_variant; babe_set_fused_variant(-1 / 0) sets it too)
 void set_fit_variant(int v) { g_fit_variant = v; }
 
@@ -1086,7 +856,7 @@ extern "C" int babe_design_filter_vjp(const float* fc, const float* A, int K,
 }
 
 extern "C" int babe_set_fit_variant(int v) {
-  if (v < -1 || v > 1) return BABE_EBADARG;
+  if (v != 0 && v != -1) return BABE_EBADARG;
   babe::set_fit_variant(v);
   return BABE_OK;
 }
@@ -1100,21 +870,6 @@ extern "C" int babe_fit_params(const double* abc, const float* w, const float* f
   FitArgs a{abc, w, freqs, F, params, K, *cfg, iters_out};
   if (K <= 8 && F <= FIT3_NC * FIT_THREADS * FIT3_NB && g_fit_variant == 0) {     // cluster kernel (default)
     return launch_fit3<false>(a, 1, static_cast<cudaStream_t>(stream));
-  }
-  if (K <= 8 && F <= FIT_THREADS * FIT2_NB && g_fit_variant >= 0) {     // second-generation kernel
-    const size_t smem2 = (size_t)F * sizeof(float) + 16;
-    cudaStream_t st2 = static_cast<cudaStream_t>(stream);
-    switch (K) {
-      case 1: k_fit_params2<1><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 2: k_fit_params2<2><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 3: k_fit_params2<3><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 4: k_fit_params2<4><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 5: k_fit_params2<5><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 6: k_fit_params2<6><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      case 7: k_fit_params2<7><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-      default: k_fit_params2<8><<<1, FIT_THREADS, smem2, st2>>>(a); break;
-    }
-    return check_launch("k_fit_params2");
   }
   cudaFuncSetAttribute(k_fit_params, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   k_fit_params<<<1, FIT_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(a);

@@ -78,15 +78,15 @@ int babe_get_fused_variant(void);
  *    2 (default)  prime-factor passes (csrc/cqt_pfa.cuh) for the instantiated lengths (Ls = 184184, 368368):
  *                 twiddle-free in-place stages, r2c / c2r / filter / synthesis gather fused into pass 2
  *                 (2 launches per transform, 3 for the spectral filter); other lengths run variant -1;
- *    0, 1         round 2's tiled passes (csrc/cqt_fft.cuh), 16 / 8 sequences per CTA -- slower, kept for A/B;
- *   -1            the round-1 generic mixed-radix passes with separate post / pre / gather kernels. */
+ *   -1            the round-1 generic mixed-radix passes with separate post / pre / gather kernels.
+ * Other values return BABE_EBADARG and leave the setting unchanged. */
 int babe_set_cqt_variant(int variant);
 int babe_get_cqt_variant(void);
-/* Band kernels of babe_cqt_analysis / babe_cqt_synthesis: 1 (default) packed register FFTs with per-band
- * synchronisation for every octave size 32 ... 4096 (csrc/bandfft_v.cuh); the analysis stages each band's window slice
- * of the spectrum with one TMA bulk copy per row, the synthesis its coefficient rows with cp.async (faster at the
- * sampler's batch and planar layout); 2: cp.async staging for both (also serves misaligned inputs); 3: TMA staging
- * for both; 0: round 2's cores (A/B). */
+/* Band kernels of babe_cqt_analysis / babe_cqt_synthesis: packed register FFTs with per-band synchronisation for every
+ * octave size 32 ... 4096 (csrc/bandfft_v.cuh); the synthesis stages its coefficient rows with cp.async (faster at the
+ * sampler's batch and planar layout).  The analysis stages each band's window slice of the spectrum with 1 (default)
+ * one TMA bulk copy per row where the spectrum allows it (even row pitch, 16-byte aligned), cp.async otherwise;
+ * 2: cp.async always.  Other values return BABE_EBADARG and leave the setting unchanged. */
 int babe_set_cqt_band_variant(int variant);
 /* Programmatic dependent launch of the kernels of a CQT call: each kernel lets its successor start while its own last
  * wave runs and waits (griddepcontrol.wait) only before it touches the chain's buffers.  Bit mask of the kernels
@@ -216,8 +216,9 @@ typedef struct {
   int clamp_fc, clamp_A, only_negative_A;
 } babe_fit_config;
 /* Which kernel runs the loop: 0 (default) k_fit_params3, a cluster of 4 CTAs (each evaluates a quarter of the bins,
- * sums gathered through distributed shared memory, one serial warp); 1 k_fit_params2 (one CTA); -1 round 1's
- * k_fit_params.  babe_set_fused_variant(-1 / 0) sets it too. */
+ * sums gathered through distributed shared memory, one serial warp) for K <= 8 and F <= 4096, round 1's
+ * k_fit_params otherwise; -1 k_fit_params always.  Other values return BABE_EBADARG and leave the setting unchanged.
+ * babe_set_fused_variant(-1 / 0) sets it too. */
 int babe_set_fit_variant(int variant);
 int babe_fit_params(const double* abc, const float* w, const float* freqs, int F,
                     float* params, int K, const babe_fit_config* cfg_host,
@@ -225,7 +226,7 @@ int babe_fit_params(const double* abc, const float* w, const float* freqs, int F
 /* B independent fits: abc[B,3F] (babe_stft_stats_rows), params[B,2,K] updated in place, iters_out int[B]
  * (optional); clamps and the stopping test apply per row.  Row b's result is bitwise what babe_fit_params gives
  * on abc[b], params[b].  Fit variant 0 with K <= 8 and F <= 4096 launches B clusters of k_fit_params3 (cluster b
- * fits row b); the other variants and sizes call babe_fit_params once per row. */
+ * fits row b); variant -1 and other sizes call babe_fit_params once per row. */
 int babe_fit_params_rows(const double* abc, const float* w, const float* freqs, int F,
                          float* params, int B, int K, const babe_fit_config* cfg_host,
                          int* iters_out, void* stream);

@@ -7,7 +7,7 @@ dev = torch.device("cuda")
 cq = CQT_nsgt(7, 64, mode="oct", window=("kaiser", 1), fs=22050, audio_len=184184, device=dev)
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 64
 if len(sys.argv) > 2:
-    lib().babe_set_cqt_band_variant(int(sys.argv[2]))
+    assert lib().babe_set_cqt_band_variant(int(sys.argv[2])) == 0, "band variant: 1 (default) or 2"
 xc = torch.randn(B, 184184, device=dev) * 0.063
 for _ in range(2):
     cs = cq.fwd(xc.unsqueeze(1))

@@ -37,6 +37,14 @@ def test_version_and_errors(handle):
         _lib.check(rc, "tables")
 
 
+def test_kernel_selection_rejects_removed_values(handle):
+    """The A/B setters accept only the implementations the library still has; a rejected value changes nothing."""
+    for setter, v in [("babe_set_cqt_variant", 0), ("babe_set_cqt_variant", 1), ("babe_set_cqt_band_variant", 0),
+                      ("babe_set_cqt_band_variant", 3), ("babe_set_fit_variant", 1)]:
+        assert getattr(handle, setter)(v) == _lib.BABE_EBADARG, (setter, v)
+    assert handle.babe_get_cqt_variant() == 2
+
+
 def test_host_tables(handle):
     for nfft in (512, 1024, 2048, 4096):
         win = np.empty(nfft, np.float32)

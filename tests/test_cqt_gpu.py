@@ -137,20 +137,18 @@ def test_planar_layout_matches_interleaved(CQT):
         assert rel_l2(gp.cpu(), torch.view_as_real(gc.squeeze(1)).permute(0, 3, 1, 2).cpu()) < 1e-6
 
 
-@pytest.mark.parametrize("variant", [-1, 0, 1])
 @pytest.mark.parametrize("numocts,binsoct,fs,Ls,B", [(4, 12, 22050, 8192, 3), (7, 64, 22050, 184184, 2),
                                                      (7, 64, 22050, 132300, 1), (8, 96, 44100, 485100, 1)])
-def test_tiled_passes_vs_oracle(CQT, variant, numocts, binsoct, fs, Ls, B):
-    """The other implementations of the length-Ls transform kept in the library (`babe_set_cqt_variant`: -1 = round 1's
-    generic passes, which also serve every length the prime-factor passes are not instantiated for; 0 / 1 = round 2's
-    tiled passes of csrc/cqt_fft.cuh) against the same oracle.  The default (2 = prime-factor passes of
-    csrc/cqt_pfa.cuh for Ls = 184184 and 368368) is what every other test in this file runs."""
+def test_generic_passes_vs_oracle(CQT, numocts, binsoct, fs, Ls, B):
+    """Round 1's generic passes of the length-Ls transform (`babe_set_cqt_variant(-1)`), which serve every length the
+    prime-factor passes are not instantiated for, forced onto every length here, against the same oracle.  The default
+    (2 = prime-factor passes of csrc/cqt_pfa.cuh where instantiated) is what every other test in this file runs."""
     from babe_b200._lib import lib
     cq, ref = _pair(CQT, numocts, binsoct, fs, Ls)
     g = torch.Generator().manual_seed(Ls + 1)
     x = torch.randn(B, Ls, generator=g) * 0.063
     xc = x.cuda()
-    assert lib().babe_set_cqt_variant(variant) == 0
+    assert lib().babe_set_cqt_variant(-1) == 0
     try:
         X = cq.rfft(xc)
         Xr = torch.fft.rfft(x.double(), dim=-1)
@@ -166,13 +164,12 @@ def test_tiled_passes_vs_oracle(CQT, variant, numocts, binsoct, fs, Ls, B):
         lib().babe_set_cqt_variant(2)
 
 
-@pytest.mark.parametrize("band_variant", [0, 2, 3])
+@pytest.mark.parametrize("band_variant", [2])
 @pytest.mark.parametrize("numocts,binsoct,fs,Ls,B", [(7, 64, 22050, 184184, 2), (4, 12, 22050, 8192, 3)])
 def test_other_band_kernels_vs_oracle(CQT, band_variant, numocts, binsoct, fs, Ls, B):
-    """`babe_set_cqt_band_variant`: 0 = round 2's band kernels (BandCore on split re / im registers, CTA-wide barriers,
-    generic Stockham for the octaves below 256 points); 2 / 3 = the packed per-band cores of csrc/bandfft_v.cuh with
-    cp.async / TMA bulk-copy staging on BOTH directions (the default, 1, stages the analysis slices by TMA and the
-    synthesis rows by cp.async and is what every other test runs).  Complex and planar layouts."""
+    """`babe_set_cqt_band_variant(2)`: the analysis band kernel stages its window slices by cp.async, as it does for
+    every spectrum that cannot be bulk-copied, here also at the prime-factor lengths (the default, 1, stages them by TMA
+    bulk copies wherever it can and is what every other test runs).  Complex and planar layouts."""
     from babe_b200._lib import lib
     cq, ref = _pair(CQT, numocts, binsoct, fs, Ls)
     g = torch.Generator().manual_seed(Ls + 2)

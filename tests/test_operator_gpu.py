@@ -231,9 +231,9 @@ def test_fit_params_vs_oracle(golden):
 
 
 def test_fit_kernels_agree_bitwise(golden):
-    """The three generations of the fit loop -- round 1's k_fit_params (-1), the one-CTA k_fit_params2 (1) and the default
-    4-CTA cluster kernel k_fit_params3 (0: bins split over the CTAs, sums through distributed shared memory) -- evaluate
-    the same fp32 / fp64 expressions; only the association of the fp64 sums over bins differs.  Their 100-iteration
+    """The two fit loops -- round 1's k_fit_params (-1), which also serves K > 8 and F > 4096, and the default 4-CTA
+    cluster kernel k_fit_params3 (0: bins split over the CTAs, sums through distributed shared memory) -- evaluate the
+    same fp32 / fp64 expressions; only the association of the fp64 sums over bins differs.  Their 100-iteration
     trajectories agree to the last bit on the goldens' inputs (K = 5, K = 7, NFFT 1024) and on a 4096-point case."""
     from babe_b200 import ops, sampler
     from babe_b200._lib import lib
@@ -249,13 +249,13 @@ def test_fit_kernels_agree_bitwise(golden):
     try:
         for n, xd, yy, p0 in cases:
             out = {}
-            for v in (-1, 1, 0):
+            for v in (-1, 0):
                 assert lib().babe_set_fit_variant(v) == 0
                 fit = sampler.FilterFit(nfft=n, sample_rate=22050 if n == 4096 else sr, max_iter=100, device="cuda")
                 p, its = fit(xd, yy, p0.clone(), return_iters=True)
                 out[v] = (p.cpu(), int(its))
-            assert out[0][1] == out[1][1] == out[-1][1]
-            assert torch.equal(out[0][0], out[1][0]) and torch.equal(out[1][0], out[-1][0])
+            assert out[0][1] == out[-1][1]
+            assert torch.equal(out[0][0], out[-1][0])
     finally:
         lib().babe_set_fit_variant(0)
 
