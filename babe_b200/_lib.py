@@ -72,6 +72,10 @@ SIGNATURES = {
                                        c_void_p, c_void_p, c_void_p, c_int, c_int,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p,
                                        c_void_p]),
+    "babe_apply_filter_rows_known": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                             c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p,
+                                             c_void_p, c_void_p]),
     "babe_stft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                           c_int, c_void_p, c_void_p]),
     "babe_istft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,

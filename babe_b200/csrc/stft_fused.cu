@@ -89,7 +89,12 @@ constexpr size_t fused_smem_bytes() {
 //      3 any combination decided at run time
 // ROWS: one filter per row, fc / A are [B, K] and status is int[B]; H is (re)designed whenever the CTA's
 //       segment loop enters a new row, between two segments, when no bulk copy is in flight
-template <bool ADJ, int EPI, bool ROWS>
+// MASK (ROWS only): known-prefix observation model D_b x = m_b x + (1 - m_b) A_b x with m_b[n] = 1[n < kn],
+//       kn = known[row] (kn <= 0: no mask, kn >= T: every sample known).  Forward: samples n < kn of the output are
+//       x itself; adjoint: D_b^T x = A_b^T (x 1[n >= kn]) + x 1[n < kn].  Only the frame pairs and output blocks of the
+//       prefix take a branch (pair- / block-uniform): the adjoint zeroes their staged samples below kn at read time,
+//       the epilogues read x from global memory (the stage has been recycled by then).
+template <bool ADJ, int EPI, bool ROWS, bool MASK = false>
 __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
   using C = Core4k;
   constexpr bool SUBSTAGE = EPI == 1 || EPI == 3;
@@ -182,6 +187,7 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
     float* yr = a.y + (size_t)row * a.T;
     const float* subr = has_sub ? a.sub + (size_t)row * a.T : nullptr;
     const float rs = has_scale ? a.row_scale[row] : 1.0f;
+    const int kn = MASK ? a.known[row] : 0;
     float carry[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) carry[i] = 0.f;
@@ -204,6 +210,11 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
         } else {
 #pragma unroll
           for (int j = 0; j < 24; ++j) xs[j] = (base + 256 * j < a.T) ? stage[256 * j + t] : 0.f;
+        }
+        if (MASK && ADJ && (long long)fA * C::HOP < kn) {
+          // D^T: the known samples do not go through the filter
+#pragma unroll
+          for (int j = 0; j < 24; ++j) xs[j] = (base + 256 * j < kn) ? 0.f : xs[j];
         }
         if (ADJ && fA == 0) {
           // input block 0 is covered by one frame only: divide by w^2 instead of the interior envelope
@@ -272,11 +283,13 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
         if (blk < j0 || blk >= j1) continue;
         const long long p0 = (long long)blk * C::HOP;
         float* yb = yr + p0;
+        const bool pre = MASK && p0 < kn;                        // block overlaps the known prefix
         if (p0 + C::HOP <= a.T) {
 #pragma unroll
           for (int n1 = 0; n1 < 8; ++n1) {
             float v = o[8 * half + n1];
             const int r = 256 * n1 + t;
+            if (pre && p0 + r < kn) v = ADJ ? v + xr[p0 + r] : xr[p0 + r];
             if (SUBSTAGE && has_sub) v -= substage[C::HOP * half + r];
             if (has_scale) v *= rs;
             yb[r] = v;
@@ -288,6 +301,7 @@ __global__ void __launch_bounds__(256, 2) k_filter_fused(const FusedArgs a) {
             float v = o[8 * half + n1];
             const int r = 256 * n1 + t;
             if (p0 + r < a.T) {
+              if (pre && p0 + r < kn) v = ADJ ? v + xr[p0 + r] : xr[p0 + r];
               if (SUBSTAGE && has_sub) v -= substage[C::HOP * half + r];
               if (has_scale) v *= rs;
               yb[r] = v;
@@ -622,12 +636,12 @@ static int fused_run_length(int B, int nblk) {
   return (int)q;
 }
 
-template <bool ADJ, int EPI, bool ROWS>
+template <bool ADJ, int EPI, bool ROWS, bool MASK>
 static int launch_epi(FusedArgs a, cudaStream_t st) {
   const long long total = (long long)a.B * a.nblk;
   const int grid = (int)((total + a.q - 1) / a.q);
   constexpr size_t smem = fused_smem_bytes<EPI == 1 || EPI == 3>();
-  auto kern = k_filter_fused<ADJ, EPI, ROWS>;
+  auto kern = k_filter_fused<ADJ, EPI, ROWS, MASK>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   kern<<<grid, 256, smem, st>>>(a);
   return check_launch("k_filter_fused");
@@ -645,17 +659,17 @@ size_t fused_sumsq_slots(int B, int T) {
   return (size_t)((total + q - 1) / q) + (size_t)B;
 }
 
-template <bool ROWS>
+template <bool ROWS, bool MASK>
 static int launch_variant(const FusedArgs& a, cudaStream_t st) {
   const bool sub = a.sub != nullptr, sc = a.row_scale != nullptr, ss = a.item_sumsq != nullptr;
   if (a.adjoint) {
-    if (!sub && !sc && !ss) return launch_epi<true, 0, ROWS>(a, st);
-    if (!sub && sc && !ss) return launch_epi<true, 2, ROWS>(a, st);
-    return launch_epi<true, 3, ROWS>(a, st);
+    if (!sub && !sc && !ss) return launch_epi<true, 0, ROWS, MASK>(a, st);
+    if (!sub && sc && !ss) return launch_epi<true, 2, ROWS, MASK>(a, st);
+    return launch_epi<true, 3, ROWS, MASK>(a, st);
   }
-  if (!sub && !sc && !ss) return launch_epi<false, 0, ROWS>(a, st);
-  if (sub && !sc && ss) return launch_epi<false, 1, ROWS>(a, st);
-  return launch_epi<false, 3, ROWS>(a, st);
+  if (!sub && !sc && !ss) return launch_epi<false, 0, ROWS, MASK>(a, st);
+  if (sub && !sc && ss) return launch_epi<false, 1, ROWS, MASK>(a, st);
+  return launch_epi<false, 3, ROWS, MASK>(a, st);
 }
 
 int launch_filter_fused(FusedArgs a, double* row_sumsq, cudaStream_t st) {
@@ -663,7 +677,8 @@ int launch_filter_fused(FusedArgs a, double* row_sumsq, cudaStream_t st) {
   a.nblk = (a.T - 1) / Core4k::HOP + 1;
   a.q = fused_run_length(a.B, a.nblk);
   const bool ss = a.item_sumsq != nullptr;
-  const int rc = a.per_row ? launch_variant<true>(a, st) : launch_variant<false>(a, st);
+  const int rc = !a.per_row ? launch_variant<false, false>(a, st)
+                 : a.known != nullptr ? launch_variant<true, true>(a, st) : launch_variant<true, false>(a, st);
   if (rc || !ss) return rc;
   k_segment_sumsq<<<a.B, 1, 0, st>>>(a.item_sumsq, a.nblk, a.q, row_sumsq);
   return check_launch("k_segment_sumsq");

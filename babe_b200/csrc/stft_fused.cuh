@@ -9,7 +9,11 @@ namespace babe {
 struct FusedArgs {
   const float* x; float* y; int B, T;
   const float* window; const float2* roots;            // periodic Hamming window (N), exp(-2 pi i m / N)
-  const float* H; const float* freqs; const float* fc; const float* A; int K;
+  // H: shared filter (NULL: designed from fc, A).  known (per_row only, NULL = none): int[B] known-prefix lengths of
+  // the masked operator.  The per-row kernels never read H; sharing its slot keeps the parameter block at 128 bytes
+  // (a larger block changes the code ptxas generates for every existing instantiation).
+  union { const float* H; const int* known; };
+  const float* freqs; const float* fc; const float* A; int K;
   int adjoint;
   const float* sub; const float* row_scale; double* item_sumsq;
   int* status;

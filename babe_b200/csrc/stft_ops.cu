@@ -1000,6 +1000,100 @@ extern "C" int babe_apply_filter_rows(const float* x, float* y, int B, int T, in
   return BABE_OK;
 }
 
+// ---------------------------------------------------------------------------
+// Known-prefix masked operator D_b x = m_b x + (1 - m_b) A_b x, m_b[n] = 1[n < known[b]] (the autoregressive
+// observation model: the head of a window is known from the previous one).  NFFT = 4096 rows that can be
+// bulk-copied run the MASK instantiations of k_filter_fused; every other case filters with babe_apply_filter_rows
+// (the adjoint on a copy of x with its prefix zeroed) and k_known_prefix_epilogue applies the prefix, sub,
+// row_scale and the row sum of squares.
+// ---------------------------------------------------------------------------
+// xm[b, n] = n < known[b] ? 0 : x[b, n]
+__global__ void k_zero_known_prefix(const float* x, float* xm, int T, const int* known) {
+  const int b = blockIdx.y, kn = known[b];
+  const float* xr = x + (size_t)b * T;
+  float* mr = xm + (size_t)b * T;
+  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < T; n += gridDim.x * blockDim.x) mr[n] = n < kn ? 0.f : xr[n];
+}
+
+// y = ((n < known ? (ADJ ? y + x : x) : y) - sub) * row_scale; row_sumsq[b] += sum y^2 (one CTA per row, fixed order)
+__global__ void __launch_bounds__(256) k_known_prefix_epilogue(const float* x, float* y, int T, const int* known,
+                                                               int adjoint, const float* sub, const float* row_scale,
+                                                               double* row_sumsq) {
+  __shared__ double part[8];
+  const int b = blockIdx.x, kn = known[b];
+  const float* xr = x + (size_t)b * T;
+  float* yr = y + (size_t)b * T;
+  const float* sr = sub ? sub + (size_t)b * T : nullptr;
+  const float rs = row_scale ? row_scale[b] : 1.0f;
+  double acc = 0.0;
+  for (int n = threadIdx.x; n < T; n += 256) {
+    float v = yr[n];
+    if (n < kn) v = adjoint ? v + xr[n] : xr[n];
+    if (sr) v -= sr[n];
+    if (row_scale) v *= rs;
+    yr[n] = v;
+    acc += (double)v * (double)v;
+  }
+  if (row_sumsq == nullptr) return;
+  acc = warp_sum(acc);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < 8; ++w) s += part[w];
+    row_sumsq[b] += s;
+  }
+}
+
+extern "C" int babe_apply_filter_rows_known(const float* x, float* y, int B, int T, int nfft,
+                                            const float* window, const float* twiddle,
+                                            const float* freqs, const float* fc, const float* A, int K,
+                                            int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
+                                            void* workspace, size_t workspace_bytes, int* status, const int* known,
+                                            void* stream) {
+  if (known == nullptr)
+    return babe_apply_filter_rows(x, y, B, T, nfft, window, twiddle, freqs, fc, A, K, adjoint, sub, row_scale,
+                                  row_sumsq, workspace, workspace_bytes, status, stream);
+  BABE_REQUIRE(x && y && window && twiddle, BABE_EBADARG, "apply_filter_rows_known: null pointer");
+  BABE_REQUIRE(B >= 0 && T >= 0, BABE_EBADARG, "apply_filter_rows_known: bad shape B=%d T=%d", B, T);
+  BABE_REQUIRE(freqs && fc && A && K >= 1 && K <= BABE_MAX_BREAKPOINTS, BABE_EBADARG,
+               "apply_filter_rows_known: need (freqs, fc, A, 1<=K<=%d)", BABE_MAX_BREAKPOINTS);
+  BABE_REQUIRE(babe_stft_supported(nfft), BABE_EUNSUPPORTED, "unsupported NFFT %d", nfft);
+  if (B == 0 || T == 0) return BABE_OK;
+  const float* sub_ = adjoint ? nullptr : sub;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (nfft == 4096 && fused_filter_eligible(x, sub_, T)) {
+    FusedArgs f{};
+    f.x = x; f.y = y; f.B = B; f.T = T; f.window = window; f.roots = reinterpret_cast<const float2*>(twiddle);
+    f.freqs = freqs; f.fc = fc; f.A = A; f.K = K; f.adjoint = adjoint;
+    f.sub = sub_; f.row_scale = row_scale; f.status = status; f.per_row = 1; f.known = known;
+    if (row_sumsq != nullptr) {
+      BABE_REQUIRE(workspace != nullptr && workspace_bytes >= fused_sumsq_slots(B, T) * sizeof(double), BABE_EBADARG,
+                   "apply_filter_rows_known: row_sumsq needs a workspace of babe_apply_filter_workspace() bytes");
+      f.item_sumsq = static_cast<double*>(workspace);
+    }
+    return launch_filter_fused(f, row_sumsq, st);
+  }
+  float* xm = nullptr;
+  if (adjoint) {
+    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&xm), (size_t)B * T * sizeof(float), st);
+    BABE_REQUIRE(e == cudaSuccess, BABE_ECUDA, "apply_filter_rows_known: %s", cudaGetErrorString(e));
+    k_zero_known_prefix<<<dim3((unsigned)std::min((T + 255) / 256, 1024), B), 256, 0, st>>>(x, xm, T, known);
+    int rc = check_launch("k_zero_known_prefix");
+    if (rc == BABE_OK)
+      rc = babe_apply_filter_rows(xm, y, B, T, nfft, window, twiddle, freqs, fc, A, K, 1, nullptr, nullptr, nullptr,
+                                  nullptr, 0, status, stream);
+    cudaFreeAsync(xm, st);
+    if (rc) return rc;
+  } else {
+    const int rc = babe_apply_filter_rows(x, y, B, T, nfft, window, twiddle, freqs, fc, A, K, 0, nullptr, nullptr,
+                                          nullptr, nullptr, 0, status, stream);
+    if (rc) return rc;
+  }
+  k_known_prefix_epilogue<<<B, 256, 0, st>>>(x, y, T, known, adjoint, sub_, row_scale, row_sumsq);
+  return check_launch("k_known_prefix_epilogue");
+}
+
 extern "C" size_t babe_stft_stats_rows_workspace(int B, int T, int nfft) {
   if (!babe_stft_supported(nfft) || B < 1 || T < 1) return 0;
   const size_t fallback = babe_stft_stats_workspace(1, T, nfft);

@@ -165,10 +165,20 @@ def _row_params(x, fc, A):
 
 
 def apply_filter_rows(x, nfft, freqs, fc, A, adjoint=False, sub=None, row_scale=None, row_sumsq=None, out=None,
-                      status=None):
+                      status=None, known=None):
     """``apply_filter`` with one filter per row: row b of x[B,T] goes through the H designed from fc[b], A[b]
-    (fc, A: (B, K)).  ``status`` (optional int32[B]) flags the rows whose design the reference would reject."""
+    (fc, A: (B, K)).  ``status`` (optional int32[B]) flags the rows whose design the reference would reject.
+
+    ``known`` (optional int32[B] CUDA tensor) switches to the known-prefix masked operator of the autoregressive
+    windows, D_b x = m_b x + (1 - m_b) A_b x with m_b[n] = 1 for n < known[b]: the forward passes samples
+    n < known[b] through unfiltered, the adjoint is D_b^T (``babe_apply_filter_rows_known``)."""
     _row_params(x, fc, A)
+    if known is not None:
+        if not (torch.is_tensor(known) and known.is_cuda and known.dtype == torch.int32 and known.dim() == 1
+                and known.numel() == x.shape[0] and known.device == x.device):
+            what = f"{known.dtype} {tuple(known.shape)} on {known.device}" if torch.is_tensor(known) else type(known).__name__
+            raise ValueError(f"known must be an int32[{x.shape[0]}] tensor on {x.device}, got {what}")
+        known = known.contiguous()
     x = _cuda_f32(x, "x")
     fc = _cuda_f32(fc, "fc")
     A = _cuda_f32(A, "A")
@@ -195,6 +205,14 @@ def apply_filter_rows(x, nfft, freqs, fc, A, adjoint=False, sub=None, row_scale=
     if row_sumsq is not None:
         nbytes = lib().babe_apply_filter_workspace(B, T, int(nfft))
         ws = torch.empty(nbytes // 8, dtype=torch.float64, device=x.device)
+    if known is not None:
+        with profiling.op("apply_filter_rows_known_adj" if adjoint else "apply_filter_rows_known",
+                          2 if row_sumsq is not None else 1, (12 if sub is not None else 8) * B * T):
+            check(lib().babe_apply_filter_rows_known(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), _p(freqs), _p(fc),
+                                                     _p(A), K, int(bool(adjoint)), _p(sub), _p(row_scale),
+                                                     _p(row_sumsq), _p(ws), nbytes, _p(status), _p(known), _stream()),
+                  "apply_filter_rows_known")
+        return y
     with profiling.op("apply_filter_rows_adj" if adjoint else "apply_filter_rows",
                       2 if row_sumsq is not None else 1, (12 if sub is not None else 8) * B * T):
         check(lib().babe_apply_filter_rows(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), _p(freqs), _p(fc), _p(A),

@@ -150,13 +150,16 @@ class FilterFit:
 class _RecGuidanceNorm(torch.autograd.Function):
     """norm_b = || y_b - A_{fc,A}(x_b) ||_2  (testing/blind_bwe_sampler.py:89,117)
     with backward  g_b * A^T((A x_b - y_b) / norm_b)  (what :120 back-propagates
-    into the denoiser).  H is designed inside both kernels; fc, A of shape (B, K) give every row its own filter."""
+    into the denoiser).  H is designed inside both kernels; fc, A of shape (B, K) give every row its own filter.
+    ``known`` (int32[B], per-row filters only) replaces A by the known-prefix operator of the autoregressive windows,
+    D_b x = m_b x + (1 - m_b) A_b x with m_b[n] = 1[n < known[b]] (:259-303), and the backward applies D_b^T."""
 
     @staticmethod
-    def forward(ctx, x, y, freqs, fc, A, nfft):
+    def forward(ctx, x, y, freqs, fc, A, nfft, known=None):
         ss = torch.zeros(x.shape[0], dtype=torch.float64, device=x.device)
+        ctx.masked = {} if known is None else {"known": known}       # unmasked calls keep their exact signature
         if fc.dim() == 2:
-            r = ops.apply_filter_rows(x, nfft, freqs, fc, A, sub=y, row_sumsq=ss)
+            r = ops.apply_filter_rows(x, nfft, freqs, fc, A, sub=y, row_sumsq=ss, **ctx.masked)
         else:
             r = ops.apply_filter(x, nfft, freqs=freqs, fc=fc, A=A, sub=y, row_sumsq=ss)
         norms = torch.sqrt(ss).to(torch.float32)
@@ -170,16 +173,28 @@ class _RecGuidanceNorm(torch.autograd.Function):
         r, norms, freqs, fc, A = ctx.saved_tensors
         scale = (g / norms).contiguous()
         if fc.dim() == 2:
-            gx = ops.apply_filter_rows(r, ctx.nfft, freqs, fc, A, adjoint=True, row_scale=scale)
+            gx = ops.apply_filter_rows(r, ctx.nfft, freqs, fc, A, adjoint=True, row_scale=scale, **ctx.masked)
         else:
             gx = ops.apply_filter(r, ctx.nfft, freqs=freqs, fc=fc, A=A, adjoint=True, row_scale=scale)
-        return gx, None, None, None, None, None
+        return gx, None, None, None, None, None, None
 
 
-def rec_guidance_norms(x, y, freqs, filter_params, nfft):
-    """filter_params (2, K): one filter for all rows; (B, 2, K): row b filtered with filter_params[b]."""
+def rec_guidance_norms(x, y, freqs, filter_params, nfft, known=None):
+    """filter_params (2, K): one filter for all rows; (B, 2, K): row b filtered with filter_params[b].  ``known``
+    (int32[B] CUDA tensor, with (B, 2, K) only): the norms of the known-prefix masked operator (``_RecGuidanceNorm``)."""
     fc, A = (filter_params[:, 0], filter_params[:, 1]) if filter_params.dim() == 3 else filter_params
-    return _RecGuidanceNorm.apply(x, y, freqs, fc.contiguous(), A.contiguous(), int(nfft))
+    if known is not None and filter_params.dim() != 3:
+        raise ValueError("known-prefix guidance needs per-row (B, 2, K) filter parameters")
+    return _RecGuidanceNorm.apply(x, y, freqs, fc.contiguous(), A.contiguous(), int(nfft), known)
+
+
+def known_prefix_lengths(mask):
+    """k_b of a (B, T) mask whose every row is a known prefix (1 for n < k_b, 0 from k_b on; all ones: k_b = T,
+    all zeros: 0), as an int32[B] host tensor; None for any other mask."""
+    m = mask.detach().cpu()
+    k = (m == 1).to(torch.int64).cumprod(-1).sum(-1)
+    prefix = torch.arange(m.shape[-1]) < k.unsqueeze(-1)
+    return k.to(torch.int32) if torch.equal(m, prefix.to(m.dtype)) else None
 
 
 _PINNED_NOISE = {}
@@ -776,21 +791,30 @@ class BlindSamplerFused:
                 new[i:i + size] = left
         return new.unsqueeze(0).expand(B, -1)
 
-    def _generic_rec_grads(self, x_den, y, x_in, t_in, degradation, fused_params=None):
+    @classmethod
+    def prepare_smooth_mask_rows(cls, mask, size=10):
+        """``prepare_smooth_mask`` of every row of a (B, T) mask on its own (the per-row mode's windows differ)."""
+        return torch.cat([cls.prepare_smooth_mask(mask[b:b + 1], size) for b in range(mask.shape[0])])
+
+    def _generic_rec_grads(self, x_den, y, x_in, t_in, degradation, fused_params=None, known=None):
         """get_rec_grads (:75-135) for an arbitrary differentiable degradation (2-norm branch); a parametric
-        fc_A filter (``fused_params``) takes the fused design + filter + residual-norm kernels."""
+        fc_A filter (``fused_params``) takes the fused design + filter + residual-norm kernels, with ``known`` through
+        the known-prefix masked operator.  With ``filter_per_row`` every row gets its own normaliser."""
         ps = self.args.tester.posterior_sampling
         if ps.SNR_observations != "None" or ps.stft_distance.use or ps.norm not in (1, 2, "fro"):
             raise NotImplementedError("generic degradations support the plain 1-/2-norm guidance")
         if fused_params is not None and ps.norm == 2:
-            norm = rec_guidance_norms(x_den, y, self.freqs, fused_params, self.args.tester.blind_bwe.NFFT)
+            norm = rec_guidance_norms(x_den, y, self.freqs, fused_params, self.args.tester.blind_bwe.NFFT, known)
         else:
             norm = torch.linalg.norm(y - degradation(x_den), dim=1, ord=ps.norm)
         (g,) = torch.autograd.grad(outputs=norm.sum(), inputs=x_in)
-        normguide = torch.linalg.norm(g) / self.args.exp.audio_len ** 0.5
+        if self.filter_per_row:
+            normguide = torch.linalg.norm(g, dim=1, keepdim=True) / self.args.exp.audio_len ** 0.5
+        else:
+            normguide = torch.linalg.norm(g) / self.args.exp.audio_len ** 0.5
         return self.xi / (normguide + 1e-6) * g / t_in
 
-    def get_score(self, x, y, t_i, degradation, dc_step=None, fused_params=None):
+    def get_score(self, x, y, t_i, degradation, dc_step=None, fused_params=None, known=None):
         """testing/blind_bwe_sampler.py:160-209.  ``dc_step(x_hat)``: optional data-consistency step."""
         if y is None:
             with torch.no_grad():
@@ -798,7 +822,7 @@ class BlindSamplerFused:
         if self.xi > 0:
             x = x.detach().requires_grad_(True)
             x_den = self.get_denoised_estimate(x, t_i)
-            rec = self._generic_rec_grads(x_den, y, x, t_i, degradation, fused_params)
+            rec = self._generic_rec_grads(x_den, y, x, t_i, degradation, fused_params, known)
             x = x.detach()
             score = self.denoised2score(x_den.detach(), x, t_i) - rec
             if dc_step is not None:
@@ -810,7 +834,7 @@ class BlindSamplerFused:
                 x_hat = dc_step(x_hat)
             return self.denoised2score(x_hat, x, t_i)
 
-    def predict_conditional(self, y, degradation, rid=False, dc_step=None, fused_params=None):
+    def predict_conditional(self, y, degradation, rid=False, dc_step=None, fused_params=None, known=None):
         """testing/blind_bwe_sampler.py:387-497 (``predict`` with observations y)."""
         shape, device = y.shape, y.device
         self._keyed_begin(shape[0], device)
@@ -828,7 +852,7 @@ class BlindSamplerFused:
         for i in range(self.nb_steps):
             self._keyed_step(i)
             x_hat, t_hat = self.move_timestep(x, t[i], gamma[i], self.diff_params.Snoise)
-            score = self.get_score(x_hat, y, t_hat, degradation, dc_step, fused_params)
+            score = self.get_score(x_hat, y, t_hat, degradation, dc_step, fused_params, known)
             d = -t_hat * score
             if rid:
                 data_denoised[i] = self.score2denoised(score, x_hat, t_hat)
@@ -837,7 +861,7 @@ class BlindSamplerFused:
             if float(t_host[i + 1]) != 0 and self.order == 2:
                 t_prime = t[i + 1]
                 x_prime = x_hat + h * d
-                score = self.get_score(x_prime, y, t_prime, degradation, dc_step, fused_params)
+                score = self.get_score(x_prime, y, t_prime, degradation, dc_step, fused_params, known)
                 x = x_hat + h * ((1 / 2) * d + (1 / 2) * (-t_prime * score))
             else:
                 x = x_hat + h * d
@@ -851,10 +875,15 @@ class BlindSamplerFused:
         """testing/blind_bwe_sampler.py:259-303: bandwidth extension of a segment whose head (mask = 1)
         is already known from the previous segment: y = mask y_masked + (1 - mask) ylpf, degradation
         x -> mask x + (1 - mask) A(x); with ``complete_recording.inpaint_DC`` the known part is also
-        enforced by a data-consistency step through a hann-smoothed mask."""
+        enforced by a data-consistency step through a hann-smoothed mask.
+
+        With ``filter_per_row`` the rows are independent windows: ``filt`` is (2, K) (every row) or (B, 2, K), the
+        (B, T) mask may differ per row and each row gets its own smoothed mask and guidance normaliser."""
         assert mask is not None
         if test_filter_fit or compute_sweep:
             raise NotImplementedError("test_filter_fit / compute_sweep logging on the AR path")
+        if self.filter_per_row:
+            return self._predict_bwe_AR_rows(ylpf, y_masked, filt, filt_type, rid, mask)
         device = ylpf.device
         mask = mask.to(device)
         if filt_type == "fc_A":
@@ -875,6 +904,36 @@ class BlindSamplerFused:
             dc_step = lambda x_hat: y_smooth + x_hat - smooth * x_hat     # data_consistency_step_classic (:63-73)
         return self.predict_conditional(y, degradation, rid, dc_step)
 
+    def _predict_bwe_AR_rows(self, ylpf, y_masked, filt, filt_type, rid, mask):
+        """predict_bwe_AR with ``filter_per_row``.  When every mask row is a 0/1 known prefix (what the
+        autoregressive driver builds) the 2-norm guidance runs through the masked fused kernel pair; any other mask
+        keeps the eager composition on the per-row filter."""
+        if filt_type != "fc_A":
+            raise NotImplementedError(f"filter_per_row with filt_type {filt_type!r}: only the parametric fc_A filter "
+                                      "has per-row kernels (the FIR kernel shares its taps over the rows)")
+        device = ylpf.device
+        B, T = ylpf.shape
+        params = filt.to(device)
+        if params.dim() == 2:
+            params = params.unsqueeze(0).expand(B, -1, -1)
+        if params.dim() != 3 or params.shape[0] != B or params.shape[1] != 2:
+            raise ValueError(f"per-row filter parameters must be (2, K) or ({B}, 2, K), got {tuple(filt.shape)}")
+        self.freqs = torch.fft.rfftfreq(self.args.tester.blind_bwe.NFFT, d=1 / self.args.exp.sample_rate).to(device)
+        self.params = params = params.contiguous()
+        mask = mask.to(device).expand(B, T)
+        y = mask * y_masked + (1 - mask) * ylpf
+        degradation = lambda x: mask * x + (1 - mask) * self.apply_filter_fcA(x, params)
+        known = known_prefix_lengths(mask)
+        if known is not None:
+            known = known.to(device)
+        dc_step = None
+        if self.args.tester.complete_recording.inpaint_DC:
+            smooth = self.prepare_smooth_mask_rows(mask, 50)
+            y_smooth = smooth * y_masked
+            dc_step = lambda x_hat: y_smooth + x_hat - smooth * x_hat
+        return self.predict_conditional(y, degradation, rid, dc_step, fused_params=None if known is None else params,
+                                        known=known)
+
     def predict_bwe(self, ylpf, filt, filt_type, rid=False, test_filter_fit=False, compute_sweep=False):
         """testing/blind_bwe_sampler.py:306-364: non-blind bandwidth extension with a KNOWN observation model,
         routed like the reference through ``predict_conditional`` / ``get_score`` (:160-209, 387-497): with
@@ -887,6 +946,9 @@ class BlindSamplerFused:
                                       "CUDA operators; the IIR / resampling models are outside this path")
         if test_filter_fit or compute_sweep:
             raise NotImplementedError("test_filter_fit / compute_sweep logging on the non-blind path")
+        if self.filter_per_row and filt_type != "fc_A":
+            raise NotImplementedError(f"filter_per_row with filt_type {filt_type!r}: only the parametric fc_A filter "
+                                      "has per-row kernels (the FIR kernel shares its taps over the rows)")
         args = self.args
         device = ylpf.device
         fused = None

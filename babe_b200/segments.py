@@ -46,6 +46,17 @@ def _row_seeds(sampler, seeds):
         sampler.row_seeds = was
 
 
+@contextlib.contextmanager
+def _filter_per_row(sampler, on):
+    """Set the sampler's ``filter_per_row`` for one call and restore the previous value afterwards."""
+    was = sampler.filter_per_row
+    sampler.filter_per_row = on
+    try:
+        yield
+    finally:
+        sampler.filter_per_row = was
+
+
 def segment_spans(L, seg_len, ola=256, discard_end=200, discard_start=0):
     """Start indices exactly as the while-loop at testing/blind_bwe_tester.py:469-521
     produces them; the last span is the incomplete tail (:526-533)."""
@@ -150,6 +161,22 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
     return final, [(spans[s], all_filt[s]) for s in range(len(spans))]
 
 
+def ar_windows(L, seg_len, overlap, discard_end=200, discard_start=0):
+    """Windows ``(start, length)`` that the autoregressive restoration of a recording of L samples visits, in order:
+    the first window (0, seg_len) (``predict_bwe``), the autoregressive windows advancing by
+    ``seg_len - overlap - discard_end`` samples, and the last window (start, n) with n = L - start <= seg_len, which
+    is zero padded to seg_len (testing/blind_bwe_tester.py:799-859).  The reference stops at
+    ix >= L - seg_len - discard_end (:820) and then fails on a remainder longer than one window (:852-859); full
+    windows are placed here as long as more than one window is left."""
+    step = seg_len - overlap - discard_end
+    windows, ix = [(0, seg_len)], step
+    while ix < L - seg_len - discard_end - discard_start or L - ix > seg_len:
+        windows.append((ix, seg_len))
+        ix += step
+    windows.append((ix, L - ix))
+    return windows
+
+
 def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25, n_segments_blindstep=2,
                          ix_start_s=0, std=0.1, typefilter="fc_A", discard_end=200, discard_start=0,
                          rng=None, estimated_filter=None, seed=None):
@@ -195,7 +222,7 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
         final[0, ix_first:ix_first + segL] = pred[0]
     overlap = int(overlap_s * sample_rate)
     keep = segL - discard_end
-    ix = 0
+    windows = ar_windows(L, segL, overlap, discard_end, discard_start)
     window = [0]
 
     def keyed():                                             # the seeds of the next window
@@ -203,27 +230,23 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
         window[0] += 1
         return _row_seeds(sampler, None if seed is None else [row_seed(seed, w)])
 
-    seg = degraded[..., ix:ix + segL]
+    seg = degraded[..., :segL]
     with keyed():
         pred = sampler.predict_bwe(seg, estimated_filter, typefilter, rid=False)
     previous = pred[..., :keep]
-    final[..., ix:ix + keep] = previous
-    ix += segL - overlap - discard_end
+    final[..., :keep] = previous
     y_masked = torch.zeros_like(pred)
     mask = torch.ones_like(seg)
     mask[..., overlap:] = 0
-    # the reference stops at ix >= L - segL - discard_end (:820) and then fails on a remainder longer than one
-    # window (:852-859); full windows are processed here as long as more than one window is left
-    while ix < L - segL - discard_end - discard_start or L - ix > segL:
+    for ix, _ in windows[1:-1]:
         y_masked[..., :overlap] = previous[..., segL - overlap - discard_end:]
         seg = degraded[..., ix:ix + segL]
         with keyed():
             pred = sampler.predict_bwe_AR(seg, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
         previous = pred[..., :keep]
         final[..., ix:ix + keep] = previous
-        ix += segL - overlap - discard_end
+    ix, n = windows[-1]
     seg = degraded[..., ix:]
-    n = seg.shape[-1]
     y_masked[..., :overlap] = pred[..., -overlap:]          # sic (:842): the tail of the FULL last prediction
     if n < segL:
         seg_zp = torch.cat((seg, seg.new_zeros((1, segL - n))), -1)
@@ -235,3 +258,120 @@ def restore_recording_ar(sampler, degraded, seg_len, sample_rate, overlap_s=0.25
         pred = sampler.predict_bwe_AR(seg_zp, y_masked, estimated_filter, typefilter, rid=False, mask=mask)
     final[..., ix:ix + n] = pred[..., :n]
     return final * scale.unsqueeze(-1) / std, estimated_filter
+
+
+def restore_recordings_ar(sampler, recordings, seg_len, sample_rate, overlap_s=0.25, n_segments_blindstep=2,
+                          ix_start_s=0, std=0.1, typefilter="fc_A", discard_end=200, discard_start=0, seeds=None,
+                          estimated_filters=None, rng=None):
+    """``restore_recording_ar`` on N recordings at once: window w of every recording that still has one goes into ONE
+    sampler call with ``filter_per_row`` (round 0 ``predict_bwe``, later rounds ``predict_bwe_AR``), so the denoiser
+    runs at batch N instead of N times at batch 1.  The batch shrinks as the shorter recordings finish.  Row r of a
+    call is independent of the other rows, so recording r is restored as ``restore_recording_ar`` restores it alone:
+    the same normalisation, known heads, last padded window and final scale.
+
+    ``recordings``: (1, L_r) tensors on one device, each at least ``seg_len`` long.  ``seeds`` (one int per
+    recording) switches to keyed noise with the seeds ``restore_recording_ar(seed=seeds[r])`` uses: window w draws
+    with ``row_seed(seeds[r], w)``, blind-step row j with ``row_seed(seeds[r], 2**32 + j)``; the restorations then
+    agree to rounding.  ``estimated_filters`` (N filters (2, K)) skips the blind step.  Otherwise
+    ``n_segments_blindstep == 1`` estimates the N filters in ONE per-row ``predict_blind_bwe`` call on the first
+    windows, and larger counts run one blind call per recording, in recording order, drawing window positions from
+    ``rng`` as N sequential ``restore_recording_ar`` calls do.  Single process: sharding recordings over ranks is
+    the caller's.  Returns [(restored (1, L_r), filter (2, K)), ...]."""
+    import numpy as np
+    if getattr(sampler, "joint", False):
+        raise ValueError("restore_recordings_ar restores every recording with its own filter; joint=True shares one")
+    if typefilter != "fc_A":
+        raise NotImplementedError(f"typefilter {typefilter!r}: only the parametric fc_A filter has per-row kernels")
+    segL = int(seg_len)
+    recs = [r.reshape(1, -1) for r in recordings]
+    N = len(recs)
+    if N == 0:
+        return []
+    device = recs[0].device
+    for i, r in enumerate(recs):
+        if r.device != device:
+            raise ValueError(f"recording {i} is on {r.device}, recording 0 on {device}: one device for all")
+        if r.shape[-1] < segL:
+            raise ValueError(f"recording {i} has {r.shape[-1]} samples, fewer than seg_len = {segL}")
+    if seeds is not None and len(seeds) != N:
+        raise ValueError(f"{len(seeds)} seeds for {N} recordings")
+    if estimated_filters is not None and len(estimated_filters) != N:
+        raise ValueError(f"{len(estimated_filters)} filters for {N} recordings")
+    scales = [r.std(-1) for r in recs]
+    deg = [std * r / sc.unsqueeze(-1) for r, sc in zip(recs, scales)]
+    finals = [torch.zeros_like(d) for d in deg]
+    ix_first = int(sample_rate * ix_start_s)
+
+    def keyed(rows, k):                                      # seeds of unit k of the given recordings
+        return _row_seeds(sampler, None if seeds is None else [row_seed(seeds[r], k) for r in rows])
+
+    if estimated_filters is None:
+        if n_segments_blindstep == 1:
+            y = torch.cat([d[..., ix_first:ix_first + segL] for d in deg])
+            with _filter_per_row(sampler, True), keyed(range(N), 1 << 32):
+                pred, filts = sampler.predict_blind_bwe(y, rid=False)
+            for r in range(N):
+                finals[r][0, ix_first:ix_first + segL] = pred[r]
+        else:
+            rng = rng if rng is not None else np.random
+            fl = []
+            for r, d in enumerate(deg):
+                L = d.shape[-1]
+                y = d[..., ix_first:ix_first + segL].repeat(n_segments_blindstep, 1)
+                for j in range(n_segments_blindstep):
+                    ix = int(rng.randint(0, L - segL))
+                    y[j] = d[0, ix:ix + segL]
+                blind = None if seeds is None else [row_seed(seeds[r], (1 << 32) + j) for j in range(y.shape[0])]
+                with _filter_per_row(sampler, False), _row_seeds(sampler, blind):
+                    pred, f = sampler.predict_blind_bwe(y, rid=False)
+                finals[r][0, ix_first:ix_first + segL] = pred[0]
+                fl.append(f)
+            filts = torch.stack(fl)
+    else:
+        filts = torch.stack([f.to(device) for f in estimated_filters])
+    overlap = int(overlap_s * sample_rate)
+    keep = segL - discard_end
+    windows = [ar_windows(d.shape[-1], segL, overlap, discard_end, discard_start) for d in deg]
+    preds = [None] * N                                       # last prediction of each recording
+    previous = [None] * N
+    y_masked = [None] * N
+    masks = [None] * N
+    with _filter_per_row(sampler, True):
+        for w in range(max(len(ws) for ws in windows)):
+            rows = [r for r in range(N) if w < len(windows[r])]
+            segs = []
+            for r in rows:
+                ix, n = windows[r][w]
+                if w == 0:
+                    segs.append(deg[r][..., :segL])
+                elif w < len(windows[r]) - 1:
+                    y_masked[r][..., :overlap] = previous[r][..., segL - overlap - discard_end:]
+                    segs.append(deg[r][..., ix:ix + segL])
+                else:
+                    y_masked[r][..., :overlap] = preds[r][..., -overlap:]     # sic (:842), as restore_recording_ar
+                    seg = deg[r][..., ix:]
+                    if n < segL:
+                        seg = torch.cat((seg, seg.new_zeros((1, segL - n))), -1)
+                        y_masked[r][..., n:segL] = 0
+                        masks[r][..., n:segL] = 0
+                    segs.append(seg[..., :segL])
+            with keyed(rows, w):
+                if w == 0:
+                    out = sampler.predict_bwe(torch.cat(segs), filts, typefilter, rid=False)
+                else:
+                    out = sampler.predict_bwe_AR(torch.cat(segs), torch.cat([y_masked[r] for r in rows]),
+                                                 filts[rows], typefilter, rid=False,
+                                                 mask=torch.cat([masks[r] for r in rows]))
+            for i, r in enumerate(rows):
+                ix, n = windows[r][w]
+                preds[r] = pred = out[i:i + 1]
+                if w == 0:
+                    y_masked[r] = torch.zeros_like(pred)
+                    masks[r] = torch.ones_like(pred)
+                    masks[r][..., overlap:] = 0
+                if w < len(windows[r]) - 1:
+                    previous[r] = pred[..., :keep]
+                    finals[r][..., ix:ix + keep] = previous[r]
+                else:
+                    finals[r][..., ix:ix + n] = pred[..., :n]
+    return [(f * sc.unsqueeze(-1) / std, filts[r]) for r, (f, sc) in enumerate(zip(finals, scales))]

@@ -128,6 +128,20 @@ int babe_apply_filter_rows(const float* x, float* y, int B, int T, int nfft,
                            int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
                            void* workspace, size_t workspace_bytes, int* status, void* stream);
 
+/* babe_apply_filter_rows through the known-prefix masked operator D_b x = m_b x + (1 - m_b) A_b x with
+ * m_b[n] = 1 for n < known[b], 0 after (int32[B]; known[b] <= 0: no mask, >= T: every sample known):
+ *   forward  y[b,n] = (n < known[b] ? x[b,n] : (A_b x_b)[n]) - sub[b,n]
+ *   adjoint  y[b,n] = row_scale[b] * (A_b^T (x_b 1[n >= known[b]])[n] + (n < known[b] ? x[b,n] : 0))
+ * (row_sumsq and the other epilogues as above).  known == NULL is babe_apply_filter_rows.  NFFT 4096 rows that can
+ * be bulk-copied run the masked variant of the fused kernel; the other cases filter row by row and fix the prefix
+ * in a second pass (the adjoint allocates a B x T copy of x, stream ordered). */
+int babe_apply_filter_rows_known(const float* x, float* y, int B, int T, int nfft,
+                                 const float* window, const float* twiddle,
+                                 const float* freqs, const float* fc, const float* A, int K,
+                                 int adjoint, const float* sub, const float* row_scale, double* row_sumsq,
+                                 void* workspace, size_t workspace_bytes, int* status, const int* known,
+                                 void* stream);
+
 /* ---- a1: STFT, a2: filter + iSTFT (unfused signatures) ------------------ */
 /* apply_stft (utils/blind_bwe_utils.py:15-26): x[B,T] -> X[B,F,frames,2].
  * frames = 0 means the reference's 1 + T/(nfft/2) (x is treated as right
