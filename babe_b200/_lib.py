@@ -83,16 +83,20 @@ SIGNATURES = {
     "babe_fir_filter": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int,
                                 c_void_p]),
     "babe_gn_slices": (c_int, [c_int, c_int, c_int, c_longlong]),
-    "babe_gn_stats": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_longlong, c_int, c_void_p]),
-    "babe_gn_film_gelu": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int,
-                                  c_int, c_longlong, c_float, c_void_p]),
+    "babe_net_chunks": (c_int, [c_longlong]),
+    "babe_gn_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_longlong, c_int,
+                              c_void_p]),
+    "babe_gn_film_gelu": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                  c_longlong, c_float, c_void_p]),
     "babe_gate_residual": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_longlong,
                                    c_float, c_void_p]),
-    "babe_gn_bwd_slices": (c_int, [c_int, c_int, c_longlong]),
-    "babe_gn_film_gelu_bwd_reduce": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
-                                             c_void_p, c_int, c_int, c_int, c_longlong, c_float, c_void_p]),
-    "babe_gn_film_gelu_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
-                                      c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_longlong, c_float,
+    "babe_gate_residual_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_int, c_int, c_int, c_longlong, c_float, c_void_p]),
+    "babe_gn_film_gelu_bwd_reduce": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                             c_void_p, c_void_p, c_int, c_int, c_int, c_longlong, c_float,
+                                             c_void_p]),
+    "babe_gn_film_gelu_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_longlong, c_float,
                                       c_float, c_void_p]),
     "babe_resample2": (c_int, [c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p, c_int, c_void_p]),
     "babe_stft_stats_workspace": (c_size_t, [c_int, c_int, c_int]),

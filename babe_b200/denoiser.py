@@ -140,15 +140,19 @@ class ResnetBlock(nn.Module):
 
     def forward(self, input_x, sigma):
         x = self.proj_in(input_x)
-        for norm, affine, gate, conv in zip(self.norm, self.affine, self.gate, self.H):
-            if FUSED and net_ops.usable(x, norm.gamma, conv.weight, affine.weight, gate.weight, sigma):
-                # csrc/net_ops.cu: 3 launches around the convolution instead of ~8 PyTorch kernels
-                x = net_ops.res_layer(x, norm.gamma, affine(sigma), gate(sigma), conv.weight,
-                                      conv.dilation, norm.num_groups, norm.eps)
-                continue
-            x0 = x
-            x = norm(x) * (affine(sigma)[:, :, None, None] + 1)
-            x = (x0 + conv(F.gelu(x)) * gate(sigma)[:, :, None, None]) / (2 ** 0.5)
+        layers = list(zip(self.norm, self.affine, self.gate, self.H))
+        norm0 = self.norm[0]
+        if FUSED and all(n.num_groups == norm0.num_groups and n.eps == norm0.eps for n in self.norm) and \
+                all(net_ops.usable(x, norm.gamma, conv.weight, affine.weight, gate.weight, sigma)
+                    for norm, affine, gate, conv in layers):
+            # csrc/net_ops.cu: at most 3 launches around each convolution instead of ~8 PyTorch kernels
+            x = net_ops.res_chain(x, [(norm.gamma, affine(sigma), gate(sigma), conv.weight, conv.dilation)
+                                      for norm, affine, gate, conv in layers], norm0.num_groups, norm0.eps)
+        else:
+            for norm, affine, gate, conv in layers:
+                x0 = x
+                x = norm(x) * (affine(sigma)[:, :, None, None] + 1)
+                x = (x0 + conv(F.gelu(x)) * gate(sigma)[:, :, None, None]) / (2 ** 0.5)
         if self.proj_place == 'after':
             x = self.proj_out(x)
         return _add_scale(x, self.res_conv(input_x))

@@ -32,49 +32,86 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+# Arrival counters of the kernels whose last CTA finishes a group's statistics: one per (n, group), zero
+# between calls (every kernel resets the ones it used).  N * G <= N * C <= 65535 (``usable``).  Calls
+# sharing counters must not overlap, so there is one buffer per (device, stream): kernels on one stream
+# run in order, and two streams never count on the same buffer.
+_COUNTERS = {}
+
+
+def _counters(device):
+    key = (device.index, torch.cuda.current_stream(device).cuda_stream)
+    c = _COUNTERS.get(key)
+    if c is None:
+        c = _COUNTERS[key] = torch.zeros(65536, dtype=torch.int32, device=device)
+    return c
+
+
 def gn_stats(x, groups):
+    """Finished statistics {mean, std} of every (sample, group) of x, and the number of partial slices
+    they were summed from."""
     N, C, Fd, T = x.shape
     P = Fd * T
     S = lib().babe_gn_slices(N, C, groups, P)
     part = torch.empty(N * groups * S * 2, dtype=torch.float64, device=x.device)
+    stats = torch.empty(N * groups, 2, dtype=torch.float32, device=x.device)
     with profiling.op("gn_stats", 1, 4 * x.numel()):
-        check(lib().babe_gn_stats(_p(x), _p(part), N, C, groups, P, S, _stream()), "gn_stats")
-    return part, S
+        check(lib().babe_gn_stats(_p(x), _p(part), _p(stats), _p(_counters(x.device)), N, C, groups, P, S,
+                                  _stream()), "gn_stats")
+    return stats, S
 
 
-def gn_film_gelu(x, part, S, gamma, aff, groups, eps):
+def gn_film_gelu(x, stats, S, gamma, aff, groups, eps):
+    """``(stats, S)``: what gn_stats (or gate_residual with ``groups``) returned.  The record is finished and
+    no kernel reads S; it stays in the tuple so that the four glue wrappers keep their positional
+    signatures (tests/test_net_ops_plumbing_cpu.py substitutes them by position)."""
     N, C, Fd, T = x.shape
     h = torch.empty_like(x)
     with profiling.op("gn_film_gelu", 1, 8 * x.numel()):
-        check(lib().babe_gn_film_gelu(_p(x), _p(h), _p(part), S, _p(gamma), _p(aff), N, C, groups,
+        check(lib().babe_gn_film_gelu(_p(x), _p(h), _p(stats), _p(gamma), _p(aff), N, C, groups,
                                       Fd * T, eps, _stream()), "gn_film_gelu")
     return h
 
 
-def gate_residual(x0, v, gate, scale=RSQRT2):
-    """(x0 + v * gate[n,c]) * scale; ``x0`` and ``gate`` may be None."""
+def gate_residual(x0, v, gate, scale=RSQRT2, *, groups=None):
+    """(x0 + v * gate[n,c]) * scale; ``x0`` and ``gate`` may be None.  With ``groups``: also the group
+    statistics of the result, returned as ``out, (stats, S)`` like gn_stats(out, groups)."""
     N, C, Fd, T = v.shape
+    P = Fd * T
     out = torch.empty_like(v)
     with profiling.op("gate_residual", 1, (8 if x0 is None else 12) * v.numel()):
-        check(lib().babe_gate_residual(_p(x0), _p(v), _p(gate), _p(out), N, C, Fd * T, scale, _stream()),
+        if groups is None:
+            check(lib().babe_gate_residual(_p(x0), _p(v), _p(gate), _p(out), N, C, P, scale, _stream()),
+                  "gate_residual")
+            return out
+        S = C // groups * lib().babe_net_chunks(P)
+        part = torch.empty(N * groups * S * 2, dtype=torch.float64, device=v.device)
+        stats = torch.empty(N * groups, 2, dtype=torch.float32, device=v.device)
+        check(lib().babe_gate_residual_stats(_p(x0), _p(v), _p(gate), _p(out), _p(part), _p(stats),
+                                             _p(_counters(v.device)), N, C, groups, P, scale, _stream()),
               "gate_residual")
-    return out
+    return out, (stats, S)
 
 
-def gn_film_gelu_bwd(gh, x, gy, part, S, gamma, aff, groups, eps, res_scale=RSQRT2):
+def gn_film_gelu_bwd(gh, x, gy, stats, S, gamma, aff, groups, eps, res_scale=RSQRT2, *, gate_prev=None):
+    """g_x of the layer (``gy`` may be None).  With ``gate_prev``: returns ``gx, gv`` where
+    gv = gate_residual(None, gx, gate_prev, res_scale) comes from the same kernel."""
     N, C, Fd, T = x.shape
     P = Fd * T
-    S2 = lib().babe_gn_bwd_slices(N, C, P)
-    scratch = torch.empty(N * C * S2, dtype=torch.float64, device=x.device)
+    scratch = torch.empty(N * C * lib().babe_net_chunks(P), dtype=torch.float64, device=x.device)
+    coef = torch.empty(N * groups, dtype=torch.float32, device=x.device)
     gx = torch.empty_like(x)
+    gv = torch.empty_like(x) if gate_prev is not None else None
     with profiling.op("gn_bwd_reduce", 1, 8 * x.numel()):
-        check(lib().babe_gn_film_gelu_bwd_reduce(_p(gh), _p(x), _p(part), S, _p(scratch), S2, _p(gamma),
-                                                 _p(aff), N, C, groups, P, eps, _stream()), "gn_bwd_reduce")
-    with profiling.op("gn_film_gelu_bwd", 1, (16 if gy is not None else 12) * x.numel()):
-        check(lib().babe_gn_film_gelu_bwd(_p(gh), _p(x), _p(gy), _p(gx), _p(part), S, _p(scratch), S2,
-                                          _p(gamma), _p(aff), N, C, groups, P, eps, res_scale, _stream()),
+        check(lib().babe_gn_film_gelu_bwd_reduce(_p(gh), _p(x), _p(stats), _p(scratch), _p(coef),
+                                                 _p(_counters(x.device)), _p(gamma), _p(aff), N, C, groups, P,
+                                                 eps, _stream()), "gn_bwd_reduce")
+    nbytes = (16 if gy is not None else 12) + (4 if gv is not None else 0)
+    with profiling.op("gn_film_gelu_bwd", 1, nbytes * x.numel()):
+        check(lib().babe_gn_film_gelu_bwd(_p(gh), _p(x), _p(gy), _p(gx), _p(stats), _p(coef), _p(gamma), _p(aff),
+                                          _p(gate_prev), _p(gv), N, C, groups, P, eps, res_scale, _stream()),
               "gn_film_gelu_bwd")
-    return gx
+    return gx if gv is None else (gx, gv)
 
 
 def _same_padding(weight, dilation):
@@ -153,35 +190,59 @@ def conv_same(inp, weight, pad, dilation, transposed=False, wobj=None):
     return direct() if choice == 0 else other()
 
 
-class _ResLayer(torch.autograd.Function):
+class _ResChain(torch.autograd.Function):
+    """The dilated layers of one ResnetBlock in sequence.  Each layer's output carries the statistics the
+    next layer normalises with (gate_residual with ``groups``), and in the backward pass each layer's g_x
+    kernel also writes g_v of the layer before it (gn_film_gelu_bwd with ``gate_prev``), so only the first
+    layer reads its input for statistics and only the last one has a separate g_v pass.  Saved: every
+    layer's input and statistics record."""
+
     @staticmethod
-    def forward(ctx, x, gamma, aff, gate, weight, dilation, groups, eps):
+    def forward(ctx, x, layers, groups, eps):
         x = x.contiguous()
         N, C = x.shape[:2]
-        gamma = gamma.detach().reshape(-1).contiguous().float()
-        aff, gate = _rows(aff, N, C), _rows(gate, N, C)
-        wobj, weight = weight, weight.detach()
-        pad = _same_padding(weight, dilation)
-        part, S = gn_stats(x, groups)
-        h = gn_film_gelu(x, part, S, gamma, aff, groups, eps)
-        v = conv_same(h, weight, pad, dilation, wobj=wobj)
-        del h
-        y = gate_residual(x, v, gate)
-        ctx.save_for_backward(x, part, gamma, aff, gate, weight)
-        ctx.cfg = (S, dilation, groups, eps, pad)
-        ctx.wobj = wobj                      # the caller's weight object: key of the flipped-copy cache
-        return y
+        cfg = []
+        stats = gn_stats(x, groups)
+        xs, recs = [], []
+        for i, (gamma, aff, gate, weight, dilation) in enumerate(layers):
+            gamma = gamma.detach().reshape(-1).contiguous().float()
+            aff, gate = _rows(aff, N, C), _rows(gate, N, C)
+            wobj, weight = weight, weight.detach()
+            pad = _same_padding(weight, dilation)
+            h = gn_film_gelu(x, *stats, gamma, aff, groups, eps)
+            v = conv_same(h, weight, pad, dilation, wobj=wobj)
+            del h
+            xs.append(x)
+            recs.append(stats)
+            if i + 1 < len(layers):
+                x, stats = gate_residual(x, v, gate, groups=groups)
+            else:
+                x = gate_residual(x, v, gate)
+            # the caller's weight object: key of the flipped-copy cache
+            cfg.append((gamma, aff, gate, weight, wobj, pad, dilation))
+        ctx.save_for_backward(*xs, *(st for st, _ in recs))
+        ctx.slices = [S for _, S in recs]
+        ctx.cfg = (cfg, groups, eps)
+        return x
 
     @staticmethod
     def backward(ctx, gy):
-        x, part, gamma, aff, gate, weight = ctx.saved_tensors
-        S, dilation, groups, eps, pad = ctx.cfg
+        cfg, groups, eps = ctx.cfg
+        n = len(cfg)
+        saved = ctx.saved_tensors
         gy = gy.contiguous()
-        gv = gate_residual(None, gy, gate)
-        gh = conv_same(gv, weight, pad, dilation, transposed=True, wobj=ctx.wobj)
-        del gv
-        gx = gn_film_gelu_bwd(gh.contiguous(), x, gy, part, S, gamma, aff, groups, eps)
-        return gx, None, None, None, None, None, None, None
+        gv = gate_residual(None, gy, cfg[-1][2])
+        for i in range(n - 1, -1, -1):
+            gamma, aff, gate, weight, wobj, pad, dilation = cfg[i]
+            gh = conv_same(gv, weight, pad, dilation, transposed=True, wobj=wobj).contiguous()
+            del gv
+            rec = (saved[n + i], ctx.slices[i])
+            if i > 0:
+                gy, gv = gn_film_gelu_bwd(gh, saved[i], gy, *rec, gamma, aff, groups, eps, gate_prev=cfg[i - 1][2])
+            else:
+                gy = gn_film_gelu_bwd(gh, saved[i], gy, *rec, gamma, aff, groups, eps)
+            del gh
+        return gy, None, None, None
 
 
 class _ConvSame(torch.autograd.Function):
@@ -235,7 +296,12 @@ def usable(x, *params):
 
 def res_layer(x, gamma, aff, gate, weight, dilation, groups, eps):
     """(x + conv(gelu(groupnorm(x) * gamma * (aff + 1))) * gate) / sqrt(2), conv with "same" padding."""
-    return _ResLayer.apply(x, gamma, aff, gate, weight, _pair(dilation), groups, eps)
+    return _ResChain.apply(x, ((gamma, aff, gate, weight, _pair(dilation)),), groups, eps)
+
+
+def res_chain(x, layers, groups, eps):
+    """res_layer applied in turn for every (gamma, aff, gate, weight, dilation) of ``layers``."""
+    return _ResChain.apply(x, tuple((g, a, t, w, _pair(d)) for g, a, t, w, d in layers), groups, eps)
 
 
 def add_scale(a, b):

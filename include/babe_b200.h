@@ -323,28 +323,41 @@ int babe_cqt_synthesis(const babe_cqt_plan* plan, const float* const* in_octaves
  *   h = gelu(BiasFreeGroupNorm_G(x) * gamma[c] * (aff[n,c] + 1))     (norm: networks/cqtdiff+.py:137-163,
  *                                                                     x / (unbiased std of (n, group) + eps))
  *   y = (x0 + v * gate[n,c]) * scale                                 (v = conv(h), scale = 1/sqrt(2))
- * babe_gn_stats writes per-slice (sum, sum of squares) doubles part[N*G][slices][2]
- * (slices = babe_gn_slices(...)); the consumers finish the statistics themselves. */
+ * Group statistics travel as a finished record stats[N*G] = {mean, unbiased std} (float pairs), written by
+ * the last CTA of the producing kernel to finish its group: the producer's CTAs store fp64 partial sums
+ * in fixed slots of `part` and count their arrival in counters[n*G + g]; the last one sums the slots in a
+ * fixed order and resets the counter.  counters: >= N*G unsigned ints, zero
+ * before the call and left zero, shared only by stream-ordered calls.
+ * babe_gn_stats: part[N*G][slices][2] (slices = babe_gn_slices(...)). */
 int babe_gn_slices(int N, int C, int G, long long P);
-int babe_gn_stats(const float* x, double* part, int N, int C, int G, long long P, int slices,
-                  void* stream);
-int babe_gn_film_gelu(const float* x, float* h, const double* part, int slices, const float* gamma,
-                      const float* aff, int N, int C, int G, long long P, float eps, void* stream);
+int babe_gn_stats(const float* x, double* part, float* stats, unsigned* counters, int N, int C, int G,
+                  long long P, int slices, void* stream);
+int babe_gn_film_gelu(const float* x, float* h, const float* stats, const float* gamma, const float* aff,
+                      int N, int C, int G, long long P, float eps, void* stream);
 /* gate == NULL: gate = 1;  x0 == NULL: out = v * gate * scale (the backward wrt v). */
 int babe_gate_residual(const float* x0, const float* v, const float* gate, float* out, int N, int C,
                        long long P, float scale, void* stream);
+/* babe_gate_residual that also writes the group statistics of out (what babe_gn_stats would compute from
+ * it, summed in a different partition); part[N*G][(C/G) * babe_net_chunks(P)][2]. */
+int babe_gate_residual_stats(const float* x0, const float* v, const float* gate, float* out, double* part,
+                             float* stats, unsigned* counters, int N, int C, int G, long long P, float scale,
+                             void* stream);
+/* CTAs per plane of the streaming glue kernels. */
+int babe_net_chunks(long long P);
 /* Backward of (babe_gn_stats + babe_gn_film_gelu) wrt x, with the residual branch folded in:
  *   gx = gy * res_scale + d/dx <gh, h(x)>      (gy may be NULL)
- * in two launches: _reduce fills gr_part[N*C][slices2] (slices2 = babe_gn_bwd_slices(...)) with the
- * partial sums of the statistic's gradient, then babe_gn_film_gelu_bwd writes gx. */
-int babe_gn_bwd_slices(int N, int C, long long P);
-int babe_gn_film_gelu_bwd_reduce(const float* gh, const float* x, const double* part, int slices,
-                                 double* gr_part, int slices2, const float* gamma, const float* aff,
+ * in two launches: _reduce sums the statistic's gradient G_r per group (partials in
+ * gr_part[N*C][babe_net_chunks(P)]) and writes coef[N*G] = G_r r^2 / ((cnt - 1) std), r = 1 / (std + eps);
+ * then babe_gn_film_gelu_bwd writes gx.  gate_prev / gv_prev (both or neither): also
+ * gv_prev = gx * gate_prev[n,c] * res_scale, the gradient wrt the preceding layer's convolution output,
+ * bit-identical to babe_gate_residual(NULL, gx, gate_prev, ..., res_scale). */
+int babe_gn_film_gelu_bwd_reduce(const float* gh, const float* x, const float* stats, double* gr_part,
+                                 float* coef, unsigned* counters, const float* gamma, const float* aff,
                                  int N, int C, int G, long long P, float eps, void* stream);
-int babe_gn_film_gelu_bwd(const float* gh, const float* x, const float* gy, float* gx,
-                          const double* part, int slices, const double* gr_part, int slices2,
-                          const float* gamma, const float* aff, int N, int C, int G, long long P,
-                          float eps, float res_scale, void* stream);
+int babe_gn_film_gelu_bwd(const float* gh, const float* x, const float* gy, float* gx, const float* stats,
+                          const float* coef, const float* gamma, const float* aff, const float* gate_prev,
+                          float* gv_prev, int N, int C, int G, long long P, float eps, float res_scale,
+                          void* stream);
 
 /* x2 anti-aliased time resampling of UpDownResample (networks/cqtdiff+.py:522-580, mode "T",
  * reflect padding fused) on `rows` independent rows; T = length of the x-side row (even):
