@@ -105,6 +105,9 @@ SIGNATURES = {
     "babe_stft_stats_rows_workspace": (c_size_t, [c_int, c_int, c_int]),
     "babe_stft_stats_rows": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_size_t, c_void_p]),
+    "babe_stft_stats_groups_workspace": (c_size_t, [c_int, c_int, c_int]),
+    "babe_stft_stats_groups": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                       c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "babe_spec_mag_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                     c_void_p, c_void_p]),
     "babe_spec_mag_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,

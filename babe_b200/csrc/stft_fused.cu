@@ -351,9 +351,10 @@ constexpr size_t stats_smem_bytes() {
          sizeof(float) * 2 * Core4k::N + 32;
 }
 
-// ROWS: statistics per row.  A CTA's run of frames may cross row boundaries: its register sums are written out and
-// cleared whenever the row changes, one partial per (CTA, row) segment at slot CTA + row (as k_segment_sumsq indexes
-// the residual partials), and k_reduce_stats_rows adds a row's slots in a fixed order.
+// ROWS: statistics per group of consecutive rows (a.offsets; NULL: one group per row).  A CTA's run of frames may cross
+// group boundaries: its register sums are written out and cleared whenever the next frame starts a new group, one
+// partial per (CTA, group) segment at slot CTA + group (as k_segment_sumsq indexes the residual partials), and
+// k_reduce_stats_rows adds a group's slots in a fixed order.  Slots stay below grid + G - 1 <= grid + B.
 template <bool ROWS>
 __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) {
   using C = Core4k;
@@ -415,6 +416,21 @@ __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) 
       out[2 * C::F + 2048] = 0.25f * nc;
     }
   };
+  // ROWS: group of the current frame and the first row past it
+  int grp = 0, gend = 0;
+  if (ROWS && g0 < g1) {
+    const int row0 = (int)(g0 / a.frames);
+    if (a.offsets == nullptr) {
+      grp = row0;
+    } else {
+      int hi = a.G;                                   // offsets[grp] <= row0 < offsets[hi]
+      while (hi - grp > 1) {
+        const int mid = (grp + hi) >> 1;
+        if (a.offsets[mid] <= row0) grp = mid; else hi = mid;
+      }
+    }
+    gend = a.offsets == nullptr ? grp + 1 : a.offsets[grp + 1];
+  }
   if (t == 0 && g0 < g1) issue(g0);
   for (long long g = g0; g < g1; ++g) {
     float2 z[16];
@@ -466,34 +482,41 @@ __global__ void __launch_bounds__(256, 2) k_stats_fused(const FusedStatsArgs a) 
       const float sx = 4.f * z[8].x * z[8].x, sy = 4.f * z[8].y * z[8].y;
       na += sx; nb += sqrtf(sx * sy); nc += sy;
     }
-    if (ROWS && (g + 1 == g1 || (g + 1) % a.frames == 0)) {    // last frame of the run or of its row
-      flush(blockIdx.x + (int)(g / a.frames));
+    if (ROWS && (g + 1 == g1 || g + 1 == (long long)gend * a.frames)) {    // last frame of the run or of its group
+      flush(blockIdx.x + grp);
 #pragma unroll
       for (int i = 0; i < 8; ++i) { sa[i] = 0.f; sb[i] = 0.f; sc[i] = 0.f; }
       na = nb = nc = 0.f;
+      if (g + 1 < g1) {
+        ++grp;
+        gend = a.offsets == nullptr ? grp + 1 : a.offsets[grp + 1];
+      }
     }
   }
   if (!ROWS) flush(blockIdx.x);
 }
 
-// abc[row][i] = sum of the row's segment partials (slots g + row of the CTAs g whose run touches the row); the same
-// 8-slice fixed-order sum as k_reduce_stats, so one row alone gives k_reduce_stats' result bit for bit
-__global__ void __launch_bounds__(256) k_reduce_stats_rows(const float* partial, int frames, int q, int n, double* abc) {
+// abc[grp][i] = sum of the group's segment partials (slots g + grp of the CTAs g whose run touches the group's rows
+// [r0, r1); offsets NULL: group = row); the same 8-slice fixed-order sum as k_reduce_stats, so one group of all rows
+// gives k_reduce_stats' result bit for bit
+__global__ void __launch_bounds__(256) k_reduce_stats_rows(const float* partial, int frames, int q, int n, double* abc,
+                                                           const int* offsets) {
   __shared__ double sl[8][33];
-  const int row = blockIdx.y;
+  const int grp = blockIdx.y;
+  const int r0 = offsets == nullptr ? grp : offsets[grp], r1 = offsets == nullptr ? grp + 1 : offsets[grp + 1];
   const int o = threadIdx.x & 31, sidx = threadIdx.x >> 5;
   const int i = blockIdx.x * 32 + o;
-  const long long g_lo = ((long long)row * frames) / q, g_hi = ((long long)(row + 1) * frames - 1) / q;
+  const long long g_lo = ((long long)r0 * frames) / q, g_hi = ((long long)r1 * frames - 1) / q;
   double s = 0.0;
   if (i < n)
-    for (long long g = g_lo + sidx; g <= g_hi; g += 8) s += (double)partial[(size_t)(g + row) * n + i];
+    for (long long g = g_lo + sidx; g <= g_hi; g += 8) s += (double)partial[(size_t)(g + grp) * n + i];
   sl[sidx][o] = s;
   __syncthreads();
   if (sidx == 0 && i < n) {
     double t = 0.0;
 #pragma unroll
     for (int k = 0; k < 8; ++k) t += sl[k][o];
-    abc[(size_t)row * n + i] = t;
+    abc[(size_t)grp * n + i] = t;
   }
 }
 
@@ -727,7 +750,8 @@ int launch_stats_rows_fused(FusedStatsArgs a, double* abc, cudaStream_t st) {
   int rc = check_launch("k_stats_fused");
   if (rc) return rc;
   const int n = 3 * Core4k::F;
-  k_reduce_stats_rows<<<dim3((n + 31) / 32, a.B), 256, 0, st>>>(a.partial, a.frames, a.q, n, abc);
+  const int groups = a.offsets == nullptr ? a.B : a.G;
+  k_reduce_stats_rows<<<dim3((n + 31) / 32, groups), 256, 0, st>>>(a.partial, a.frames, a.q, n, abc, a.offsets);
   return check_launch("k_reduce_stats_rows");
 }
 

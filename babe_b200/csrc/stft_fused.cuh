@@ -31,11 +31,15 @@ struct FusedStatsArgs {
   const float* window; const float2* roots;
   float* partial;                                       // [CTAs][3][F]
   int q, frames;                                        // filled by the launcher (q: frames per CTA)
+  // per-row statistics only: DEVICE int[G + 1] group offsets 0 = o_0 < ... < o_G = B (group g is rows
+  // [o_g, o_{g+1})); NULL: every row is its own group (G = B)
+  const int* offsets; int G;
 };
 bool fused_stats_eligible(const float* x, const float* y, int T, int mode);
 // launches k_stats_fused; *n_partials = rows of `partial` written (<= 2 * SM count)
 int launch_stats_fused(FusedStatsArgs a, int* n_partials, cudaStream_t st);
-// per-row statistics: abc[B][3][F]; `partial` needs fused_stats_rows_slots(B, T) rows of 3 F floats
+// per-row (offsets NULL) or per-group statistics: abc[G][3][F]; `partial` needs fused_stats_rows_slots(B, T) rows of
+// 3 F floats
 size_t fused_stats_rows_slots(int B, int T);
 int launch_stats_rows_fused(FusedStatsArgs a, double* abc, cudaStream_t st);
 

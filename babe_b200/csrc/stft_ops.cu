@@ -1126,3 +1126,56 @@ extern "C" int babe_stft_stats_rows(const float* x, const float* y, int B, int T
   }
   return BABE_OK;
 }
+
+// ---------------------------------------------------------------------------
+// Statistics per group of consecutive rows.  NFFT 4096 rows that can be bulk-copied: the per-row launch of the fused
+// statistics kernel with the group offsets (one partial per (CTA, group) segment).  Every other case: per-row
+// statistics into the workspace, then k_group_sum adds each group's rows in row order.
+// ---------------------------------------------------------------------------
+// abc[g][i] = rows[o_g][i] + rows[o_g + 1][i] + ... (fixed order; a singleton group is copied exactly)
+__global__ void __launch_bounds__(256) k_group_sum(const double* rows, const int* offsets, int n, double* abc) {
+  const int grp = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  const int r0 = offsets[grp], r1 = offsets[grp + 1];
+  double s = rows[(size_t)r0 * n + i];
+  for (int r = r0 + 1; r < r1; ++r) s += rows[(size_t)r * n + i];
+  abc[(size_t)grp * n + i] = s;
+}
+
+// fallback layout of the workspace: the per-row statistics (double[B,3F]), then babe_stft_stats_rows' workspace
+static size_t group_rows_bytes(int B, int nfft) {
+  return ((size_t)B * 3 * (nfft / 2 + 1) * sizeof(double) + 255) & ~(size_t)255;
+}
+
+extern "C" size_t babe_stft_stats_groups_workspace(int B, int T, int nfft) {
+  if (!babe_stft_supported(nfft) || B < 1 || T < 1) return 0;
+  return group_rows_bytes(B, nfft) + babe_stft_stats_rows_workspace(B, T, nfft);
+}
+
+extern "C" int babe_stft_stats_groups(const float* x, const float* y, int B, int T, int nfft,
+                                      const float* window, const float* twiddle, const int* offsets, int G,
+                                      double* abc, void* workspace, size_t workspace_bytes, void* stream) {
+  BABE_REQUIRE(x && y && window && twiddle && offsets && abc, BABE_EBADARG, "stft_stats_groups: null pointer");
+  BABE_REQUIRE(B >= 1 && T >= 1, BABE_EBADARG, "stft_stats_groups: bad shape B=%d T=%d", B, T);
+  BABE_REQUIRE(G >= 1 && G <= B, BABE_EBADARG, "stft_stats_groups: %d groups for %d rows", G, B);
+  BABE_REQUIRE(babe_stft_supported(nfft), BABE_EUNSUPPORTED, "unsupported NFFT %d", nfft);
+  const size_t need = babe_stft_stats_groups_workspace(B, T, nfft);
+  BABE_REQUIRE(workspace != nullptr && workspace_bytes >= need, BABE_EBADARG,
+               "stft_stats_groups: workspace too small (%zu < %zu)", workspace_bytes, need);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (nfft == 4096 && fused_stats_eligible(x, y, T, 0)) {
+    FusedStatsArgs f{};
+    f.x = x; f.y = y; f.B = B; f.T = T; f.window = window; f.roots = reinterpret_cast<const float2*>(twiddle);
+    f.partial = static_cast<float*>(workspace);
+    f.offsets = offsets; f.G = G;
+    return launch_stats_rows_fused(f, abc, st);
+  }
+  const size_t rows_bytes = group_rows_bytes(B, nfft);
+  double* rows = static_cast<double*>(workspace);
+  const int rc = babe_stft_stats_rows(x, y, B, T, nfft, window, twiddle, rows,
+                                      static_cast<char*>(workspace) + rows_bytes, workspace_bytes - rows_bytes, stream);
+  if (rc) return rc;
+  const int n = 3 * (nfft / 2 + 1);
+  k_group_sum<<<dim3((n + 255) / 256, G), 256, 0, st>>>(rows, offsets, n, abc);
+  return check_launch("k_group_sum");
+}

@@ -293,6 +293,59 @@ def stft_stats_rows(x, y, nfft):
     return abc
 
 
+_GROUP_OFFSETS = {}
+
+
+def group_sizes(sizes, B):
+    """``sizes`` as a tuple of positive ints summing to B (ValueError otherwise)."""
+    try:
+        out = tuple(sizes)
+    except TypeError:
+        raise ValueError(f"group sizes must be a list of positive ints, got {sizes!r}") from None
+    for n in out:
+        if isinstance(n, bool) or not isinstance(n, int) and not hasattr(n, "__index__") or int(n) < 1:
+            raise ValueError(f"group sizes must be positive ints, got {list(out)!r}")
+    out = tuple(int(n) for n in out)
+    if not out or sum(out) != B:
+        raise ValueError(f"group sizes {list(out)} must sum to the {B} rows")
+    return out
+
+
+def group_offsets(sizes, device):
+    """Device int32[G + 1] offsets 0, n_0, n_0 + n_1, ..., B of a group layout, cached per (sizes, device) so that a
+    captured graph keeps reading a live buffer."""
+    dev = torch.device(device)
+    key = (tuple(sizes), dev.index if dev.index is not None else torch.cuda.current_device())
+    if key not in _GROUP_OFFSETS:
+        off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int32)
+        _GROUP_OFFSETS[key] = torch.from_numpy(off).to(dev)
+    return _GROUP_OFFSETS[key]
+
+
+def stft_stats_groups(x, y, nfft, sizes):
+    """float64[G,3,F]: ``stft_stats`` (mode 0) summed over each group of consecutive rows; ``sizes`` (host ints
+    n_0, ..., n_{G-1}, each >= 1, summing to B): group g is rows [n_0 + ... + n_{g-1}, ... + n_g)."""
+    if not (torch.is_tensor(x) and torch.is_tensor(y)):
+        raise TypeError("x and y must be tensors")
+    if x.shape != y.shape or x.dim() != 2:
+        raise ValueError("x and y must both be (B, T)")
+    sizes = group_sizes(sizes, x.shape[0])
+    x = _cuda_f32(x, "x")
+    y = _cuda_f32(y, "y")
+    B, T = x.shape
+    G = len(sizes)
+    win, tw = stft_tables(nfft, x.device)
+    off = group_offsets(sizes, x.device)
+    F = nfft // 2 + 1
+    nbytes = lib().babe_stft_stats_groups_workspace(B, T, int(nfft))
+    ws = torch.empty(nbytes // 4, dtype=torch.float32, device=x.device)
+    abc = torch.empty(G, 3, F, dtype=torch.float64, device=x.device)
+    with profiling.op("stft_stats_groups", 2, 8 * B * T):
+        check(lib().babe_stft_stats_groups(_p(x), _p(y), B, T, int(nfft), _p(win), _p(tw), _p(off), G, _p(abc),
+                                           _p(ws), nbytes, _stream()), "stft_stats_groups")
+    return abc
+
+
 def spec_mag_stats(X, Xref, H=None, w=None):
     """float64[4,F]: a, b, c and s_k = sum (w_k (H_k|X| - |Xref|))^2."""
     X = _cuda_f32(X, "X")

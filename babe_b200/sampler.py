@@ -25,7 +25,9 @@ purely in execution:
 One behaviour goes beyond the reference: with ``filter_per_row`` every row of ``y``
 is an independent restoration (its own fit statistics, filter fit, guidance
 filter and guidance normaliser), i.e. row r of one call with B rows is what a
-call on ``y[r:r+1]`` alone returns with the same noise for that row.
+call on ``y[r:r+1]`` alone returns with the same noise for that row.  Between the
+two, ``filter_groups`` (sizes of consecutive row groups) gives every group one
+filter: group g of one call is what a shared-filter call on its rows alone returns.
 """
 import types
 import warnings
@@ -112,6 +114,7 @@ class FilterFit:
         self.w = w if w is not None else torch.ones(self.nfft // 2 + 1, device=device)
         self.joint = False
         self.per_row = False           # True: params (B, 2, K), one fit per row on that row's statistics
+        self.groups = None             # group sizes: params (G, 2, K), one fit per group of consecutive rows
 
     @classmethod
     def from_args(cls, args, device):
@@ -127,6 +130,8 @@ class FilterFit:
                 c.clamp_fc, c.clamp_A, c.only_negative_A)
 
     def stats(self, x_den, y):
+        if self.groups is not None:
+            return ops.stft_stats_groups(x_den, y, self.nfft, self.groups)
         if self.per_row:
             return ops.stft_stats_rows(x_den, y, self.nfft)
         return ops.stft_stats(x_den, y, self.nfft, mode=0)
@@ -136,7 +141,7 @@ class FilterFit:
         testing/blind_bwe_sampler.py:577-583) and returned; (B,2,K) per row with ``per_row``."""
         if abc is None:
             abc = self.stats(x_den, y)
-        if self.per_row:
+        if self.per_row or self.groups is not None:
             return ops.fit_params_rows(abc, self.w, self.freqs, params, self.cfg, return_iters=return_iters)
         if self.joint:                 # one filter for the rows of ALL ranks (SURVEY 8e)
             from . import distributed
@@ -242,6 +247,11 @@ class BlindSamplerFused:
         # True: every row of y is an independent restoration (own filter estimate and guidance scale); Hydra-style
         # configs switch it on with tester.blind_bwe.filter_per_row
         self.filter_per_row = bool(getattr(args.tester.blind_bwe, "filter_per_row", False))
+        # None, or the sizes [n_0, ..., n_{G-1}] (sum = B) of consecutive row groups of the next predict_blind_bwe
+        # call: group g (rows o_g .. o_g + n_g - 1) is restored with ONE filter, as a shared-filter call on its rows
+        # alone would restore it (statistics summed over the group, one fit, the group's guidance normaliser)
+        self.filter_groups = None
+        self._groups = None            # during a grouped call: sizes and the device row -> group maps
         self._fit = None
 
     def update_diff_params(self):
@@ -426,6 +436,7 @@ class BlindSamplerFused:
         ps = self.args.tester.posterior_sampling
         self._maybe_noise_observations(y, self._eval_slot + 2)
         nfft = self.args.tester.blind_bwe.NFFT
+        filter_params = self._row_params(filter_params)
         if ps.norm == 2 and not ps.stft_distance.use:
             norm = rec_guidance_norms(x_den, y, self.freqs, filter_params, nfft)
         else:
@@ -448,7 +459,12 @@ class BlindSamplerFused:
             else:
                 norm = torch.linalg.norm(y - den_rec, dim=1, ord=ps.norm)
         (rec_grads,) = torch.autograd.grad(outputs=norm.sum(), inputs=x)
-        if self.filter_per_row:        # each row is its own restoration: its own normaliser
+        if self._groups is not None:   # Frobenius norm over each group's rows, in fp64, gathered back to the rows
+            g = self._groups
+            sq = (rec_grads.double() ** 2).sum(1)
+            gsq = torch.cat((sq, sq.new_zeros(1)))[g.pad].sum(1)       # padding reads the appended zero
+            normguide = torch.sqrt(gsq).float()[g.row_group].unsqueeze(1) / self.args.exp.audio_len ** 0.5
+        elif self.filter_per_row:      # each row is its own restoration: its own normaliser
             normguide = torch.linalg.norm(rec_grads, dim=1, keepdim=True) / self.args.exp.audio_len ** 0.5
         elif self.joint:               # Frobenius norm over the rows of ALL ranks (:125)
             from . import distributed
@@ -461,7 +477,13 @@ class BlindSamplerFused:
 
     def data_consistency_step_classic(self, x_hat, y, filter_params):
         """testing/blind_bwe_sampler.py:63-73."""
-        return y + x_hat - self.apply_filter_fcA(x_hat, filter_params)
+        return y + x_hat - self.apply_filter_fcA(x_hat, self._row_params(filter_params))
+
+    def _row_params(self, filter_params):
+        """Grouped calls: the (B, 2, K) parameters of the rows, row r taking its group's filter; else unchanged."""
+        if self._groups is None:
+            return filter_params
+        return filter_params.index_select(0, self._groups.row_group)
 
     def _evaluate(self, x_in, t_in, y, filter_params, slot=1):
         """Lines :689-:709 (and :733-:752 for the Heun correction, keyed draw slot 4)."""
@@ -493,6 +515,36 @@ class BlindSamplerFused:
         if compute_sweep:
             raise NotImplementedError("filter_per_row with compute_sweep: the sweep evaluates one loss surface on "
                                       "the statistics of the whole batch")
+
+    def _begin_groups(self, B, device, compute_sweep):
+        """Check ``filter_groups`` against a call on B rows and build its device row -> group maps (None: off)."""
+        self._groups = None
+        if self.filter_groups is None:
+            return
+        sizes = ops.group_sizes(self.filter_groups, B)
+        if self.joint or self.filter_per_row:
+            raise ValueError("filter_groups excludes joint and filter_per_row: choose one way of sharing filters "
+                             "(joint: one over all ranks, filter_per_row: one per row, filter_groups: one per group)")
+        sd = self.args.tester.posterior_sampling.stft_distance
+        if sd.use:
+            raise NotImplementedError("filter_groups with the STFT-distance guidance: its norm is one sum over the "
+                                      "whole batch, not a per-group quantity")
+        if compute_sweep:
+            raise NotImplementedError("filter_groups with compute_sweep: the sweep evaluates one loss surface on the "
+                                      "statistics of the whole batch")
+        G, nmax = len(sizes), max(sizes)
+        row_group = torch.repeat_interleave(torch.arange(G), torch.tensor(sizes))
+        pad = torch.full((G, nmax), B, dtype=torch.int64)              # index B: the zero appended to the rows
+        o = 0
+        for g, n in enumerate(sizes):
+            pad[g, :n] = torch.arange(o, o + n)
+            o += n
+        self._groups = types.SimpleNamespace(sizes=sizes, row_group=row_group.to(device), pad=pad.to(device))
+
+    def _no_groups(self, what):
+        if self.filter_groups is not None:
+            raise ValueError(f"{what} does not support filter_groups (set it to None): only predict_blind_bwe "
+                             "estimates a filter per group")
 
     def compute_sweep(self, denoised_estimate, y):
         """testing/blind_bwe_sampler.py:598-616 on the collapsed statistics."""
@@ -535,8 +587,9 @@ class BlindSamplerFused:
         keyed = self._keyed
         # keyed noise is generated inside the step from the graph's seed and draw-index buffers: the key records that
         # it is on, not the seed values (new seeds are copied into the buffers, no recapture)
+        groups = self._groups
         key = (tuple(y.shape), y.device, tuple(filter_params.shape), self.filter_per_row, keyed is not None,
-               self._fit.cfg_key())
+               self._fit.cfg_key(), None if groups is None else groups.sizes)
         if self._step_key != key:
             self._step_key, self._step_graphs = key, {}
         if heun in self._step_graphs:
@@ -551,7 +604,7 @@ class BlindSamplerFused:
             y=y.clone(), fit=self._fit, freqs=self.freqs,
             x=torch.zeros_like(y), fp=filter_params.clone(), eps=None if keyed is not None else torch.zeros_like(y),
             t_i=torch.ones((), device=dev), gamma=torch.zeros((), device=dev), t_next=torch.ones((), device=dev) * 0.5,
-            seeds=None, draw=None, graph=None, x_out=None, fp_out=None, den=None, launches=0)
+            seeds=None, draw=None, graph=None, x_out=None, fp_out=None, den=None, launches=0, groups=groups)
         if keyed is not None:
             st.seeds, st.draw = keyed.seeds.clone(), torch.zeros_like(keyed.draw)
             self._keyed = types.SimpleNamespace(seeds=st.seeds, draw=st.draw)     # what the captured kernels read
@@ -603,8 +656,10 @@ class BlindSamplerFused:
 
         With ``filter_per_row`` the rows of y are independent restorations: the returned filter is (B, 2, K),
         ``init_params`` may be (2, K) (every row) or (B, 2, K), and with ``rid`` the logged filters are
-        (T, B, 2, K)."""
+        (T, B, 2, K).  With ``filter_groups`` (G sizes) the same holds per group: (G, 2, K) filters, ``init_params``
+        (2, K) or (G, 2, K), logged filters (T, G, 2, K)."""
         args = self.args
+        self._begin_groups(y.shape[0], y.device, compute_sweep)
         self._keyed_begin(y.shape[0], y.device)
         if self.filter_per_row:
             self._check_per_row(compute_sweep)
@@ -613,6 +668,7 @@ class BlindSamplerFused:
         self._fit = FilterFit.from_args(args, device)
         self._fit.joint = self.joint
         self._fit.per_row = self.filter_per_row
+        self._fit.groups = None if self._groups is None else self._groups.sizes
         shape = y.shape
         filter_params = torch.Tensor([args.tester.blind_bwe.initial_conditions.fc,
                                       args.tester.blind_bwe.initial_conditions.A]).to(device)
@@ -620,11 +676,12 @@ class BlindSamplerFused:
             filter_params.unsqueeze_(1)
         if init_params is not None:
             filter_params = init_params.to(device).clone()
-        if self.filter_per_row:
+        if self.filter_per_row or self._groups is not None:
+            n, what = (shape[0], "per-row") if self._groups is None else (len(self._groups.sizes), "per-group")
             if filter_params.dim() == 2:
-                filter_params = filter_params.unsqueeze(0).expand(shape[0], -1, -1)
-            if filter_params.dim() != 3 or filter_params.shape[0] != shape[0]:
-                raise ValueError(f"per-row filter parameters must be (2, K) or ({shape[0]}, 2, K), "
+                filter_params = filter_params.unsqueeze(0).expand(n, -1, -1)
+            if filter_params.dim() != 3 or filter_params.shape[0] != n:
+                raise ValueError(f"{what} filter parameters must be (2, K) or ({n}, 2, K), "
                                  f"got {tuple(filter_params.shape)}")
             filter_params = filter_params.contiguous().clone()
         if compute_sweep:
@@ -715,6 +772,7 @@ class BlindSamplerFused:
                 step_hook(i, x, filter_params)
 
         self._keyed = None
+        self._groups = None
         if rid:
             out = (x.detach(), filter_params.detach(), data_denoised.detach(), t.detach(), data_filters.detach())
             if compute_sweep:
@@ -724,6 +782,7 @@ class BlindSamplerFused:
 
     def predict_unconditional(self, shape, device, rid=False):
         """testing/blind_bwe_sampler.py:366-374,406-497 with y = None."""
+        self._no_groups("predict_unconditional")
         self._keyed_begin(shape[0], device)
         t = self.diff_params.create_schedule(self.nb_steps).to(device)
         x = self._initial_state(shape, device, t[0])
@@ -836,6 +895,7 @@ class BlindSamplerFused:
 
     def predict_conditional(self, y, degradation, rid=False, dc_step=None, fused_params=None, known=None):
         """testing/blind_bwe_sampler.py:387-497 (``predict`` with observations y)."""
+        self._no_groups("predict_conditional")
         shape, device = y.shape, y.device
         self._keyed_begin(shape[0], device)
         if self.start_sigma is None:
@@ -880,6 +940,7 @@ class BlindSamplerFused:
         With ``filter_per_row`` the rows are independent windows: ``filt`` is (2, K) (every row) or (B, 2, K), the
         (B, T) mask may differ per row and each row gets its own smoothed mask and guidance normaliser."""
         assert mask is not None
+        self._no_groups("predict_bwe_AR")
         if test_filter_fit or compute_sweep:
             raise NotImplementedError("test_filter_fit / compute_sweep logging on the AR path")
         if self.filter_per_row:
@@ -941,6 +1002,7 @@ class BlindSamplerFused:
         applies the classic data-consistency step and xi == 0 uses the plain denoiser.  ``fc_A`` (parametric filter,
         fused design + STFT filter guidance) and the FIR models run on the CUDA operators; the IIR / biquad /
         resampling models and the logging-only ``test_filter_fit`` / ``compute_sweep`` flags raise."""
+        self._no_groups("predict_bwe")
         if filt_type not in ("fc_A", "firwin", "firwin_hpf"):
             raise NotImplementedError(f"filt_type {filt_type!r}: 'fc_A', 'firwin' and 'firwin_hpf' run on the "
                                       "CUDA operators; the IIR / resampling models are outside this path")

@@ -57,6 +57,17 @@ def _filter_per_row(sampler, on):
         sampler.filter_per_row = was
 
 
+@contextlib.contextmanager
+def _filter_groups(sampler, sizes):
+    """Set the sampler's ``filter_groups`` for one call and restore the previous value afterwards."""
+    was = sampler.filter_groups
+    sampler.filter_groups = sizes
+    try:
+        yield
+    finally:
+        sampler.filter_groups = was
+
+
 def segment_spans(L, seg_len, ola=256, discard_end=200, discard_start=0):
     """Start indices exactly as the while-loop at testing/blind_bwe_tester.py:469-521
     produces them; the last span is the incomplete tail (:526-533)."""
@@ -159,6 +170,73 @@ def restore_recording(sampler, degraded, seg_len, ola=256, discard_end=200, join
     all_filt = bd.gather_rows(filts)
     final = merge(all_pred, spans, degraded.shape[-1], ola, discard_end)
     return final, [(spans[s], all_filt[s]) for s in range(len(spans))]
+
+
+def pack_recordings(sizes, max_rows=None):
+    """Consecutive runs of recordings (lists of indices) whose segment counts ``sizes`` add up to at most
+    ``max_rows`` each, filled greedily in order; one run of all recordings when ``max_rows`` is None."""
+    if max_rows is not None and (isinstance(max_rows, bool) or not isinstance(max_rows, int) or max_rows < 1):
+        raise ValueError(f"max_rows must be a positive int, got {max_rows!r}")
+    if max_rows is None or not sizes:
+        return [list(range(len(sizes)))] if sizes else []
+    calls, cur, rows = [], [], 0
+    for r, n in enumerate(sizes):
+        if n > max_rows:
+            raise ValueError(f"recording {r} has {n} segments, more than max_rows = {max_rows}: a recording's "
+                             "segments share one filter and cannot be split over calls")
+        if rows + n > max_rows:
+            calls.append(cur)
+            cur, rows = [], 0
+        cur.append(r)
+        rows += n
+    calls.append(cur)
+    return calls
+
+
+def restore_recordings(sampler, recordings, seg_len, ola=256, discard_end=200, seeds=None, max_rows=None):
+    """Blind restoration of N recordings with ONE filter each, the segments of many recordings in one sampler call.
+
+    Every recording is cut as ``restore_recording`` cuts it; the segments of consecutive recordings go into one
+    ``predict_blind_bwe`` call with ``filter_groups = [S_0, S_1, ...]`` (recording r's S_r segments are one group:
+    summed fit statistics, one filter fit, one guidance normaliser), so recording r is restored as
+    ``restore_recording(joint=True)`` restores it alone in one process.  ``max_rows`` bounds the rows of a call:
+    whole recordings are packed greedily, in order (a recording with more than ``max_rows`` segments raises
+    ValueError); None puts every recording into one call.
+
+    ``recordings``: mono (1, L_r) tensors on one device.  ``seeds`` (one int per recording) switches to keyed noise:
+    segment s of recording r draws with ``row_seed(seeds[r], s)``, the seed ``restore_recording(seed=seeds[r])``
+    gives it.  Single process: sharding recordings over ranks is the caller's.  The sampler's ``filter_groups``,
+    ``filter_per_row`` and ``row_seeds`` are restored afterwards.  Returns [(restored (1, L_r), filter_data), ...],
+    ``filter_data`` the list [((ix0, ix1), filter (2, K)), ...] of ``restore_recording`` with the recording's one
+    filter on every span."""
+    if getattr(sampler, "joint", False):
+        raise ValueError("restore_recordings gives every recording its own filter; joint=True shares one over all "
+                         "rows of all ranks")
+    recs = [r.reshape(1, -1) if r.dim() == 1 else r for r in recordings]
+    N = len(recs)
+    for i, r in enumerate(recs):
+        if r.dim() != 2 or r.shape[0] != 1:
+            raise ValueError(f"recording {i} must be mono (1, L), got {tuple(r.shape)}")
+        if r.device != recs[0].device:
+            raise ValueError(f"recording {i} is on {r.device}, recording 0 on {recs[0].device}: one device for all")
+    if seeds is not None and len(seeds) != N:
+        raise ValueError(f"{len(seeds)} seeds for {N} recordings")
+    cuts = [split(r, seg_len, ola, discard_end) for r in recs]
+    sizes = [segs.shape[0] for segs, _ in cuts]
+    out = [None] * N
+    for rows in pack_recordings(sizes, max_rows):
+        y = torch.cat([cuts[r][0] for r in rows])
+        row_seeds = None if seeds is None else [row_seed(seeds[r], s) for r in rows for s in range(sizes[r])]
+        with _filter_groups(sampler, [sizes[r] for r in rows]), _filter_per_row(sampler, False), \
+                _row_seeds(sampler, row_seeds):
+            pred, filts = sampler.predict_blind_bwe(y, rid=False)
+        o = 0
+        for g, r in enumerate(rows):
+            spans = cuts[r][1]
+            final = merge(pred[o:o + sizes[r]], spans, recs[r].shape[-1], ola, discard_end)
+            out[r] = (final, [(sp, filts[g]) for sp in spans])
+            o += sizes[r]
+    return out
 
 
 def ar_windows(L, seg_len, overlap, discard_end=200, discard_start=0):

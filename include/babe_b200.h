@@ -190,6 +190,18 @@ size_t babe_stft_stats_rows_workspace(int B, int T, int nfft);
 int babe_stft_stats_rows(const float* x, const float* y, int B, int T, int nfft,
                          const float* window, const float* twiddle,
                          double* abc, void* workspace, size_t workspace_bytes, void* stream);
+/* Mode-0 statistics per group of consecutive rows: abc is double[G,3F], group g's block sums the statistics of rows
+ * [offsets[g], offsets[g+1]).  offsets is a DEVICE int[G+1] that the caller guarantees to hold
+ * 0 = offsets[0] < offsets[1] < ... < offsets[G] = B (1 <= G <= B); it is read by the kernels, not on the host, so
+ * that a captured graph reads it by address.  NFFT 4096 rows that can be bulk-copied: one launch of the fused
+ * statistics kernel with one partial per (CTA, group) segment and a fixed-order fp64 reduction per group (one group
+ * of all rows is bitwise babe_stft_stats, all-singleton groups bitwise babe_stft_stats_rows); otherwise
+ * babe_stft_stats_rows into the workspace and a fixed-order fp64 sum per group.  Deterministic; a group's result does
+ * not depend on the other groups' rows.  workspace: babe_stft_stats_groups_workspace() bytes. */
+size_t babe_stft_stats_groups_workspace(int B, int T, int nfft);
+int babe_stft_stats_groups(const float* x, const float* y, int B, int T, int nfft,
+                           const float* window, const float* twiddle, const int* offsets, int G,
+                           double* abc, void* workspace, size_t workspace_bytes, void* stream);
 /* Same statistics from precomputed spectrograms X, Xref [B,F,frames,2] as the
  * reference signature apply_filter_and_norm_STFTmag_fweighted(X, Xref, H, w)
  * (utils/blind_bwe_utils.py:250-296) receives them.  out is double[4F]:
